@@ -2,7 +2,7 @@
 """bench.py -- frames/s of the SRFDet3D point-cloud -> region-feature hot path on B200.
 
   python bench.py --gpus N --steps K --warmup W [--workload nusc_LC|nusc_L|waymo_L|kitti_L]
-                  [--scope full|path] [--precision fp16|fp32|bf16|fp32_simt] [--frames-in-flight F]
+                  [--scope full|path] [--precision fp16|fp32|bf16|fp32_simt] [--frames-in-flight F] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...          (one rank per GPU; frames are independent)
   python bench.py --impl reference ...        (restated reference CPU path on the host cores)
 
@@ -177,6 +177,25 @@ def kernel_families(pipe, pts, pk, torch, reps=3):
     return fams, round(tot, 4), [dict(flops=f, bytes=b, **d) for f, b, d in sparse]
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(frames_out, out_dir):
+    """Writes what the caller of run_frame / run_frames receives for each frame j of one step, as float32
+    out_dir/frame<j>_bev.npy (dense BEV map) and out_dir/frame<j>_result.npy (scope 'full': decoded boxes and class scores;
+    scope 'path': region features).  An array larger than its equal share of DUMP_BYTES is stored as a sample of its
+    flattened elements at seeded indices, the same in every run, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = (DUMP_BYTES // (2 * len(frames_out)) - 4096) // 4          # float32 elements per array (4 KB kept for the header)
+    for j, arrays in enumerate(frames_out):
+        for name, t in zip(('bev', 'result'), arrays):
+            a = t.float().cpu().numpy()
+            if a.size > share:
+                a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+            np.save(os.path.join(out_dir, f'frame{j}_{name}.npy'), a)
+
+
 def pipe_enc(pipe):
     from srfdet_b200 import _lib as L
     from srfdet_b200.plugin import registry
@@ -256,7 +275,13 @@ def main():
     ap.add_argument('--profiler-range', action='store_true',
                     help='cudaProfilerStart/Stop around the device-resident timed steps (ncu --profile-from-start off: launch list of the timed region only)')
     ap.add_argument('--kernels-out', default=None, help='write the kernel-family table and the per-layer sparse-conv work (JSON) here')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the outputs of the last device-resident timed step to DIR/<name>.npy (float32, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     wl = WORKLOADS[args.workload]
     if args.impl == 'reference':
@@ -296,15 +321,16 @@ def main():
         return c, [torch.as_tensor(x).cuda() for x in c], [torch.as_tensor(x).pin_memory() for x in c]
 
     def timed(pipe, inputs, steps, warmup, fif, host):
-        """`steps` steps of `fif` concurrent frames; events on the current stream bracket each step; L2 flushed between."""
+        """`steps` steps of `fif` concurrent frames; events on the current stream bracket each step; L2 flushed between.
+        The per-frame outputs of the last step are left in timed.last."""
         def step(i):
             batch = [inputs[(i * fif + j) % N_CLOUDS] for j in range(fif)]
             if fif == 1 and not host:
-                pipe.run_frame(batch[0])
+                return [pipe.run_frame(batch[0])]
             elif fif == 1:
-                pipe.run_frame_host(batch[0])
+                return [pipe.run_frame_host(batch[0])]
             else:
-                pipe.run_frames(batch, host=host)
+                return pipe.run_frames(batch, host=host)
         for i in range(warmup):
             step(i)
         barrier()
@@ -316,7 +342,7 @@ def main():
             flush.zero_()                                # evict the previous frames from L2 (not timed)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            step(i)
+            timed.last = step(i)
             e1.record()
             evs.append((e0, e1))
         barrier()
@@ -339,6 +365,8 @@ def main():
     launches_per_frame = int(lib.srf_launch_count() - n0)      # this library's kernels per frame (counted eagerly)
     pipe.use_graph = not args.no_graph
     ms_dev = timed(pipe, clouds_dev, args.steps, args.warmup, fif, host=False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(timed.last, args.dump_outputs)     # before the end-to-end steps replay the same graphs
     ms_e2e = timed(pipe, clouds_pin, args.steps, args.warmup, fif, host=True)
     clocks = sampler.stop() if rank == 0 else None
     fps = world * args.steps * fif / (ms_dev * 1e-3)

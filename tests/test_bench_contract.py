@@ -39,6 +39,33 @@ def test_reference_arm_line_and_isolation():
     assert line['config']['workload'] == 'nusc_LC'
 
 
+def test_dump_outputs_budget_and_fixed_sample(tmp_path):
+    """--dump-outputs: float32 .npy per frame output, small arrays whole, large ones sampled at the same indices in every
+    run, the directory within bench.DUMP_BYTES even at many frames in flight."""
+    import importlib.util
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location('bench_under_test', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    bev = torch.randn(1, 256, 184, 184, generator=g)                    # the nuScenes BEV map: 34.7 MB in float32
+    result = torch.randn(900, 19, generator=g, dtype=torch.float64)
+    for fif in (1, 4, 16):
+        d = tmp_path / str(fif)
+        bench.dump_outputs([(bev, result)] * fif, str(d))
+        files = sorted(os.listdir(d))
+        assert files == sorted(f'frame{j}_{n}.npy' for j in range(fif) for n in ('bev', 'result'))
+        assert sum(os.path.getsize(d / f) for f in files) <= bench.DUMP_BYTES
+        r = np.load(d / 'frame0_result.npy')
+        assert r.dtype == np.float32 and np.array_equal(r, result.float().numpy())
+        b = np.load(d / f'frame{fif - 1}_bev.npy')
+        assert b.dtype == np.float32 and b.ndim == 1 and b.size < bev.numel()
+        assert np.isin(b, bev.numpy()).all()
+    bench.dump_outputs([(bev, result)] * 4, str(tmp_path / 'again'))
+    assert np.array_equal(np.load(tmp_path / 'again' / 'frame3_bev.npy'), np.load(tmp_path / '4' / 'frame3_bev.npy'))
+
+
 def test_committed_b200_line_contract():
     line = json.load(open(os.path.join(ROOT, 'profiles', 'r02_bench_nusc_LC.json')))
     _check_base(line)

@@ -67,15 +67,19 @@ def test_config_builds_drop_in_modules(tag, golden_dir):
     assert tuple(w.shape) == (16, 3, 3, 3, e['in_channels'])          # spconv-2 layout
 
 
-def test_reference_config_files_load_if_present():
-    """In the build container the reference's unmodified config files build the modules."""
-    path = '/root/reference/configs/waymo/srfdet_dvoxel_waymo_L.py'
-    if not os.path.exists(path):
-        pytest.skip('reference tree not present (GPU box)')
+def test_reference_config_files_load_if_present(golden_dir):
+    """Config files in the reference's plain-Python form (tests/golden/configs: the model sections of two of its configs)
+    build the modules."""
     from srfdet_b200.plugin import SRFDetPointPath, build_head, build_roi_extractor, load_config
-    det = SRFDetPointPath.from_config(path)
+    with open(os.path.join(golden_dir, 'encoder_plan.json')) as f:
+        recorded = json.load(f)
+    for tag, name in [('waymo', 'waymo/srfdet_dvoxel_waymo_L.py'), ('nusc', 'nus/srfdet_voxel_nusc_LC.py')]:
+        enc = dict(load_config(os.path.join(golden_dir, 'configs', name))['model']['pts_middle_encoder'])
+        assert enc.pop('type') == 'SparseEncoderCustom'
+        assert json.loads(json.dumps(enc)) == recorded[tag]['cfg']        # what the original config files hold
+    det = SRFDetPointPath.from_config(os.path.join(golden_dir, 'configs', 'waymo', 'srfdet_dvoxel_waymo_L.py'))
     assert det.is_dynamic and len(det.pts_middle_encoder.layer_plan()) == 21
-    cfg = load_config('/root/reference/configs/nus/srfdet_voxel_nusc_LC.py')['model']['bbox_head']
+    cfg = load_config(os.path.join(golden_dir, 'configs', 'nus', 'srfdet_voxel_nusc_LC.py'))['model']['bbox_head']
     head = build_head(cfg['single_head_lidar'] | dict(num_classes=10, feat_channels=128))
     assert head.use_fusion and head.inst_interact_lidar.dynamic_dim == 32
     pooler = build_roi_extractor(cfg['roi_extractor_img'])
