@@ -448,6 +448,26 @@ int srf_dpg_mix(const float* logits_a, const float* logits_b, int32_t n_batch, i
 int srf_decode_boxes(const float* logits, int64_t n_logits, const float* boxes, int32_t k, int32_t dim,
                      float* scores, float* out, void* stream);
 
+/* ---------------------------------------------------------------------------------- *
+ * BEV NMS of SRFDetHead.get_bboxes with test_cfg.use_nms=True (sparse_heads/srfdet_head.py:1269-1296:
+ * xywhr2xyxyr -> mmdet3d box3d_multiclass_nms -> mmcv nms_bev / nms_normal_bev).  csrc/nms_bev.cu.
+ * Footprint of a box row: centre (x, y), extent dx along (cos yaw, sin yaw), dy along (-sin yaw, cos yaw).
+ * IoU = inter / (area a + area b - inter), 0 when an area is < 1e-14; suppression is IoU > iou_thr. */
+/* pairwise BEV IoU; box rows of width lda/ldb >= 7 with x, y, dx, dy, yaw at columns 0, 1, 3, 4, 6; rotated = 0: axis-aligned
+ * dx x dy (yaw ignored).  iou (m, n) row-major. */
+int srf_iou_bev(const float* a, int32_t m, int32_t lda, const float* b, int32_t n, int32_t ldb, int32_t rotated, float* iou, void* stream);
+size_t srf_nms_bev_ws_bytes(int32_t bs, int32_t k, int32_t n_cls);
+/* multi-class BEV NMS of get_bboxes; boxes (bs, k, dim >= 7), scores (bs, k, n_cls); post_center_range: host values passed into the kernel
+ * arguments like srf_apply_deltas' pc_range, NULL = no filter.  Per sample and class c: candidates scores[:, c] > score_thr in
+ * (score desc, index asc) order, greedy NMS; the kept lists are concatenated class-major; above max_num the max_num best scores are
+ * kept in (score desc, class-major position asc) order; then the range filter on columns 0..2 (order preserved).  Outputs of
+ * capacity max_num per sample: out_boxes (bs, max_num, dim), out_scores / out_labels (class) / out_index (row in boxes)
+ * (bs, max_num), d_count (bs); rows past the count hold a zero box, score 0, label and index -1.  k <= 1024, n_cls <= 32
+ * (SRF_ERR_UNSUPPORTED otherwise).  3 launches, no host synchronisation. */
+int srf_nms_bev(const float* boxes, int32_t bs, int32_t k, int32_t dim, const float* scores, int32_t n_cls, float score_thr,
+                float iou_thr, int32_t rotated, int32_t max_num, const float post_center_range[6], void* ws, size_t ws_bytes,
+                float* out_boxes, float* out_scores, int32_t* out_labels, int32_t* out_index, int32_t* d_count, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -180,6 +180,10 @@ PROTOTYPES = {
                                        POINTER(c_float), POINTER(RoiOut), c_void_p, c_void_p]),
     'srf_dynconv_interact': (c_int32, [c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    'srf_iou_bev': (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    'srf_nms_bev_ws_bytes': (c_size_t, [c_int32, c_int32, c_int32]),
+    'srf_nms_bev': (c_int32, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_float, c_float, c_int32, c_int32,
+                              POINTER(c_float), c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

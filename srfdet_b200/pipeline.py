@@ -87,7 +87,9 @@ def backbone_cfg(kind):
                 pts_neck=neck)
 
 
-def head_cfg(kind, fusion):
+def head_cfg(kind, fusion, use_nms=False):
+    """use_nms=True: the post-processing of every reference config (configs/nus/srfdet_voxel_nusc_LC.py:194-199,
+    configs/kitti/srfdet_voxel_kitti_L.py:183-188, configs/waymo/srfdet_dvoxel_waymo_L.py:171-176)."""
     h = HEAD_CFG[kind]
     layer = MODEL_CFG[kind]['pts_voxel_layer']
     wts = [1.0] * 8 + ([0.2, 0.2] if h['box_dim'] == 10 else [])
@@ -102,7 +104,8 @@ def head_cfg(kind, fusion):
                 hidden_dim=128, lidar_feat_lvls=4, img_feat_lvls=4, num_proposals=N_PROP, num_heads=N_STAGES, deep_supervision=True,
                 with_lidar_encoder=False, grid_size=h['grid'], out_size_factor=8, code_weights=wts, with_dpg=True, num_dpg_exp=4,
                 single_head_lidar=single, roi_extractor_lidar=roi([8, 16, 32, 64]), roi_extractor_img=roi([4, 8, 16, 32]),
-                test_cfg=dict(use_nms=False, max_per_img=300, post_center_range=[-61.2, -61.2, -10.0, 61.2, 61.2, 10.0]))
+                test_cfg=dict(use_nms=use_nms, max_per_img=300, post_center_range=[-61.2, -61.2, -10.0, 61.2, 61.2, 10.0],
+                              **(dict(nms_thr=0.4, use_rotate_nms=True) if use_nms else {})))
 N_STAGES = 5
 N_PROP = 900
 
@@ -147,12 +150,15 @@ def _randomize_bn(module, seed):
 class RegionFeaturePipeline:
     """kind in {'nusc','waymo','kitti'}; fusion=True adds the 6-camera image branch + fusion
     projection of srfdet_voxel_nusc_LC.  Weights: torch.manual_seed(0) random init with
-    non-trivial BatchNorm statistics (no checkpoints offline)."""
+    non-trivial BatchNorm statistics (no checkpoints offline).  use_nms=True (scope 'full'): the frame ends in the configs'
+    rotated NMS (srf_nms_bev) and returns (max_per_img, box_dim + 1) rows [box | score | label], label -1 past the count."""
 
     def __init__(self, kind='nusc', fusion=False, device='cuda', precision=None, seed=0, channels_last=True, use_graph=False,
-                 scope='path'):
+                 scope='path', use_nms=False):
         assert scope in ('path', 'full')
+        assert scope == 'full' or not use_nms, 'use_nms needs scope="full"'
         self.scope = scope
+        self.use_nms = use_nms
         self.kind, self.fusion, self.device = kind, fusion, torch.device(device)
         self.use_graph = use_graph
         self._graphs = {}
@@ -196,7 +202,7 @@ class RegionFeaturePipeline:
             cfg = backbone_cfg(kind)
             self.backbone = R.build_backbone(cfg['pts_backbone'])
             self.neck = R.build_neck(cfg['pts_neck'])
-            self.head = R.build_head(head_cfg(kind, fusion))
+            self.head = R.build_head(head_cfg(kind, fusion, use_nms=use_nms))
             init_synthetic_backbone(self.backbone, seed + 41)
             init_synthetic_backbone(self.neck, seed + 42)
             init_synthetic_head(self.head, seed + 43)
@@ -344,8 +350,9 @@ class RegionFeaturePipeline:
 
     @torch.no_grad()
     def full_chain(self, bev, dpg_img=None):
-        """dense BEV map -> SECONDCustom -> FPN -> SRFDetHead (DPG, chained stages) -> decode.
-        Returns the decoded boxes + scores; logits / boxes / pyramid in self.last."""
+        """dense BEV map -> SECONDCustom -> FPN -> SRFDetHead (DPG, chained stages) -> decode (-> NMS when use_nms).
+        Returns the decoded boxes + scores (with use_nms: the kept rows [box | score | label]); logits / boxes / pyramid
+        in self.last."""
         from .plugin.bev_backbone import nchw_to_rows, _tc_enc
         n, c, h, w = bev.shape
         feats = self.backbone.forward_rows(nchw_to_rows(bev, _tc_enc(self.precision)), n, h, w, self.precision)
@@ -355,6 +362,10 @@ class RegionFeaturePipeline:
         scores, dec = self.head.decode(logits, boxes)
         self.last = dict(pyramid=pyramid, logits=logits, boxes=boxes, scores=scores, det_boxes=dec)
         self.last_pyramid = pyramid
+        if self.use_nms:
+            nb, ns, nl, cnt = self.head._nms_decoded(scores, dec)
+            self.last['nms_count'] = cnt
+            return torch.cat([nb[0], ns[0, :, None], nl[0, :, None].float()], dim=1)      # (max_per_img, box_dim + 1)
         return torch.cat([dec[0], scores[0]], dim=1)          # (P, box_dim-1 + classes): what a caller post-processes
 
     @torch.no_grad()

@@ -73,7 +73,7 @@ class SRFDetHead(nn.Module):
             self.roi_extractor_img = build_roi_extractor(roi_extractor_img)
         self.code_weights = nn.Parameter(torch.tensor(code_weights, dtype=torch.float32), requires_grad=False)
         self.use_nms = self.test_cfg.get('use_nms', True)
-        self.nms_fn = None      # rotated NMS is third-party (mmdet3d box3d_multiclass_nms): plug it in here when use_nms=True
+        self.nms_fn = None      # optional user NMS (boxes, scores, cfg) -> (boxes, scores, labels); None: nms_bboxes (srf_nms_bev)
         self._cache = {}
         self.eval()
 
@@ -226,18 +226,46 @@ class SRFDetHead(nn.Module):
         return scores, out
 
     @torch.no_grad()
+    def nms_bboxes(self, pred_logits, pred_bboxes):
+        """use_nms=True branch of get_bboxes (:1269-1296: xywhr2xyxyr -> box3d_multiclass_nms) on the last stage, then the
+        post_center_range filter, all on device.  -> out_boxes (bs, max_per_img, dim-1), scores (bs, max_per_img),
+        labels (bs, max_per_img) int32 and counts (bs,) int32; rows past a sample's count hold a zero box, score 0 and
+        label -1.  No host synchronisation (captures into a CUDA graph)."""
+        return self._nms_decoded(*self.decode(pred_logits, pred_bboxes))
+
+    def _nms_decoded(self, scores, boxes):
+        from .nms import nms_device
+        cfg = self.test_cfg
+        if cfg.get('nms_thr') is None:
+            raise ValueError('test_cfg.use_nms=True needs test_cfg.nms_thr (the reference configs use 0.4)')
+        # Assumptions not checked against the reference source (one line each):
+        fg_scores = scores[..., :self.num_classes]          # no background column: all num_classes real classes take part
+        score_thr = cfg.get('score_thr', 0.0)               # candidates are scores > score_thr
+        rotated = cfg.get('use_rotate_nms', True)           # nms_bev (rotated) unless use_rotate_nms=False (nms_normal_bev)
+        ob, osc, olab, _, cnt = nms_device(boxes, fg_scores, score_thr, cfg['nms_thr'], rotated, cfg['max_per_img'],
+                                           cfg.get('post_center_range'))
+        return ob, osc, olab, cnt
+
+    @torch.no_grad()
     def get_bboxes(self, pred_logits, pred_bboxes, img_metas=None):
         """:1228-1340.  -> per sample [boxes (n, dim-1), scores (n,), labels (n,)]; boxes are wrapped in
-        img_metas[i]['box_type_3d'] when given."""
+        img_metas[i]['box_type_3d'] when given.  use_nms=True without a user nms_fn: nms_bboxes (one read-back of
+        the per-sample counts); a missing test_cfg.nms_thr raises ValueError here."""
+        if self.use_nms and self.nms_fn is None:
+            boxes, scores, labels, counts = self.nms_bboxes(pred_logits, pred_bboxes)
+            results = []
+            for i, n in enumerate(counts.tolist()):
+                bx = boxes[i, :n]
+                if img_metas is not None and 'box_type_3d' in img_metas[i]:
+                    bx = img_metas[i]['box_type_3d'](bx, bx.shape[-1])
+                results.append([bx, scores[i, :n], labels[i, :n].long()])
+            return results
         scores, boxes = self.decode(pred_logits, pred_bboxes)
         cfg = self.test_cfg
         results = []
         for i in range(scores.shape[0]):
             sc, bx = scores[i], boxes[i]
             if self.use_nms:
-                if self.nms_fn is None:
-                    raise NotImplementedError('test_cfg.use_nms=True needs the third-party rotated NMS: set head.nms_fn = '
-                                              'lambda boxes, scores, cfg: (boxes, scores, labels)  (e.g. mmdet3d box3d_multiclass_nms)')
                 bx, sc, labels = self.nms_fn(bx, sc, cfg)
             else:
                 sc, idx = sc.flatten(0, 1).topk(cfg['max_per_img'])

@@ -1,7 +1,7 @@
 """Micro-benchmarks of single C-ABI entry points at the production shapes of srfdet_voxel_nusc_LC
 (CUDA events on the launching stream, 512 MiB L2 flush between iterations, median of `--iters`).
 
-    python tools/bench_kernels.py [attention] [dwconv] [--iters 20]
+    python tools/bench_kernels.py [attention] [dwconv] [encoder] [nms] [frame_nms] [--iters 20]
 
 Prints one JSON line per case: {"case", "us", "gbs" (algorithmic bytes / time), "bytes"}.
 """
@@ -90,12 +90,57 @@ def bench_encoder(iters, flush):
     print(json.dumps({'case': 'encoder frame, serialised kernel time', 'ms': tot}))
 
 
-CASES = {'attention': bench_attention, 'dwconv': bench_dwconv, 'encoder': bench_encoder}
+def _full_pipe(kind, fusion, use_nms=False, use_graph=False):
+    from srfdet_b200 import synth
+    from srfdet_b200.pipeline import RegionFeaturePipeline
+    pipe = RegionFeaturePipeline(kind, fusion=fusion, scope='full', use_nms=use_nms, use_graph=use_graph)
+    pipe.calibrate(torch.as_tensor(synth.cloud(kind, 999)).cuda())
+    return pipe
+
+
+def bench_nms(iters, flush):
+    """srf_nms_bev (IoU mask + per-class scans + merge) with the configs' settings (nms_thr 0.4, rotated, 300 per image,
+    score_thr 0) on the decoded outputs of one real full frame: nusc (900 proposals, 10 classes), waymo (3 classes)."""
+    from srfdet_b200 import synth
+    from srfdet_b200.plugin.nms import nms_device
+    for kind, fusion in [('nusc', True), ('waymo', False)]:
+        pipe = _full_pipe(kind, fusion)
+        pipe.run_frame(torch.as_tensor(synth.cloud(kind, 1000)).cuda())
+        scores, boxes = pipe.last['scores'].contiguous(), pipe.last['det_boxes'].contiguous()
+        cfg = pipe.head.test_cfg
+        run = lambda: nms_device(boxes, scores, 0.0, 0.4, True, cfg['max_per_img'], cfg['post_center_range'])
+        cnt = int(run()[-1][0])
+        us = timed(run, iters, flush)
+        bs, k, n_cls = scores.shape
+        report(f'nms_bev {kind} bs{bs} P{k} cls{n_cls} (kept {cnt})', us, boxes.numel() * 4 + scores.numel() * 4)
+        del pipe
+
+
+def bench_frame_nms(iters, flush):
+    """run_frames of the nusc_LC frame (CUDA graphs, 4 frames in flight) with use_nms off and on, alternated in one
+    process; frames/s of each (L2 flushed before every step of 4 frames)."""
+    from srfdet_b200 import synth
+    clouds = [torch.as_tensor(synth.cloud('nusc', 1000 + i)).cuda() for i in range(4)]
+    pipes = {tag: _full_pipe('nusc', True, use_nms=on, use_graph=True) for tag, on in [('off', False), ('on', True)]}
+    ms = {tag: [] for tag in pipes}
+    for rep in range(6):
+        for tag, pipe in pipes.items():
+            us = timed(lambda: pipe.run_frames(clouds), iters, flush)
+            if rep:                                      # the first round captures the graphs
+                ms[tag].append(us)
+    for tag in pipes:
+        us = sorted(ms[tag])[len(ms[tag]) // 2]
+        print(json.dumps({'case': f'frame_nms nusc_LC run_frames x4, use_nms {tag}', 'us_per_step': round(us, 1),
+                          'frames_per_s': round(4 / (us * 1e-6), 1)}), flush=True)
+
+
+CASES = {'attention': bench_attention, 'dwconv': bench_dwconv, 'encoder': bench_encoder, 'nms': bench_nms, 'frame_nms': bench_frame_nms}
 
 if __name__ == '__main__':
-    args = [a for a in sys.argv[1:] if not a.startswith('--')]
     iters = int(sys.argv[sys.argv.index('--iters') + 1]) if '--iters' in sys.argv else 20
+    args = [a for i, a in enumerate(sys.argv[1:], 1) if not a.startswith('--') and sys.argv[i - 1] != '--iters']
     torch.cuda.set_device(0)
     flush = torch.empty(512 << 20, dtype=torch.uint8, device='cuda')
+    print(json.dumps({'gpu': torch.cuda.get_device_name(0)}), flush=True)
     for name in (args or list(CASES)):
         CASES[name](iters, flush)
