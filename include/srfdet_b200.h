@@ -88,6 +88,27 @@ int srf_hard_voxelize(const float* points, int32_t n, int32_t c, const srf_geom*
                       int32_t* coors, int32_t* num_points, float* mean, int32_t* point2voxel,
                       int32_t* d_voxel_num, void* ws, size_t ws_bytes, void* stream);
 
+/* Batched hard voxelization without a host read of the per-sample voxel counts: the
+ * reference voxelizes each sample alone and concatenates the valid rows (srfdet.py:218-232);
+ * here every sample writes a fixed block of block_rows rows (srf_hard_voxelize with its own
+ * d_voxel_num) and this call packs the valid rows of all blocks, in block order, in one launch.
+ * For each of the n_arrays arrays (4-byte elements): row r < min(d_counts[b], block_rows) of
+ * block b is row (b * block_rows + r) of `src` (rows src_ld elements apart); its first `width`
+ * elements go to row (sum_{j<b} min(d_counts[j], block_rows) + r) of `dst` (rows dst_ld apart).
+ * d_total (device scalar) = number of packed rows.  Output rows >= *d_total are left untouched:
+ * consumers read the count (e.g. the sparse encoder's d_n).  src and dst must not overlap.
+ * No allocation, no host synchronisation (capturable in a CUDA graph). */
+#define SRF_CONCAT_MAX_ARRAYS 4
+typedef struct srf_rows {
+  const void* src;
+  void* dst;
+  int32_t src_ld;
+  int32_t dst_ld;
+  int32_t width;
+} srf_rows;
+int srf_concat_counted_rows(const int32_t* d_counts, int32_t n_blocks, int32_t block_rows,
+                            const srf_rows* arrays_host, int32_t n_arrays, int32_t* d_total, void* stream);
+
 /* ---------------------------------------------------------------------------------- *
  * Cell index: occupancy bitmap + per-word rank over a dense (B,Z,Y,X) grid.  rank(cell)
  * enumerates occupied cells in ascending linear order, i.e. lexicographic (b,z,y,x):

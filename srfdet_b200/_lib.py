@@ -85,6 +85,10 @@ class LinearArgs(Structure):
                 ('out2', c_void_p), ('out2_enc', c_int32), ('k_splits', c_int32)]
 
 
+class Rows(Structure):
+    _fields_ = [('src', c_void_p), ('dst', c_void_p), ('src_ld', c_int32), ('dst_ld', c_int32), ('width', c_int32)]
+
+
 class Map(Structure):
     _fields_ = [('ptr', c_void_p), ('c', c_int32), ('sn', c_int64), ('sc', c_int64), ('sh', c_int64), ('sw', c_int64)]
 
@@ -114,6 +118,7 @@ PROTOTYPES = {
     'srf_hard_voxelize_ws_bytes': (c_size_t, [c_int32, c_int32, c_int32]),
     'srf_hard_voxelize': (c_int32, [c_void_p, c_int32, c_int32, POINTER(Geom), c_int32, c_int32, c_int32, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'srf_concat_counted_rows': (c_int32, [c_void_p, c_int32, c_int32, POINTER(Rows), c_int32, c_void_p, c_void_p]),
     'srf_index_bytes': (c_size_t, [c_int64]),
     'srf_index_clear': (c_int32, [c_void_p, c_int64, c_void_p]),
     'srf_index_mark': (c_int32, [c_void_p, POINTER(c_int32), c_void_p, c_int32, c_void_p, c_void_p]),

@@ -213,6 +213,44 @@ __global__ void hv_payload_kernel(const float* __restrict__ pts, int c, const in
   }
 }
 
+// ---- batched hard voxelization: compaction of per-sample blocks ---------------------------
+// Block b of every array holds counts[b] valid rows at rows [b * block_rows, ...); they land at
+// rows [sum_{j<b} counts[j], ...) of the packed output, in sample order.  Grid (x, n_blocks):
+// one CTA row per block; each CTA recomputes its block's offset from the (few) device counts.
+struct ConcatArrays {
+  const uint32_t* src[SRF_CONCAT_MAX_ARRAYS];
+  uint32_t* dst[SRF_CONCAT_MAX_ARRAYS];
+  int32_t src_ld[SRF_CONCAT_MAX_ARRAYS], dst_ld[SRF_CONCAT_MAX_ARRAYS], width[SRF_CONCAT_MAX_ARRAYS];
+  int32_t n;
+};
+
+__global__ void concat_counted_rows_kernel(const int32_t* __restrict__ counts, int n_blocks, int block_rows,
+                                           ConcatArrays a, int32_t* __restrict__ d_total) {
+  const int b = blockIdx.y;
+  __shared__ int s_off, s_cnt;
+  if (threadIdx.x == 0) {
+    int off = 0;
+    for (int j = 0; j < b; ++j) off += min(max(counts[j], 0), block_rows);
+    const int cnt = min(max(counts[b], 0), block_rows);
+    s_off = off;
+    s_cnt = cnt;
+    if (b == n_blocks - 1 && blockIdx.x == 0) *d_total = off + cnt;
+  }
+  __syncthreads();
+  const int off = s_off, cnt = s_cnt;
+  for (int k = 0; k < a.n; ++k) {
+    const int w = a.width[k];
+    const uint32_t* src = a.src[k] + (size_t)b * block_rows * a.src_ld[k];
+    uint32_t* dst = a.dst[k] + (size_t)off * a.dst_ld[k];
+    const int64_t total = (int64_t)cnt * w;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+      const int64_t r = e / w;
+      const int j = (int)(e - r * w);
+      dst[r * a.dst_ld[k] + j] = __ldg(src + r * a.src_ld[k] + j);
+    }
+  }
+}
+
 struct HvWs {
   unsigned long long* table;
   uint32_t cap;
@@ -347,6 +385,39 @@ int srf_hard_voxelize(const float* points, int32_t n, int32_t c, const srf_geom*
   if (voxels)
     hv_payload_kernel<<<launch_grid((int64_t)max_voxels * max_points * c, 256), 256, 0, st>>>(
         points, c, w.lists, max_points, d_voxel_num, voxels);
+  SRF_LAUNCH_CHECK();
+  return SRF_OK;
+}
+
+int srf_concat_counted_rows(const int32_t* d_counts, int32_t n_blocks, int32_t block_rows, const srf_rows* arrays,
+                            int32_t n_arrays, int32_t* d_total, void* stream) {
+  SRF_CHECK_ARG(d_total && arrays, "srf_concat_counted_rows: null arg");
+  SRF_CHECK_ARG(n_blocks >= 0 && n_blocks <= 65535 && block_rows > 0,
+                "srf_concat_counted_rows: need 0 <= n_blocks <= 65535 and block_rows > 0");
+  SRF_CHECK_ARG(n_arrays >= 1 && n_arrays <= SRF_CONCAT_MAX_ARRAYS, "srf_concat_counted_rows: need 1 <= n_arrays <= %d",
+                SRF_CONCAT_MAX_ARRAYS);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n_blocks == 0) {
+    SRF_CUDA(cudaMemsetAsync(d_total, 0, 4, st));
+    return SRF_OK;
+  }
+  SRF_CHECK_ARG(d_counts, "srf_concat_counted_rows: null counts");
+  ConcatArrays a;
+  a.n = n_arrays;
+  for (int k = 0; k < n_arrays; ++k) {
+    const srf_rows& r = arrays[k];
+    SRF_CHECK_ARG(r.src && r.dst && r.src != r.dst, "srf_concat_counted_rows: array %d: null or in-place", k);
+    SRF_CHECK_ARG(r.width > 0 && r.width <= r.src_ld && r.width <= r.dst_ld,
+                  "srf_concat_counted_rows: array %d: need 0 < width <= src_ld, dst_ld", k);
+    a.src[k] = (const uint32_t*)r.src;
+    a.dst[k] = (uint32_t*)r.dst;
+    a.src_ld[k] = r.src_ld;
+    a.dst_ld[k] = r.dst_ld;
+    a.width[k] = r.width;
+  }
+  const int gx = max(1, launch_grid(block_rows, 256) / n_blocks);
+  SRF_COUNT(1);
+  concat_counted_rows_kernel<<<dim3(gx, n_blocks), 256, 0, st>>>(d_counts, n_blocks, block_rows, a, d_total);
   SRF_LAUNCH_CHECK();
   return SRF_OK;
 }

@@ -12,4 +12,4 @@ from .pillar import PFNLayer, PillarFeatureNetCustom, PointPillarsScatter  # noq
 from .bev_backbone import FPN, SECONDCustom  # noqa: F401
 from .srfdet_head import SRFDetHead  # noqa: F401
 from .nms import box3d_multiclass_nms, boxes_iou_bev, nms_bev, nms_normal_bev, xywhr2xyxyr  # noqa: F401
-from .detector import SRFDetPointPath  # noqa: F401
+from .detector import SRFDet, SRFDetPointPath, SRFDetWaymo  # noqa: F401

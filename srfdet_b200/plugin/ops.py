@@ -43,24 +43,29 @@ class Voxelization(nn.Module):
                                               L.ptr(coors), L.stream_ptr()), 'srf_dynamic_voxelize')
         return coors
 
-    def hard_padded(self, points, batch_idx=-1, want_voxels=True, want_mean=False, want_p2v=False):
+    def hard_padded(self, points, batch_idx=-1, want_voxels=True, want_mean=False, want_p2v=False, out=None):
         """No host sync: outputs have max_voxels rows, the valid count stays on the device.
-        -> dict(voxels, coors, num_points, mean, point2voxel, count)"""
+        -> dict(voxels, coors, num_points, mean, point2voxel, count).  out: caller-owned contiguous
+        coors / num_points / mean / count tensors (one block of a batch buffer) written instead of
+        new ones; their row count replaces max_voxels."""
         points = points.contiguous().float()
         n, c = points.shape
         dev = points.device
         mv, T = int(self._max_voxels()), int(self.max_num_points)
         if mv <= 0:
             mv = max(n, 1)
+        if out is not None:
+            mv = out['coors'].shape[0]
         lib = L.load()
         ws = _ws(lib.srf_hard_voxelize_ws_bytes(n, T, mv), dev)
-        out = dict(
-            voxels=torch.empty((mv, T, c), dtype=torch.float32, device=dev) if want_voxels else None,
-            coors=torch.empty((mv, 3 if batch_idx < 0 else 4), dtype=torch.int32, device=dev),
-            num_points=torch.empty((mv,), dtype=torch.int32, device=dev),
-            mean=torch.empty((mv, c), dtype=torch.float32, device=dev) if want_mean else None,
-            point2voxel=torch.empty((n,), dtype=torch.int32, device=dev) if want_p2v else None,
-            count=torch.zeros((1,), dtype=torch.int32, device=dev))
+        if out is None:
+            out = dict(
+                coors=torch.empty((mv, 3 if batch_idx < 0 else 4), dtype=torch.int32, device=dev),
+                num_points=torch.empty((mv,), dtype=torch.int32, device=dev),
+                mean=torch.empty((mv, c), dtype=torch.float32, device=dev) if want_mean else None,
+                count=torch.zeros((1,), dtype=torch.int32, device=dev))
+        out = dict(out, voxels=torch.empty((mv, T, c), dtype=torch.float32, device=dev) if want_voxels else None,
+                   point2voxel=torch.empty((n,), dtype=torch.int32, device=dev) if want_p2v else None)
         L.check(lib.srf_hard_voxelize(L.ptr(points), n, c, ctypes.byref(self.geom), T, mv, batch_idx,
                                       L.ptr(out['voxels']), L.ptr(out['coors']), L.ptr(out['num_points']),
                                       L.ptr(out['mean']), L.ptr(out['point2voxel']), L.ptr(out['count']),

@@ -251,16 +251,28 @@ class SRFDetHead(nn.Module):
         """:1228-1340.  -> per sample [boxes (n, dim-1), scores (n,), labels (n,)]; boxes are wrapped in
         img_metas[i]['box_type_3d'] when given.  use_nms=True without a user nms_fn: nms_bboxes (one read-back of
         the per-sample counts); a missing test_cfg.nms_thr raises ValueError here."""
-        if self.use_nms and self.nms_fn is None:
-            boxes, scores, labels, counts = self.nms_bboxes(pred_logits, pred_bboxes)
-            results = []
-            for i, n in enumerate(counts.tolist()):
-                bx = boxes[i, :n]
-                if img_metas is not None and 'box_type_3d' in img_metas[i]:
-                    bx = img_metas[i]['box_type_3d'](bx, bx.shape[-1])
-                results.append([bx, scores[i, :n], labels[i, :n].long()])
-            return results
-        scores, boxes = self.decode(pred_logits, pred_bboxes)
+        if self.device_nms:
+            return self.format_nms(*self.nms_bboxes(pred_logits, pred_bboxes), img_metas)
+        return self.select_decoded(*self.decode(pred_logits, pred_bboxes), img_metas)
+
+    @property
+    def device_nms(self):
+        """get_bboxes post-processes with nms_bboxes (True) or from the decoded boxes (select_decoded)."""
+        return self.use_nms and self.nms_fn is None
+
+    def format_nms(self, boxes, scores, labels, counts, img_metas=None):
+        """nms_bboxes outputs -> get_bboxes' per-sample [boxes, scores, labels] (one read-back of the counts)."""
+        results = []
+        for i, n in enumerate(counts.tolist()):
+            bx = boxes[i, :n]
+            if img_metas is not None and 'box_type_3d' in img_metas[i]:
+                bx = img_metas[i]['box_type_3d'](bx, bx.shape[-1])
+            results.append([bx, scores[i, :n], labels[i, :n].long()])
+        return results
+
+    def select_decoded(self, scores, boxes, img_metas=None):
+        """decode outputs -> get_bboxes' per-sample [boxes, scores, labels]: a user nms_fn, or without NMS the top
+        max_per_img (box, class) pairs; then the post_center_range filter."""
         cfg = self.test_cfg
         results = []
         for i in range(scores.shape[0]):
