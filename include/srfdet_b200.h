@@ -489,6 +489,34 @@ int srf_nms_bev(const float* boxes, int32_t bs, int32_t k, int32_t dim, const fl
                 float iou_thr, int32_t rotated, int32_t max_num, const float post_center_range[6], void* ws, size_t ws_bytes,
                 float* out_boxes, float* out_scores, int32_t* out_labels, int32_t* out_index, int32_t* d_count, void* stream);
 
+/* ---------------------------------------------------------------------------------- *
+ * Multi-sweep point input (mmdet3d 1.0.0rc6 LoadPointsFromMultiSweeps + PointsRangeFilter): the key frame and its
+ * sweeps merged into one fixed-capacity cloud.  Source s holds cap rows of ld floats at `points` (device), of which
+ * the first clamp(d_counts[s], 0, cap) are points.  In source order, then row order, a point is dropped when
+ * SRF_SWEEP_REMOVE_CLOSE and |x| < close_radius and |y| < close_radius (raw values), or when range_host (host
+ * values, NULL = none) is given and not lo < p < hi on x, y, z (after the transform).  SRF_SWEEP_TRANSFORM:
+ * xyz = fl32(fl32(R xyz) + t) in float64 with numpy's rounding (R row-major then t: d_poses[s][12]);
+ * SRF_SWEEP_TIME_LAG: column 4 becomes d_lags[s].  Kept points are written, columns cols_host[0..n_cols) of the
+ * modified row, to consecutive rows of out (sum cap, n_cols); *d_total = their number; rows past it are NaN, which
+ * every voxelizer drops as out of range.  2 launches, no allocation, no host synchronisation: a captured call
+ * replays with new counts, poses and lags.
+ * ---------------------------------------------------------------------------------- */
+#define SRF_SWEEP_MAX_SOURCES 64
+#define SRF_SWEEP_MAX_COLS 8
+#define SRF_SWEEP_TRANSFORM 1
+#define SRF_SWEEP_TIME_LAG 2
+#define SRF_SWEEP_REMOVE_CLOSE 4
+typedef struct srf_sweep_src {
+  const float* points;
+  int32_t cap;
+  int32_t ld;
+  int32_t flags;
+} srf_sweep_src;
+size_t srf_merge_sweeps_ws_bytes(const srf_sweep_src* srcs_host, int32_t n_src);
+int srf_merge_sweeps(const srf_sweep_src* srcs_host, int32_t n_src, const int32_t* d_counts, const double* d_poses,
+                     const float* d_lags, const int32_t* cols_host, int32_t n_cols, const float range_host[6],
+                     float close_radius, float* out, int32_t* d_total, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

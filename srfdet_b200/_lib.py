@@ -89,6 +89,14 @@ class Rows(Structure):
     _fields_ = [('src', c_void_p), ('dst', c_void_p), ('src_ld', c_int32), ('dst_ld', c_int32), ('width', c_int32)]
 
 
+class SweepSrc(Structure):
+    _fields_ = [('points', c_void_p), ('cap', c_int32), ('ld', c_int32), ('flags', c_int32)]
+
+
+SWEEP_TRANSFORM, SWEEP_TIME_LAG, SWEEP_REMOVE_CLOSE = 1, 2, 4      # include/srfdet_b200.h srf_sweep_src flags
+SWEEP_MAX_SOURCES, SWEEP_MAX_COLS = 64, 8
+
+
 class Map(Structure):
     _fields_ = [('ptr', c_void_p), ('c', c_int32), ('sn', c_int64), ('sc', c_int64), ('sh', c_int64), ('sw', c_int64)]
 
@@ -189,6 +197,9 @@ PROTOTYPES = {
     'srf_nms_bev_ws_bytes': (c_size_t, [c_int32, c_int32, c_int32]),
     'srf_nms_bev': (c_int32, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_float, c_float, c_int32, c_int32,
                               POINTER(c_float), c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    'srf_merge_sweeps_ws_bytes': (c_size_t, [POINTER(SweepSrc), c_int32]),
+    'srf_merge_sweeps': (c_int32, [POINTER(SweepSrc), c_int32, c_void_p, c_void_p, c_void_p, POINTER(c_int32), c_int32,
+                                   POINTER(c_float), c_float, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

@@ -2,6 +2,8 @@
 
     python tools/infer.py CONFIG CHECKPOINT --points a.bin [b.bin ...] [--load-dim 5 --use-dim 0 1 2 3 4]
                           [--img-feats feats.npz --lidar2img l2i.npy] [--precision fp16|fp32] [--trusted] [--out results.npz]
+    python tools/infer.py CONFIG CHECKPOINT --info nuscenes_infos_val.pkl --index 0 1 2 [--data-root data/nuscenes]
+                          [--max-points 40000] [--precision fp16|fp32] [--trusted] [--out results.npz]
 """
 import argparse
 import os
@@ -12,13 +14,19 @@ import numpy as np
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..'))
 
 EPILOG = """\
-Point files are raw float32 arrays of load-dim values per point (mmdet3d LoadPointsFromFile); use-dim selects the
-columns the model reads.  Each file is one cloud, used as it is: multi-sweep aggregation (nuScenes
-LoadPointsFromMultiSweeps) and the rest of the data pipeline are not part of this tool, so pass clouds that already
-hold what the config's pipeline would have produced.  LiDAR-only configs run all clouds as one batch; camera-fusion
+--points: point files are raw float32 arrays of load-dim values per point (mmdet3d LoadPointsFromFile); use-dim selects
+the columns the model reads.  Each file is one cloud, used as it is, so pass clouds that already hold what the config's
+pipeline would have produced.  LiDAR-only configs run all clouds as one batch; camera-fusion
 configs take one cloud plus the image-neck outputs (the image backbone and neck are not built here): --img-feats is an
 .npz with one (n_cam, C, H, W) or (1, n_cam, C, H, W) float32 array per FPN level, in level order, and --lidar2img an
-(n_cam, 4, 4) .npy.  --out writes <i>.boxes_3d, <i>.scores_3d and <i>.labels_3d per sample i.
+(n_cam, 4, 4) .npy.
+--info: frames --index of an mmdet3d nuscenes_infos_*.pkl (read without running any pickled code) go through the point
+steps of the config's test_pipeline on the GPU -- LoadPointsFromFile, LoadPointsFromMultiSweeps (the key frame and its
+sweeps moved into the key frame's LiDAR frame, with the time lag column) and PointsRangeFilter -- one frame at a time
+into a fixed-capacity cloud, so one CUDA graph serves every frame.  --data-root re-roots the infos' paths at their
+samples/ or sweeps/ component; --max-points is the capacity per point file (a larger file is an error).  LiDAR-only
+configs.  The image pipeline is not part of this tool.
+--out writes <i>.boxes_3d, <i>.scores_3d and <i>.labels_3d per sample i.
 """
 
 
@@ -27,7 +35,12 @@ def main(argv=None):
                                  formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument('config', help='reference config file (plain Python with a `model` dict)')
     ap.add_argument('checkpoint', help='checkpoint file (a state dict, or a dict with a "state_dict" entry)')
-    ap.add_argument('--points', nargs='+', required=True, help='raw float32 point files')
+    src = ap.add_mutually_exclusive_group(required=True)
+    src.add_argument('--points', nargs='+', help='raw float32 point files')
+    src.add_argument('--info', help="mmdet3d nuscenes_infos_*.pkl: run the config's point pipeline on frames --index")
+    ap.add_argument('--index', type=int, nargs='+', default=[0], help='--info: frame indices (default 0)')
+    ap.add_argument('--data-root', help='--info: directory the infos\' samples/ and sweeps/ paths are re-rooted at')
+    ap.add_argument('--max-points', type=int, default=40000, help='--info: capacity per point file (default 40000)')
     ap.add_argument('--load-dim', type=int, default=5, help='float32 values per point in the files (default 5)')
     ap.add_argument('--use-dim', type=int, nargs='+', default=None, help='columns passed to the model (default: all)')
     ap.add_argument('--img-feats', help='.npz of image-neck maps, one array per level (fusion configs)')
@@ -48,6 +61,8 @@ def main(argv=None):
     keys = det.load_checkpoint(a.checkpoint, strict=True, trusted=a.trusted)
     if keys.set_aside_keys:
         print(f'checkpoint: {len(keys.set_aside_keys)} image backbone / neck entries set aside (modules not built)')
+    if a.info:
+        return run_infos(det, a)
     use_dim = a.use_dim if a.use_dim is not None else list(range(a.load_dim))
     clouds = []
     for path in a.points:
@@ -68,12 +83,40 @@ def main(argv=None):
     results = det.simple_test(clouds, metas, img_feats=img_feats)
     out = {}
     for i, (path, r) in enumerate(zip(a.points, results)):
-        b = r['pts_bbox']
-        for k in ('boxes_3d', 'scores_3d', 'labels_3d'):
-            out[f'{i}.{k}'] = b[k].numpy()
-        n = b['scores_3d'].numel()
-        top = f', top score {float(b["scores_3d"].max()):.3f}' if n else ''
-        print(f'{path}: {clouds[i].shape[0]} points, {n} boxes{top}, labels {np.bincount(b["labels_3d"].numpy()).tolist()}')
+        report(out, i, path, clouds[i].shape[0], r)
+    if a.out:
+        np.savez(a.out, **out)
+
+
+def report(out, i, name, n_points, r):
+    b = r['pts_bbox']
+    for k in ('boxes_3d', 'scores_3d', 'labels_3d'):
+        out[f'{i}.{k}'] = b[k].numpy()
+    n = b['scores_3d'].numel()
+    top = f', top score {float(b["scores_3d"].max()):.3f}' if n else ''
+    print(f'{name}: {n_points} points, {n} boxes{top}, labels {np.bincount(b["labels_3d"].numpy()).tolist()}')
+
+
+def run_infos(det, a):
+    from srfdet_b200.plugin import registry
+    from srfdet_b200.plugin.points import MultiSweepLoader, load_nuscenes_infos
+    cfg = registry.load_config(a.config)
+    if 'test_pipeline' not in cfg:
+        sys.exit(f'{a.config} has no test_pipeline: --info runs the point steps of the config\'s test_pipeline '
+                 '(use --points for clouds that are already merged)')
+    if det.bbox_head.use_img:
+        sys.exit('--info runs LiDAR-only configs (the image pipeline is not part of this tool)')
+    infos = load_nuscenes_infos(a.info, data_root=a.data_root)
+    loader = MultiSweepLoader.from_config(cfg, batch_size=1, max_points=a.max_points)
+    det.use_graph = True
+    out = {}
+    for i, idx in enumerate(a.index):
+        if not 0 <= idx < len(infos):
+            sys.exit(f'--index {idx}: {a.info} has {len(infos)} frames')
+        loader.stage([infos[idx]])
+        clouds, counts = loader()
+        results = det.simple_test(clouds, [{}])
+        report(out, i, infos[idx]['lidar_path'], int(counts[0]), results[0])
     if a.out:
         np.savez(a.out, **out)
 
