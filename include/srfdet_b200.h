@@ -193,6 +193,20 @@ int srf_pillar_vfe(const float* voxels, const int32_t* num_points, const int32_t
                    float* out, void* stream);
 int srf_pillars_scatter(const float* feats, const int32_t* coors, int32_t cap, const int32_t* d_n, int32_t c,
                         int32_t ny, int32_t nx, int32_t channels_last, float* canvas, void* stream);
+/* srf_pillar_encode_rows: srf_pillar_vfe -> srf_pillars_scatter -> srf_nchw_to_rows in one pass, bit for bit, for a
+ *   batch of n_blocks per-sample blocks as srf_hard_voxelize writes them: voxels (n_blocks, block_rows, t, c),
+ *   num_points (n_blocks, block_rows), coors (n_blocks, block_rows, 4) (b,z,y,x), d_counts (n_blocks) device counts.
+ *   Pillars are the rows v < clamp(d_counts[b], 0, block_rows) of block b; the batch index is the block index (the
+ *   b column of coors is not read); pillars whose (y, x) is off the ny x nx grid are skipped.
+ *   rows (>= n_blocks*ny*nx rows of enc_width(enc, cout) elements, enc any of SRF_F32 .. SRF_F16X2): row
+ *   (b*ny + y)*nx + x holds the PFN output of block b's pillar at (y, x), encoded like srf_nchw_to_rows (SRF_F32:
+ *   plain); every other row below n_blocks*ny*nx is zero.  Rows from n_blocks*ny*nx on (e.g. the 128-row padding of
+ *   the backbone's row buffers) are left untouched.  Same flags / weights / limits as srf_pillar_vfe, and cout <= 512.
+ *   Two launches (zero, write), no allocation, no host synchronisation (capturable in a CUDA graph). */
+int srf_pillar_encode_rows(const float* voxels, const int32_t* num_points, const int32_t* coors, const int32_t* d_counts,
+                           int32_t n_blocks, int32_t block_rows, int32_t t, int32_t c, const float* w_folded,
+                           const float* b_folded, int32_t cout, const float voxel_size_host[3], const float offsets_host[3],
+                           int32_t flags, int32_t ny, int32_t nx, int32_t enc, void* rows, void* stream);
 
 /* ---------------------------------------------------------------------------------- *
  * Rulebook: replaces spconv get_indice_pairs for SubMConv3d / SparseConv3d

@@ -146,6 +146,9 @@ PROTOTYPES = {
     'srf_pillar_vfe': (c_int32, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_int32,
                                  POINTER(c_float), POINTER(c_float), c_int32, c_void_p, c_void_p]),
     'srf_pillars_scatter': (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    'srf_pillar_encode_rows': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p,
+                                         c_void_p, c_int32, POINTER(c_float), POINTER(c_float), c_int32, c_int32, c_int32,
+                                         c_int32, c_void_p, c_void_p]),
     'srf_dense_rulebook': (c_int32, [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
     'srf_nchw_to_rows': (c_int32, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     'srf_upsample_add': (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p]),

@@ -24,30 +24,13 @@ __global__ void __launch_bounds__(256) nchw_to_rows_kernel(const float* __restri
     tile[j][tx] = (ch < c && p < hw) ? __ldg(src + (size_t)ch * hw + p) : 0.f;
   }
   __syncthreads();
-  const bool f16 = enc_is_f16(enc), split = enc_is_split(enc);
-  const int width = split ? 2 * c : c;
+  const int width = enc_is_split(enc) ? 2 * c : c;
   const int ch = c0 + 2 * tx;
 #pragma unroll
   for (int j = ty; j < 32; j += 8) {
     const int p = p0 + j;
     if (p >= hw || ch >= c) continue;
-    const float v0 = tile[2 * tx][j], v1 = tile[2 * tx + 1][j];
-    uint16_t* row = out + ((size_t)img * hw + p) * width;
-    if (ch + 1 < c && (c & 1) == 0) {
-      uint32_t h, l;
-      split16x2(f16, v0, v1, h, l);
-      *reinterpret_cast<uint32_t*>(row + ch) = h;
-      if (split) *reinterpret_cast<uint32_t*>(row + c + ch) = l;
-    } else {
-      const uint16_t h0 = pack16(f16, v0);
-      row[ch] = h0;
-      if (split) row[c + ch] = pack16(f16, v0 - unpack16(f16, h0));
-      if (ch + 1 < c) {
-        const uint16_t h1 = pack16(f16, v1);
-        row[ch + 1] = h1;
-        if (split) row[c + ch + 1] = pack16(f16, v1 - unpack16(f16, h1));
-      }
-    }
+    store_row_pair(enc, out + ((size_t)img * hw + p) * width, c, ch, tile[2 * tx][j], tile[2 * tx + 1][j]);
   }
 }
 

@@ -125,6 +125,35 @@ __device__ __forceinline__ void split16x2(bool f16, float a, float b, uint32_t& 
   lo = pack16x2(f16, a - h.x, b - h.y);
 }
 
+// Row encoder of srf_nchw_to_rows and srf_pillar_encode_rows: stores channel ch (value v0) and channel ch + 1 (v1, when
+// ch + 1 < c) of one row of c values in encoding enc.  ch is even.  SRF_F32 rows are plain; the 16-bit forms store the
+// pair as one 32-bit word (hi, then lo for the split forms) when c is even, element by element otherwise.
+__device__ __forceinline__ void store_row_pair(int enc, void* row, int c, int ch, float v0, float v1) {
+  if (enc == SRF_F32) {
+    float* r = static_cast<float*>(row);
+    r[ch] = v0;
+    if (ch + 1 < c) r[ch + 1] = v1;
+    return;
+  }
+  const bool f16 = enc_is_f16(enc), split = enc_is_split(enc);
+  uint16_t* r = static_cast<uint16_t*>(row);
+  if (ch + 1 < c && (c & 1) == 0) {
+    uint32_t h, l;
+    split16x2(f16, v0, v1, h, l);
+    *reinterpret_cast<uint32_t*>(r + ch) = h;
+    if (split) *reinterpret_cast<uint32_t*>(r + c + ch) = l;
+  } else {
+    const uint16_t h0 = pack16(f16, v0);
+    r[ch] = h0;
+    if (split) r[c + ch] = pack16(f16, v0 - unpack16(f16, h0));
+    if (ch + 1 < c) {
+      const uint16_t h1 = pack16(f16, v1);
+      r[ch + 1] = h1;
+      if (split) r[c + ch + 1] = pack16(f16, v1 - unpack16(f16, h1));
+    }
+  }
+}
+
 
 // ---------------------------------------------------------------------------------------
 // Programmatic dependent launch: a kernel launched through launch_pdl() may be scheduled while

@@ -2,7 +2,8 @@
 `model` config dict.
 
 `SRFDetPointPath`: the point-cloud side, `voxelize` (:204-247) and `extract_point_features` (:249-276) up to the
-middle encoder.  `SRFDet` / `SRFDetWaymo` (registry names of the reference, srfdet.py / srfdetwaymo.py): the whole
+middle encoder.  Pillar configs (PillarFeatureNetCustom + PointPillarsScatter) are recognised from the modules the config
+builds; `pillar_rows` takes them straight to the backbone's input rows (srf_pillar_encode_rows), with no canvas.  `SRFDet` / `SRFDetWaymo` (registry names of the reference, srfdet.py / srfdetwaymo.py): the whole
 detector above it -- point path, SECONDCustom + FPN (`pts_backbone`, `pts_neck`) and SRFDetHead (`bbox_head`) --
 with the reference's test-time call contract (`forward_test` / `simple_test`), checkpoint loading by the reference's
 attribute names and a device-resident, optionally graph-captured `infer`.  The image backbone and image neck are not
@@ -18,6 +19,7 @@ from torch import nn
 from .. import _lib as L
 from . import registry
 from .ops import Voxelization
+from .pillar import PillarFeatureNetCustom, PointPillarsScatter
 from .registry import DETECTORS, build_backbone, build_head, build_middle_encoder, build_neck, build_voxel_encoder
 from .voxel_encoder import HardSimpleVFE
 
@@ -46,6 +48,44 @@ class SRFDetPointPath(nn.Module):
     def is_dynamic(self):
         return self.pts_voxel_layer_cfg['max_num_points'] == -1
 
+    @property
+    def is_pillar(self):
+        return isinstance(self.pts_voxel_encoder, PillarFeatureNetCustom) and isinstance(self.pts_middle_encoder, PointPillarsScatter)
+
+    @torch.no_grad()
+    def hard_voxel_blocks(self, points, want_voxels=False, want_mean=False):
+        """Hard voxelization of B clouds without a host read: sample i fills block i of max_voxels rows.
+        -> dict(voxels (B, M, T, C) | None, num_points (B, M), coors (B, M, 4) bzyx, mean (B, M, C) | None,
+        count (B,) int32 device); rows past a block's count are unspecified."""
+        assert not self.is_dynamic
+        bs, c, dev = len(points), points[0].shape[1], points[0].device
+        if any(p.shape[1] != c for p in points):
+            raise ValueError('all clouds of a batch need the same number of point features')
+        mv = int(self.pts_voxel_layer._max_voxels())
+        if mv <= 0:
+            mv = max(max(p.shape[0] for p in points), 1)
+        T = int(self.pts_voxel_layer.max_num_points)
+        blk = dict(voxels=torch.empty((bs, mv, T, c), dtype=torch.float32, device=dev) if want_voxels else None,
+                   num_points=torch.empty((bs, mv), dtype=torch.int32, device=dev),
+                   coors=torch.empty((bs, mv, 4), dtype=torch.int32, device=dev),
+                   mean=torch.empty((bs, mv, c), dtype=torch.float32, device=dev) if want_mean else None,
+                   count=torch.zeros((bs,), dtype=torch.int32, device=dev))
+        for i, p in enumerate(points):
+            self.pts_voxel_layer.hard_padded(p, batch_idx=i, want_voxels=want_voxels, want_mean=want_mean,
+                                             out={k: None if v is None else v[i:i + 1] if k == 'count' else v[i]
+                                                  for k, v in blk.items()})
+        return blk
+
+    @torch.no_grad()
+    def pillar_rows(self, points, enc):
+        """Pillar configs: B clouds -> the first backbone convolution's input pixel rows in encoding enc, through
+        PillarFeatureNetCustom.encode_rows (PFN + PointPillarsScatter + row encoding in one kernel) without a host read.
+        -> (rows (>= B*ny*nx, enc_width(enc, C)), ny, nx)."""
+        blk = self.hard_voxel_blocks(points, want_voxels=True)
+        ny, nx = self.pts_middle_encoder.ny, self.pts_middle_encoder.nx
+        rows = self.pts_voxel_encoder.encode_rows(blk['voxels'], blk['num_points'], blk['coors'], blk['count'], ny, nx, enc)
+        return rows, ny, nx
+
     @torch.no_grad()
     def voxelize(self, points):
         """Reference contract (host-synchronising, like srfdet.py:204-247).
@@ -70,6 +110,16 @@ class SRFDetPointPath(nn.Module):
         synchronisation: voxel counts stay on the device end to end."""
         bs = len(points)
         if not self.is_dynamic:
+            if self.is_pillar:      # the modules' own kernels, one launch each per block with that block's device count
+                blk = self.hard_voxel_blocks(points, want_voxels=True)
+                mid = self.pts_middle_encoder
+                canvas = torch.empty((bs, self.pts_voxel_encoder.pfn_layers[0].units, mid.ny, mid.nx), device=points[0].device,
+                                     memory_format=torch.channels_last if mid.channels_last else torch.contiguous_format).zero_()
+                for i in range(bs):
+                    n = blk['count'][i:i + 1]
+                    feats = self.pts_voxel_encoder(blk['voxels'][i], blk['num_points'][i], blk['coors'][i], num_voxels=n)
+                    mid.scatter_into(canvas, feats, blk['coors'][i], num_voxels=n)
+                return canvas
             if bs == 1 and isinstance(self.pts_voxel_encoder, HardSimpleVFE):
                 o = self.pts_voxel_layer.hard_padded(points[0], batch_idx=0, want_voxels=False, want_mean=True)
                 c = self.pts_voxel_encoder.num_features
@@ -176,22 +226,12 @@ class SRFDet(SRFDetPointPath):
         block of max_voxels rows, then srf_concat_counted_rows packs the valid rows in sample order.
         -> (voxel means (B * max_voxels, num_features), coors (B * max_voxels, 4) bzyx, count (1,) int32 device);
         rows past the count are unspecified."""
-        assert not self.is_dynamic and isinstance(self.pts_voxel_encoder, HardSimpleVFE)
-        bs, c, dev = len(points), points[0].shape[1], points[0].device
-        if any(p.shape[1] != c for p in points):
-            raise ValueError('all clouds of a batch need the same number of point features')
-        mv = int(self.pts_voxel_layer._max_voxels())
-        if mv <= 0:
-            mv = max(max(p.shape[0] for p in points), 1)
+        assert isinstance(self.pts_voxel_encoder, HardSimpleVFE)
+        blk = self.hard_voxel_blocks(points, want_mean=True)
+        blk_coors, blk_mean, counts = blk['coors'], blk['mean'], blk['count']
+        bs, mv, c = blk_mean.shape
+        dev = blk_mean.device
         nf = self.pts_voxel_encoder.num_features
-        blk_coors = torch.empty((bs, mv, 4), dtype=torch.int32, device=dev)
-        blk_num = torch.empty((bs, mv), dtype=torch.int32, device=dev)
-        blk_mean = torch.empty((bs, mv, c), dtype=torch.float32, device=dev)
-        counts = torch.zeros((bs,), dtype=torch.int32, device=dev)
-        for i, p in enumerate(points):
-            self.pts_voxel_layer.hard_padded(p, batch_idx=i, want_voxels=False, want_mean=True,
-                                             out=dict(coors=blk_coors[i], num_points=blk_num[i], mean=blk_mean[i],
-                                                      count=counts[i:i + 1]))
         coors = torch.empty((bs * mv, 4), dtype=torch.int32, device=dev)
         mean = torch.empty((bs * mv, nf), dtype=torch.float32, device=dev)
         total = torch.zeros((1,), dtype=torch.int32, device=dev)
@@ -211,12 +251,18 @@ class SRFDet(SRFDetPointPath):
 
     @torch.no_grad()
     def extract_pts_feat(self, points, precision=None):
-        """points -> voxel encoder -> sparse encoder -> SECONDCustom -> FPN: list of BEV maps (B, C, H_l, W_l)."""
+        """points -> voxel encoder -> sparse encoder -> SECONDCustom -> FPN: list of BEV maps (B, C, H_l, W_l).
+        Pillar configs: points -> pillar_rows -> SECONDCustom -> FPN."""
         from .bev_backbone import _tc_enc, nchw_to_rows
         precision = precision or registry.get_precision()
-        bev = self.extract_point_features(points, precision)
-        n, _, h, w = bev.shape
-        feats = self.pts_backbone.forward_rows(nchw_to_rows(bev, _tc_enc(precision)), n, h, w, precision)
+        if self.is_pillar:
+            n = len(points)
+            rows, h, w = self.pillar_rows(points, _tc_enc(precision))
+        else:
+            bev = self.extract_point_features(points, precision)
+            n, _, h, w = bev.shape
+            rows = nchw_to_rows(bev, _tc_enc(precision))
+        feats = self.pts_backbone.forward_rows(rows, n, h, w, precision)
         return self.pts_neck.forward_rows(feats, n, precision)
 
     def extract_feat(self, points, img_feats=None, precision=None):

@@ -46,8 +46,8 @@ class Voxelization(nn.Module):
     def hard_padded(self, points, batch_idx=-1, want_voxels=True, want_mean=False, want_p2v=False, out=None):
         """No host sync: outputs have max_voxels rows, the valid count stays on the device.
         -> dict(voxels, coors, num_points, mean, point2voxel, count).  out: caller-owned contiguous
-        coors / num_points / mean / count tensors (one block of a batch buffer) written instead of
-        new ones; their row count replaces max_voxels."""
+        coors / num_points / mean / count tensors, and optionally voxels (one block of a batch buffer),
+        written instead of new ones; their row count replaces max_voxels."""
         points = points.contiguous().float()
         n, c = points.shape
         dev = points.device
@@ -64,7 +64,10 @@ class Voxelization(nn.Module):
                 num_points=torch.empty((mv,), dtype=torch.int32, device=dev),
                 mean=torch.empty((mv, c), dtype=torch.float32, device=dev) if want_mean else None,
                 count=torch.zeros((1,), dtype=torch.int32, device=dev))
-        out = dict(out, voxels=torch.empty((mv, T, c), dtype=torch.float32, device=dev) if want_voxels else None,
+        voxels = out.get('voxels')
+        if voxels is None and want_voxels:
+            voxels = torch.empty((mv, T, c), dtype=torch.float32, device=dev)
+        out = dict(out, voxels=voxels,
                    point2voxel=torch.empty((n,), dtype=torch.int32, device=dev) if want_p2v else None)
         L.check(lib.srf_hard_voxelize(L.ptr(points), n, c, ctypes.byref(self.geom), T, mv, batch_idx,
                                       L.ptr(out['voxels']), L.ptr(out['coors']), L.ptr(out['num_points']),

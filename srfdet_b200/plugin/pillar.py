@@ -59,25 +59,47 @@ class PillarFeatureNetCustom(nn.Module):
             self._folded = ((ver, str(device)), w.to(device).contiguous(), b.to(device).contiguous())
         return self._folded[1], self._folded[2]
 
-    def forward(self, features, num_points, coors, num_voxels=None):
-        """features (N, T, C) zero-padded pillars, num_points (N,), coors (N,4) (b,z,y,x) -> (N, C_out).
-        num_voxels: optional (1,) int32 device count of valid rows (no-sync path)."""
+    def _kernel_args(self, device):
+        """(folded weight, folded bias, flags word) of the fused PFN kernels."""
         if self.training:
             raise NotImplementedError('srfdet_b200 implements the inference path only')
         if len(self.pfn_layers) != 1:
             raise NotImplementedError('the fused kernel implements the single-PFNLayer form every reference config uses')
+        w, b = self._fold(device)
+        flags = int(self._with_cluster_center) | (int(self._with_voxel_center) << 1) | (int(self._with_distance) << 2) \
+            | (int(bool(self.legacy)) << 3) | (int(self.mode == 'avg') << 4)
+        return w, b, flags
+
+    def forward(self, features, num_points, coors, num_voxels=None):
+        """features (N, T, C) zero-padded pillars, num_points (N,), coors (N,4) (b,z,y,x) -> (N, C_out).
+        num_voxels: optional (1,) int32 device count of valid rows (no-sync path)."""
         features = features.contiguous().float()
         n, t, c = features.shape
         layer = self.pfn_layers[0]
-        w, b = self._fold(features.device)
+        w, b, flags = self._kernel_args(features.device)
         out = torch.empty((n, layer.units), dtype=torch.float32, device=features.device)
-        flags = int(self._with_cluster_center) | (int(self._with_voxel_center) << 1) | (int(self._with_distance) << 2) \
-            | (int(bool(self.legacy)) << 3) | (int(self.mode == 'avg') << 4)
         L.check(L.load().srf_pillar_vfe(L.ptr(features), L.ptr(num_points.contiguous().int()), L.ptr(coors.contiguous().int()), n,
                                         L.ptr(num_voxels), t, c, L.ptr(w), L.ptr(b), layer.units, L.f3([self.vx, self.vy, self.vz]),
                                         L.f3([self.x_offset, self.y_offset, self.z_offset]), flags, L.ptr(out), L.stream_ptr()),
                 'srf_pillar_vfe')
         return out
+
+    def encode_rows(self, voxels, num_points, coors, counts, ny, nx, enc):
+        """This module followed by PointPillarsScatter and the NCHW -> pixel-row encoding of the dense backbone, in one
+        kernel (srf_pillar_encode_rows) and without a canvas.  voxels (B, M, T, C), num_points (B, M), coors (B, M, 4)
+        int32: per-sample blocks of hard voxelization; counts (B,) int32 device counts of valid rows per block.
+        -> rows ((B*ny*nx + 127) // 128 * 128, enc_width(enc, C_out)) in encoding enc: row (b*ny + y)*nx + x holds the
+        features of sample b's pillar at (y, x), empty cells are zero; the rows past B*ny*nx are unspecified padding."""
+        bs, m, t, c = voxels.shape
+        layer = self.pfn_layers[0]
+        w, b, flags = self._kernel_args(voxels.device)
+        rows = torch.empty(((bs * ny * nx + 127) // 128 * 128, L.enc_width(enc, layer.units)), dtype=L.enc_torch_dtype(enc),
+                           device=voxels.device)
+        L.check(L.load().srf_pillar_encode_rows(L.ptr(voxels), L.ptr(num_points), L.ptr(coors), L.ptr(counts), bs, m, t, c,
+                                                L.ptr(w), L.ptr(b), layer.units, L.f3([self.vx, self.vy, self.vz]),
+                                                L.f3([self.x_offset, self.y_offset, self.z_offset]), flags, ny, nx, enc,
+                                                L.ptr(rows), L.stream_ptr()), 'srf_pillar_encode_rows')
+        return rows
 
 
 @MIDDLE_ENCODERS.register_module()
@@ -98,6 +120,12 @@ class PointPillarsScatter(nn.Module):
             batch_size = int(coors[:, 0].max().item()) + 1 if n else 1
         canvas = torch.empty((batch_size, c, self.ny, self.nx), dtype=torch.float32, device=voxel_features.device,
                              memory_format=torch.channels_last if self.channels_last else torch.contiguous_format).zero_()
+        return self.scatter_into(canvas, voxel_features, coors, num_voxels)
+
+    def scatter_into(self, canvas, voxel_features, coors, num_voxels=None):
+        """forward into a caller-owned zeroed canvas (B, C, ny, nx) (torch.channels_last when self.channels_last): lets a
+        batch voxelized in per-sample blocks be scattered block by block, each with its own device count."""
+        n, c = voxel_features.shape
         L.check(L.load().srf_pillars_scatter(L.ptr(voxel_features), L.ptr(coors), n, L.ptr(num_voxels), c, self.ny, self.nx,
                                              int(self.channels_last), canvas.data_ptr(), L.stream_ptr()), 'srf_pillars_scatter')
         return canvas

@@ -1,6 +1,6 @@
 """Detector-level timings (CUDA events on the launching stream, 512 MiB L2 flush between steps, median of `--iters`):
 
-    python tools/bench_detector.py [--kinds nusc waymo] [--iters 20]
+    python tools/bench_detector.py [--kinds nusc waymo pillar] [--iters 20]
 
 Per configuration (nusc_L, waymo_L; calibrated synthetic weights of RegionFeaturePipeline, production-size clouds,
 the configs' rotated NMS on) one JSON line per case:
@@ -15,6 +15,12 @@ nusc_L also times the multi-sweep point input (plugin/points.py, synthetic key f
                      clouds (stage + merge + one graph);
   replay             the same 8 frames again once every graph exists (median of --iters passes): the cost of voxelizing
                      over the capacity instead of the valid count, plus the loader's staging copies and merge.
+pillar (the restated srfdet_pillar_nusc_L config, seeded synthetic weights, rotated NMS on):
+  pillar kernel      srf_pillar_encode_rows against the chain it replaces (srf_pillar_vfe -> zeroed fp32 canvas +
+                     srf_pillars_scatter -> srf_nchw_to_rows) on the same blocks, B = 1, a 300k-point nuScenes cloud
+                     (up to 40000 pillars), fp16 rows; algorithmic bytes = pillars read (voxels, num_points, coors) +
+                     rows written, GB/s against that;
+  infer B=1/2/4      one CUDA graph over the batch, plain clouds and MultiSweepLoader clouds (stage + merge + graph).
 The first line names the GPU and its power limit.
 """
 import argparse
@@ -152,9 +158,68 @@ def bench_sweeps(det, name, prec, iters, flush):
     det.reset_graphs()
 
 
+def bench_pillar(iters, flush):
+    from srfdet_b200 import _lib as L
+    from srfdet_b200 import synth
+    from srfdet_b200.pipeline import init_synthetic_backbone, init_synthetic_head
+    from srfdet_b200.plugin import SRFDet, load_config
+    from srfdet_b200.plugin.bev_backbone import nchw_to_rows
+    from srfdet_b200.plugin.points import MultiSweepLoader, parse_test_pipeline
+    cfg = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'tests', 'golden', 'configs', 'pipeline',
+                       'srfdet_pillar_nusc_L.py')
+    det = SRFDet.from_config(cfg)
+    init_synthetic_backbone(det.pts_backbone, 1)
+    init_synthetic_backbone(det.pts_neck, 2)
+    init_synthetic_head(det.bbox_head, 3)
+    det = det.cuda()
+    name, prec = 'pillar_nusc_L', 'fp16'
+
+    def out(case, ms, frames_n, **extra):
+        print(json.dumps(dict(config=name, case=case, precision=prec, ms=round(ms, 4),
+                              frames_per_s=round(frames_n / ms * 1e3, 1) if frames_n else None, **extra)), flush=True)
+    # ---- the kernel against the chain, on the same blocks
+    cloud = torch.as_tensor(synth.cloud('nusc', 1000)).cuda()
+    blk = det.hard_voxel_blocks([cloud], want_voxels=True)
+    vfe, mid = det.pts_voxel_encoder, det.pts_middle_encoder
+    ny, nx, enc = mid.ny, mid.nx, L.F16
+    vox, num, coors, count = blk['voxels'], blk['num_points'], blk['coors'], blk['count']
+    fused = lambda: vfe.encode_rows(vox, num, coors, count, ny, nx, enc)
+
+    def chain():
+        feats = vfe(vox[0], num[0], coors[0], num_voxels=count)
+        return nchw_to_rows(mid(feats, coors[0], batch_size=1, num_voxels=count), enc)
+    n_hw = ny * nx
+    same = torch.equal(fused()[:n_hw].view(torch.int16), chain()[:n_hw].view(torch.int16))
+    m = int(count[0])
+    _, t, c = vox.shape[1:]
+    bytes_fused = m * (t * c * 4 + 4 + 16) + n_hw * L.enc_width(enc, 64) * 2
+    ms_f, ms_c = timed(fused, iters * 5, flush), timed(chain, iters * 5, flush)
+    out('pillar kernel srf_pillar_encode_rows (B=1, fp16 rows)', ms_f, 0, us=round(ms_f * 1e3, 1), pillars=m,
+        algorithmic_bytes=bytes_fused, gb_per_s=round(bytes_fused / ms_f / 1e6, 1), bit_identical_to_chain=same)
+    out('pillar chain vfe -> zeroed fp32 canvas + scatter -> nchw_to_rows (B=1, fp16 rows)', ms_c, 0, us=round(ms_c * 1e3, 1),
+        speedup_of_kernel=round(ms_c / ms_f, 2))
+    # ---- the detector with one graph per batch shape
+    det.use_graph = True
+    clouds = [torch.as_tensor(synth.cloud('nusc', 1000 + i)).cuda() for i in range(4)]
+    steps = parse_test_pipeline(load_config(cfg)['test_pipeline'])
+    rng = np.random.default_rng(9)
+    samples = [_sweep_sample(rng, 34000 + 600 * f, [34500 - 300 * f - 200 * j for j in range(10)]) for f in range(4)]
+    for b in (1, 2, 4):
+        out(f'infer B={b} (one graph, plain clouds)', timed(lambda: det.infer(clouds[:b]), iters, flush), b,
+            points=[int(x.shape[0]) for x in clouds[:b]])
+        loader = MultiSweepLoader(steps, batch_size=b, max_points=40000)
+
+        def staged():
+            loader.stage(samples[:b])
+            det.infer(loader()[0])
+        out(f'infer B={b} (one graph, loader clouds: stage + merge + graph)', timed(staged, iters, flush), b,
+            capacity=loader.capacity)
+    det.reset_graphs()
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo'], choices=['nusc', 'waymo', 'kitti'])
+    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar'])
     ap.add_argument('--iters', type=int, default=20)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -162,7 +227,10 @@ def main():
     print(json.dumps(gpu_info()), flush=True)
     flush = torch.empty(512 << 20, dtype=torch.uint8, device='cuda')
     for kind in a.kinds:
-        bench_kind(kind, a.iters, flush)
+        if kind == 'pillar':
+            bench_pillar(a.iters, flush)
+        else:
+            bench_kind(kind, a.iters, flush)
 
 
 if __name__ == '__main__':
