@@ -214,6 +214,8 @@ int srf_pillar_encode_rows(const float* voxels, const int32_t* num_points, const
  *   nbr[k * cap_out + o] = input row feeding output row o through kernel offset k
  *   (k = (kz*KH + ky)*KW + kx, input cell = o*stride - pad + k), or -1.
  *   tile_mask[o / 128] bit k set iff some row of that 128-row tile has a neighbour at k.
+ *   The conv kernels may skip offsets whose bit is clear, so a superset of this mask is also
+ *   valid; a live tile with no bit set (no row has any neighbour) yields act(bias (+ residual)).
  * in_perm (nullable) maps input rank -> caller row (first layer, unsorted input rows).
  * ---------------------------------------------------------------------------------- */
 int srf_rulebook_build(const void* in_index, const int32_t in_dims_host[4], const int32_t* in_perm,
@@ -257,7 +259,9 @@ int srf_conv3x3_last_used_tma(void);
  * and SparseConvTensor.dense() (sparse_encoder_custom.py:125-138).
  *   out[o] = act( sum_k W_k^T in[nbr[k][o]] + bias (+ residual[o]) )
  * srf_spconv_f32: SIMT FFMA, fp32 (cross-check mode; also the few-channel first layer of every
- *            mode: in f32, out in any encoding).  w (kvol, cin, cout) f32.
+ *            mode: in f32, out in any encoding).  in_dtype SRF_F32 or SRF_BF16 only (any other
+ *            encoding returns SRF_ERR_ARG); cin in [1,128], cout in {16,32,64,128}; out_dtype and
+ *            the residual's encoding: any of the five.  w (kvol, cin, cout) f32.
  * srf_spconv_tc : tcgen05/TMEM implicit GEMM, fp32 accumulate.  in_dtype SRF_BF16 | SRF_F16 (one MMA
  *            per product) or SRF_BF16X2 | SRF_F16X2 (hi + lo operands, three MMAs per product: the
  *            tensor-core form of the reference's FP32 mode).  out_dtype: the same encoding, or

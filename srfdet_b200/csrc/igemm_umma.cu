@@ -531,6 +531,9 @@ igemm_umma_kernel(const IgemmArgs a) {
       const int row = mt * 128 + warp * 32 + lane;
       const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(buf * COUT);
       if (SPARSE) {
+        // a tile whose mask has no active offset got no MMA, and its TMEM buffer still holds an older tile's
+        // accumulator (or uninitialised TMEM): its rows are act(bias + residual), so the sum is zero here
+        const bool no_mma = a.tile_mask && (((uint64_t)__ldg(a.tile_mask + mt) & all_k) == 0ull);
         // drain the accumulator in 32-column chunks (small register footprint)
         constexpr int NC = COUT < 32 ? COUT : 32;
 #pragma unroll 1
@@ -538,6 +541,10 @@ igemm_umma_kernel(const IgemmArgs a) {
           float v[NC];
 #pragma unroll
           for (int cc = 0; cc < NC; cc += 16) tc_ld16(taddr + c0 + cc, v + cc);
+          if (no_mma) {
+#pragma unroll
+            for (int c = 0; c < NC; ++c) v[c] = 0.f;
+          }
           if (row < m_rows && !DBG(8)) epilogue_chunk<COUT, NC>(a, row, nt * COUT + c0, v);
         }
         tc_fence_before();

@@ -443,6 +443,8 @@ extern "C" {
 
 int srf_spconv_f32(const srf_conv_args* a, void* stream) {
   SRF_CHECK_ARG(a && a->in && a->nbr && a->w && (a->out || a->dense), "srf_spconv_f32: null arg");
+  // the kernels read rows of 4-byte (SRF_F32) or 2-byte bf16 (SRF_BF16) elements; any other encoding would be misread
+  SRF_CHECK_ARG(a->in_dtype == SRF_F32 || a->in_dtype == SRF_BF16, "srf_spconv_f32: input features must be f32 or bf16 (got encoding %d)", a->in_dtype);
   SRF_CHECK_ARG(a->cin >= 1 && a->cin <= SIMT_MAXCIN, "srf_spconv_f32: cin must be in [1,%d]", SIMT_MAXCIN);
   SRF_CHECK_ARG(a->kvol >= 1 && a->kvol <= 27, "srf_spconv_f32: kvol must be in [1,27]");
   SRF_CHECK_ARG(a->cap_out > 0 && a->cap_out % 128 == 0, "srf_spconv_f32: cap_out must be a multiple of 128");
