@@ -535,6 +535,44 @@ int srf_merge_sweeps(const srf_sweep_src* srcs_host, int32_t n_src, const int32_
                      const float* d_lags, const int32_t* cols_host, int32_t n_cols, const float range_host[6],
                      float close_radius, float* out, int32_t* d_total, void* ws, size_t ws_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------- *
+ * Test-time augmentation (mmdet3d 1.0.0rc6 MultiScaleFlipAug3D around GlobalRotScaleTrans and RandomFlip3D, with
+ * merge_aug_bboxes_3d).  csrc/augment.cu, csrc/nms_bev.cu.  A view is (scale, flips): flip bit SRF_AUG_FLIP_HORIZONTAL
+ * negates y, SRF_AUG_FLIP_VERTICAL negates x.  Both entries take the workspace as (ws, *ws_bytes): ws = NULL stores the
+ * size they need in *ws_bytes and returns, without touching anything else.
+ * ---------------------------------------------------------------------------------- */
+#define SRF_AUG_MAX_VIEWS 32
+#define SRF_AUG_MAX_COLS 8
+#define SRF_AUG_FLIP_HORIZONTAL 1
+#define SRF_AUG_FLIP_VERTICAL 2
+#define SRF_MERGE_AUG_MAX_K 4096
+/* points (cap, n_cols) device, of which the first clamp(*d_count, 0, cap) rows are points (d_count NULL: all cap) ->
+ * n_views views out (n_views, cap, n_cols).  Per view a and row, in row order: xyz = fl32(xyz * scales_host[a]), then
+ * the flips of flips_host[a]; when range_host (host values, NULL = none) is given, a point is kept only if lo < p < hi
+ * on x, y and z (PointsRangeFilter after the augmentation).  Other columns are copied.  Kept rows are compacted stably
+ * to the front of their view; d_counts[a] = their number; rows past it are NaN.  2 launches, no allocation, no host
+ * synchronisation: a captured call replays with a new count.  3 <= n_cols <= SRF_AUG_MAX_COLS. */
+int srf_augment_points(const float* points, int32_t cap, int32_t n_cols, const int32_t* d_count, int32_t n_views,
+                       const float* scales_host, const int32_t* flips_host, const float range_host[6], float* out,
+                       int32_t* d_counts, void* ws, size_t* ws_bytes, void* stream);
+/* merge_aug_bboxes_3d per sample over n_views views of that sample's detections: boxes (bs, n_views, m, dim >= 7)
+ * rows [x, y, z, dx, dy, dz, yaw (, vx, vy)], scores (bs, n_views, m), labels (bs, n_views, m) int32, d_counts
+ * (bs, n_views): the first clamp(count, 0, m) rows of a view are detections (srf_nms_bev's outputs).  Each row is
+ * mapped back (bbox3d_mapping_back, fp32): a horizontal flip negates columns 1::7 then yaw = -yaw; a vertical flip
+ * negates columns 0::7 then yaw = fl32(-yaw + fl32(pi)); then every column but yaw is multiplied by
+ * inv_scales_host[a] (= fl32(1 / scale)).  The views are concatenated in order; per class (labels outside
+ * [0, n_cls) take no part) a greedy NMS in (score desc, concatenated position asc) order suppresses a box whose BEV
+ * IoU (srf_iou_bev; rotated = 0: axis-aligned) with a kept one is > iou_thr; the kept lists are concatenated
+ * class-major and sorted by (score desc, class-major position asc); the first min(max_num, total) are written.
+ * Outputs of capacity max_num per sample: out_boxes (bs, max_num, dim), out_scores, out_labels (bs, max_num), d_count
+ * (bs); rows past the count hold a zero box, score 0 and label -1.  n_views * m <= SRF_MERGE_AUG_MAX_K,
+ * n_views <= SRF_AUG_MAX_VIEWS and n_cls <= 32 (SRF_ERR_UNSUPPORTED otherwise).  4 launches, no host
+ * synchronisation. */
+int srf_merge_aug_bev(const float* boxes, const float* scores, const int32_t* labels, const int32_t* d_counts, int32_t bs,
+                      int32_t n_views, int32_t m, int32_t dim, const float* inv_scales_host, const int32_t* flips_host,
+                      int32_t n_cls, float iou_thr, int32_t rotated, int32_t max_num, void* ws, size_t* ws_bytes,
+                      float* out_boxes, float* out_scores, int32_t* out_labels, int32_t* d_count, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

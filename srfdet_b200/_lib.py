@@ -95,6 +95,8 @@ class SweepSrc(Structure):
 
 SWEEP_TRANSFORM, SWEEP_TIME_LAG, SWEEP_REMOVE_CLOSE = 1, 2, 4      # include/srfdet_b200.h srf_sweep_src flags
 SWEEP_MAX_SOURCES, SWEEP_MAX_COLS = 64, 8
+AUG_FLIP_HORIZONTAL, AUG_FLIP_VERTICAL = 1, 2                       # include/srfdet_b200.h srf_augment_points flips
+AUG_MAX_VIEWS, AUG_MAX_COLS, MERGE_AUG_MAX_K = 32, 8, 4096
 
 
 class Map(Structure):
@@ -203,6 +205,11 @@ PROTOTYPES = {
     'srf_merge_sweeps_ws_bytes': (c_size_t, [POINTER(SweepSrc), c_int32]),
     'srf_merge_sweeps': (c_int32, [POINTER(SweepSrc), c_int32, c_void_p, c_void_p, c_void_p, POINTER(c_int32), c_int32,
                                    POINTER(c_float), c_float, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'srf_augment_points': (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_int32, POINTER(c_float), POINTER(c_int32),
+                                     POINTER(c_float), c_void_p, c_void_p, c_void_p, POINTER(c_size_t), c_void_p]),
+    'srf_merge_aug_bev': (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, POINTER(c_float),
+                                    POINTER(c_int32), c_int32, c_float, c_int32, c_int32, c_void_p, POINTER(c_size_t), c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 SO = os.path.join(CSRC, 'libsrfdet_b200.so')
-SOURCES = ['index.cu', 'voxelize.cu', 'scatter.cu', 'spconv_simt.cu', 'igemm_umma.cu', 'spconv_warp16.cu', 'roi.cu', 'dynconv.cu', 'pillar.cu', 'head_tail.cu', 'bev_dense.cu', 'attention.cu', 'conv3x3_halo.cu', 'nms_bev.cu', 'sweeps.cu']
+SOURCES = ['index.cu', 'voxelize.cu', 'scatter.cu', 'spconv_simt.cu', 'igemm_umma.cu', 'spconv_warp16.cu', 'roi.cu', 'dynconv.cu', 'pillar.cu', 'head_tail.cu', 'bev_dense.cu', 'attention.cu', 'conv3x3_halo.cu', 'nms_bev.cu', 'sweeps.cu', 'augment.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-O2', '--expt-relaxed-constexpr']
 

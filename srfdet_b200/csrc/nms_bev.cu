@@ -21,6 +21,18 @@
 //                         candidates resolved in registers
 //   3. nms_merge_kernel   one CTA per sample: class-major concatenation, the max_num cut (stable top-k: ties keep
 //                         the class-major order), the post_center_range filter, fixed-capacity outputs + count
+//
+// srf_merge_aug_bev (mmdet3d merge_aug_bboxes_3d over the per-view results of test-time augmentation) is 4 launches
+// with a data-independent launch sequence.  Up to SRF_MERGE_AUG_MAX_K = 4096 candidates per sample (views x rows), all
+// possibly in one class: a k x k mask no longer fits shared memory, so it lives in the global workspace, in the order
+// of the candidates sorted by (class, score desc, position asc), and only tiles that hold a same-class pair are built:
+//   1. merge_aug_sort_kernel   one CTA per sample: the views' valid rows mapped back (bbox3d_mapping_back), sorted by
+//                              (class, score desc, concatenated position asc) with a bitonic sort; class segments
+//   2. merge_aug_mask_kernel   64 x 64 candidate tiles of the upper triangle: "same class and IoU > thr" bits
+//   3. merge_aug_scan_kernel   one CTA per (class, sample): greedy scan of the class segment, blocks of 64 resolved in
+//                              registers, the kept rows' mask words OR-ed into a shared removed set
+//   4. merge_aug_final_kernel  one CTA per sample: the class-major kept lists sorted by (score desc, class-major
+//                              position asc), the max_num cut, fixed-capacity outputs + count
 #include "common.cuh"
 
 namespace srf {
@@ -376,6 +388,271 @@ static NmsWs nms_ws(void* base, int bs, int k, int n_cls) {
   return w;
 }
 
+// ------------------------------------------------------------------------------------------- test-time augmentation
+constexpr int MERGE_AUG_THREADS = 1024;
+constexpr int MERGE_AUG_SCAN_THREADS = 256;
+constexpr int MERGE_AUG_MAX_WORDS = SRF_MERGE_AUG_MAX_K / 64;
+constexpr float MERGE_AUG_PI = 3.14159265358979323846f;     // fl32(pi), as torch adds np.pi to a float32 tensor
+
+struct MergeAugViews {
+  float inv_scale[SRF_AUG_MAX_VIEWS];
+  int32_t flips[SRF_AUG_MAX_VIEWS];
+};
+
+// bitonic sort of n2 (a power of two) keys in shared memory, ascending, by the whole CTA
+__device__ __forceinline__ void block_bitonic_sort(unsigned long long* keys, int n2) {
+  for (int size = 2; size <= n2; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = threadIdx.x; t < n2 / 2; t += blockDim.x) {
+        const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
+        const unsigned long long x = keys[lo], y = keys[hi];
+        if ((x > y) == ((lo & size) == 0)) {
+          keys[lo] = y;
+          keys[hi] = x;
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// key (class, score desc, position asc): class in bits 44.., ~score in bits 12..43, concatenated position in bits 0..11
+__global__ void __launch_bounds__(MERGE_AUG_THREADS) merge_aug_sort_kernel(
+    const float* __restrict__ boxes, const float* __restrict__ scores, const int* __restrict__ labels,
+    const int* __restrict__ counts, int n_views, int m, int dim, MergeAugViews views, int n_cls, int n2,
+    float* __restrict__ sbox, float* __restrict__ sscore, int* __restrict__ slab, int* __restrict__ cls_off) {
+  extern __shared__ __align__(16) unsigned long long aug_keys[];
+  __shared__ int voff[SRF_AUG_MAX_VIEWS + 1];
+  const int b = blockIdx.x, tid = threadIdx.x, k = n_views * m;
+  if (tid == 0) {
+    voff[0] = 0;
+    for (int a = 0; a < n_views; ++a) voff[a + 1] = voff[a] + min(max(counts[b * n_views + a], 0), m);
+  }
+  __syncthreads();
+  const int n = voff[n_views];
+  for (int p = tid; p < n2; p += blockDim.x) {
+    unsigned long long key = ~0ull;
+    if (p < n) {
+      int a = 0;
+      while (voff[a + 1] <= p) ++a;
+      const size_t row = ((size_t)b * n_views + a) * m + (p - voff[a]);
+      const int lab = labels[row];
+      if (lab >= 0 && lab < n_cls) key = ((unsigned long long)lab << 44) | ((unsigned long long)(~ordered_bits(scores[row])) << 12) | (unsigned)p;
+    }
+    aug_keys[p] = key;
+  }
+  __syncthreads();
+  block_bitonic_sort(aug_keys, n2);
+  for (int i = tid; i < k; i += blockDim.x) {
+    const unsigned long long key = aug_keys[i];
+    const size_t o = (size_t)b * k + i;
+    if (key == ~0ull) {
+      slab[o] = n_cls;                      // past the valid candidates: a class of its own
+      continue;
+    }
+    const int p = (int)(key & 0xfff);
+    int a = 0;
+    while (voff[a + 1] <= p) ++a;
+    const size_t row = ((size_t)b * n_views + a) * m + (p - voff[a]);
+    const bool hf = views.flips[a] & SRF_AUG_FLIP_HORIZONTAL, vf = views.flips[a] & SRF_AUG_FLIP_VERTICAL;
+    const float inv_s = views.inv_scale[a];
+    const float* src = boxes + row * dim;
+    float* dst = sbox + o * dim;
+    for (int d = 0; d < dim; ++d) {
+      float x = src[d];
+      if (d == 6) {                         // yaw: -yaw (horizontal), then -yaw + pi (vertical); not scaled
+        if (hf) x = -x;
+        if (vf) x = __fadd_rn(-x, MERGE_AUG_PI);
+      } else {                              // y / vy (columns 1::7), x / vx (columns 0::7), then * fl32(1 / scale)
+        if (hf && d % 7 == 1) x = -x;
+        if (vf && d % 7 == 0) x = -x;
+        x = __fmul_rn(x, inv_s);
+      }
+      dst[d] = x;
+    }
+    sscore[o] = scores[row];
+    slab[o] = (int)(key >> 44);
+  }
+  // class c occupies sorted positions [cls_off[c], cls_off[c + 1]); cls_off[n_cls] = number of valid candidates
+  for (int c = tid; c <= n_cls; c += blockDim.x) {
+    int lo = 0, hi = n2;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if ((int)min(aug_keys[mid] >> 44, (unsigned long long)n_cls) < c) lo = mid + 1; else hi = mid;
+    }
+    cls_off[b * (NMS_MAX_CLS + 1) + c] = min(lo, k);
+  }
+}
+
+// mask[b][i][w] bit t (sorted positions, j = 64w + t > i): same class and IoU(i, j) > thr.  Grid (W, W, bs); tiles below
+// the diagonal and tiles whose row and column class ranges are disjoint are skipped: the scan reads only same-class
+// bits, which lie in built tiles.
+__global__ void __launch_bounds__(64) merge_aug_mask_kernel(const float* __restrict__ sbox, const int* __restrict__ slab, int k,
+                                                            int dim, int n_cls, int rotated, float thr,
+                                                            unsigned long long* __restrict__ mask) {
+  __shared__ BevBox cols[64];
+  __shared__ int col_lab[64];
+  const int b = blockIdx.z, W = gridDim.x, R = blockIdx.y, C = blockIdx.x;
+  if (C < R) return;
+  const int* lab = slab + (size_t)b * k;
+  const int i0 = R * 64, j0 = C * 64;
+  const int lr0 = lab[i0], lr1 = lab[min(i0 + 63, k - 1)], lc0 = lab[j0], lc1 = lab[min(j0 + 63, k - 1)];
+  if (lr0 >= n_cls || lc0 > lr1 || lr0 > lc1) return;
+  const float* base = sbox + (size_t)b * k * dim;
+  const int nj = min(64, k - j0);
+  if ((int)threadIdx.x < nj) {
+    col_lab[threadIdx.x] = lab[j0 + threadIdx.x];
+    cols[threadIdx.x] = col_lab[threadIdx.x] < n_cls ? load_bev(base + (size_t)(j0 + threadIdx.x) * dim, rotated) : BevBox{};
+  }
+  __syncthreads();
+  const int i = i0 + threadIdx.x;
+  if (i >= k) return;
+  const int li = lab[i];
+  unsigned long long bits = 0;
+  if (li < n_cls) {
+    const BevBox r = load_bev(base + (size_t)i * dim, rotated);
+    for (int t = 0; t < nj; ++t)
+      if (j0 + t > i && col_lab[t] == li && bev_iou(r, cols[t], rotated) > thr) bits |= 1ull << t;
+  }
+  mask[((size_t)b * k + i) * W + C] = bits;
+}
+
+// one CTA per (class, sample): kept sorted positions of the class, in score order -> keep_idx[b][cls_off[c] + ...)
+__global__ void __launch_bounds__(MERGE_AUG_SCAN_THREADS) merge_aug_scan_kernel(const int* __restrict__ cls_off, int k,
+                                                                                const unsigned long long* __restrict__ mask,
+                                                                                int* __restrict__ kept_cnt, int* __restrict__ keep_idx) {
+  __shared__ unsigned long long rem_s[MERGE_AUG_MAX_WORDS], win_s[64], alive_s;
+  const int c = blockIdx.x, b = blockIdx.y, n_cls = gridDim.x, tid = threadIdx.x;
+  const int o = cls_off[b * (NMS_MAX_CLS + 1) + c], n = cls_off[b * (NMS_MAX_CLS + 1) + c + 1] - o;
+  const int W = (k + 63) / 64;
+  if (n <= 0) {
+    if (tid == 0) kept_cnt[b * n_cls + c] = 0;
+    return;
+  }
+  const int wlo = o >> 6, whi = (o + n - 1) >> 6;
+  for (int w = wlo + tid; w <= whi; w += blockDim.x) rem_s[w] = 0;
+  __syncthreads();
+  const unsigned long long* mb = mask + (size_t)b * k * W;
+  int* out = keep_idx + (size_t)b * k + o;
+  int base = 0;
+  for (int r0 = 0; r0 < n; r0 += 64) {
+    const int g0 = o + r0, nb = min(64, n - r0), w0 = g0 >> 6, sh = g0 & 63;
+    // window q: bit t = candidate r0 + q suppresses candidate r0 + t
+    if (tid < nb) {
+      const unsigned long long* row = mb + (size_t)(g0 + tid) * W;
+      unsigned long long win = row[w0] >> sh;
+      if (sh && w0 + 1 <= whi) win |= row[w0 + 1] << (64 - sh);
+      win_s[tid] = nb == 64 ? win : win & ((1ull << nb) - 1);
+    }
+    __syncthreads();
+    if (tid < 32) {
+      const int lane = tid;
+      const int q0 = lane, q1 = lane + 32;
+      const bool a0 = q0 < nb && !((rem_s[(g0 + q0) >> 6] >> ((g0 + q0) & 63)) & 1);
+      const bool a1 = q1 < nb && !((rem_s[(g0 + q1) >> 6] >> ((g0 + q1) & 63)) & 1);
+      unsigned long long alive = ((unsigned long long)__ballot_sync(0xffffffffu, a1) << 32) | __ballot_sync(0xffffffffu, a0);
+      unsigned long long todo = alive;
+      while (todo) {
+        const int q = __ffsll((long long)todo) - 1;
+        const unsigned long long later = q == 63 ? 0ull : (~0ull << (q + 1));
+        alive &= ~(win_s[q] & later);
+        todo = alive & later;
+      }
+      if ((alive >> q0) & 1) out[base + __popcll(alive & ((1ull << q0) - 1))] = g0 + q0;
+      if ((alive >> q1) & 1) out[base + __popcll(alive & ((1ull << q1) - 1))] = g0 + q1;
+      if (lane == 0) alive_s = alive;
+    }
+    __syncthreads();
+    const unsigned long long alive = alive_s;
+    base += __popcll(alive);
+    // the kept candidates' rows, words from the block's own to the segment's last, into the removed set
+    const int nw = whi - w0 + 1;
+    for (int e = tid; e < 64 * nw; e += blockDim.x) {
+      const int q = e / nw, w = w0 + e % nw;
+      if ((alive >> q) & 1) atomicOr(&rem_s[w], mb[(size_t)(g0 + q) * W + w]);
+    }
+    __syncthreads();
+  }
+  if (tid == 0) kept_cnt[b * n_cls + c] = base;
+}
+
+__global__ void __launch_bounds__(MERGE_AUG_THREADS) merge_aug_final_kernel(
+    const float* __restrict__ sbox, const float* __restrict__ sscore, const int* __restrict__ slab, int k, int dim, int n_cls,
+    int n2, const int* __restrict__ cls_off, const int* __restrict__ kept_cnt, const int* __restrict__ keep_idx, int max_num,
+    float* __restrict__ out_boxes, float* __restrict__ out_scores, int* __restrict__ out_labels, int* __restrict__ d_count) {
+  extern __shared__ __align__(16) unsigned long long aug_keys[];
+  __shared__ int off_s[NMS_MAX_CLS + 1], cnt_s[NMS_MAX_CLS], total_s;
+  const int b = blockIdx.x, tid = threadIdx.x;
+  if (tid <= n_cls) off_s[tid] = cls_off[b * (NMS_MAX_CLS + 1) + tid];
+  if (tid < n_cls) cnt_s[tid] = kept_cnt[b * n_cls + tid];
+  __syncthreads();
+  if (tid == 0) {
+    int t = 0;
+    for (int c = 0; c < n_cls; ++c) t += cnt_s[c];
+    total_s = t;
+  }
+  const int* idx = keep_idx + (size_t)b * k;
+  const float* sc = sscore + (size_t)b * k;
+  // slot t of class c's segment holds a kept candidate when t - off[c] < kept[c]; key (score desc, slot asc)
+  for (int t = tid; t < n2; t += blockDim.x) {
+    unsigned long long key = ~0ull;
+    if (t < off_s[n_cls]) {
+      const int c = slab[(size_t)b * k + t];
+      if (t - off_s[c] < cnt_s[c]) key = ((unsigned long long)(~ordered_bits(sc[idx[t]])) << 32) | (unsigned)t;
+    }
+    aug_keys[t] = key;
+  }
+  __syncthreads();
+  block_bitonic_sort(aug_keys, n2);
+  const int n_out = min(max_num, total_s);
+  for (int r = tid; r < max_num; r += blockDim.x) {
+    const size_t o = (size_t)b * max_num + r;
+    if (r < n_out) {
+      const int i = idx[(unsigned)aug_keys[r]];
+      const float* bx = sbox + ((size_t)b * k + i) * dim;
+      for (int d = 0; d < dim; ++d) out_boxes[o * dim + d] = bx[d];
+      out_scores[o] = sc[i];
+      out_labels[o] = slab[(size_t)b * k + i];
+    } else {
+      for (int d = 0; d < dim; ++d) out_boxes[o * dim + d] = 0.f;
+      out_scores[o] = 0.f;
+      out_labels[o] = -1;
+    }
+  }
+  if (tid == 0) d_count[b] = n_out;
+}
+
+struct MergeAugWs {
+  float *sbox, *sscore;
+  int *slab, *cls_off, *kept_cnt, *keep_idx;
+  unsigned long long* mask;
+  size_t bytes;
+};
+
+static MergeAugWs merge_aug_ws(void* base, int bs, int k, int dim, int n_cls) {
+  const size_t W = (size_t)(k + 63) / 64;
+  const size_t sizes[7] = {align256((size_t)bs * k * dim * 4), align256((size_t)bs * k * 4), align256((size_t)bs * k * 4),
+                           align256((size_t)bs * (NMS_MAX_CLS + 1) * 4), align256((size_t)bs * n_cls * 4),
+                           align256((size_t)bs * k * 4), align256((size_t)bs * k * W * 8)};
+  char* p = (char*)base;
+  char* q[7];
+  size_t total = 0;
+  for (int i = 0; i < 7; ++i) {
+    q[i] = p + total;
+    total += sizes[i];
+  }
+  MergeAugWs w;
+  w.sbox = (float*)q[0];
+  w.sscore = (float*)q[1];
+  w.slab = (int*)q[2];
+  w.cls_off = (int*)q[3];
+  w.kept_cnt = (int*)q[4];
+  w.keep_idx = (int*)q[5];
+  w.mask = (unsigned long long*)q[6];
+  w.bytes = total;
+  return w;
+}
+
 }  // namespace srf
 
 using namespace srf;
@@ -425,6 +702,51 @@ int srf_nms_bev(const float* boxes, int32_t bs, int32_t k, int32_t dim, const fl
                                                                r ? r[1] : 0.f, r ? r[2] : 0.f, r ? r[3] : 0.f, r ? r[4] : 0.f,
                                                                r ? r[5] : 0.f, w.cls_cnt, w.cls_idx, w.sel, out_boxes, out_scores,
                                                                out_labels, out_index, d_count);
+  SRF_LAUNCH_CHECK();
+  return SRF_OK;
+}
+
+int srf_merge_aug_bev(const float* boxes, const float* scores, const int32_t* labels, const int32_t* d_counts, int32_t bs,
+                      int32_t n_views, int32_t m, int32_t dim, const float* inv_scales_host, const int32_t* flips_host,
+                      int32_t n_cls, float iou_thr, int32_t rotated, int32_t max_num, void* ws, size_t* ws_bytes,
+                      float* out_boxes, float* out_scores, int32_t* out_labels, int32_t* d_count, void* stream) {
+  SRF_CHECK_ARG(ws_bytes && bs >= 1 && n_views >= 1 && m >= 1 && dim >= 7 && n_cls >= 1 && max_num >= 1, "srf_merge_aug_bev: bad args");
+  const int64_t k = (int64_t)n_views * m;
+  if (n_views > SRF_AUG_MAX_VIEWS || k > SRF_MERGE_AUG_MAX_K || n_cls > NMS_MAX_CLS) {
+    set_error("srf_merge_aug_bev: at most %d views, %d candidates (views x rows) and %d classes per sample (got %d, %lld, %d)",
+              SRF_AUG_MAX_VIEWS, SRF_MERGE_AUG_MAX_K, NMS_MAX_CLS, n_views, (long long)k, n_cls);
+    return SRF_ERR_UNSUPPORTED;
+  }
+  const MergeAugWs w = merge_aug_ws(ws, bs, (int)k, dim, n_cls);
+  if (!ws) {
+    *ws_bytes = w.bytes;
+    return SRF_OK;
+  }
+  SRF_CHECK_ARG(boxes && scores && labels && d_counts && inv_scales_host && flips_host && out_boxes && out_scores && out_labels && d_count,
+                "srf_merge_aug_bev: null arg");
+  SRF_CHECK_ARG(*ws_bytes >= w.bytes, "srf_merge_aug_bev: workspace of %zu B, need %zu", *ws_bytes, w.bytes);
+  MergeAugViews v;
+  for (int a = 0; a < n_views; ++a) {
+    SRF_CHECK_ARG((flips_host[a] & ~(SRF_AUG_FLIP_HORIZONTAL | SRF_AUG_FLIP_VERTICAL)) == 0,
+                  "srf_merge_aug_bev: view %d: unknown flip flags 0x%x", a, flips_host[a]);
+    v.inv_scale[a] = inv_scales_host[a];
+    v.flips[a] = flips_host[a];
+  }
+  int n2 = 64;
+  while (n2 < k) n2 <<= 1;
+  const int W = (int)((k + 63) / 64);
+  cudaStream_t st = (cudaStream_t)stream;
+  SRF_COUNT(4);
+  merge_aug_sort_kernel<<<bs, MERGE_AUG_THREADS, (size_t)n2 * 8, st>>>(boxes, scores, labels, d_counts, n_views, m, dim, v, n_cls, n2,
+                                                                       w.sbox, w.sscore, w.slab, w.cls_off);
+  SRF_LAUNCH_CHECK();
+  merge_aug_mask_kernel<<<dim3(W, W, bs), 64, 0, st>>>(w.sbox, w.slab, (int)k, dim, n_cls, rotated, iou_thr, w.mask);
+  SRF_LAUNCH_CHECK();
+  merge_aug_scan_kernel<<<dim3(n_cls, bs), MERGE_AUG_SCAN_THREADS, 0, st>>>(w.cls_off, (int)k, w.mask, w.kept_cnt, w.keep_idx);
+  SRF_LAUNCH_CHECK();
+  merge_aug_final_kernel<<<bs, MERGE_AUG_THREADS, (size_t)n2 * 8, st>>>(w.sbox, w.sscore, w.slab, (int)k, dim, n_cls, n2, w.cls_off,
+                                                                        w.kept_cnt, w.keep_idx, max_num, out_boxes, out_scores,
+                                                                        out_labels, d_count);
   SRF_LAUNCH_CHECK();
   return SRF_OK;
 }

@@ -304,30 +304,127 @@ class SRFDet(SRFDetPointPath):
             return self._infer_eager(points, img_feats, lidar2img, precision)
         key = (tuple(tuple(p.shape) for p in points), precision,
                None if img_feats is None else tuple((tuple(f.shape), f.stride()) for f in img_feats))
+        n, n_img = len(points), len(img_feats or [])
+
+        def statics():
+            return ([p.contiguous().clone() for p in points] + [torch.empty_like(f).copy_(f) for f in img_feats or []]
+                    + [None if lidar2img is None else lidar2img.clone()])
+
+        def run(*s):
+            return self._infer_eager(list(s[:n]), list(s[n:n + n_img]) if img_feats is not None else None, s[-1], precision)
+        return self._graph_call(key, statics, run, list(points) + list(img_feats or []) + [lidar2img])
+
+    def _graph_call(self, key, statics, run, inputs):
+        """run(*static inputs) captured into one CUDA graph per key (statics() makes the static copies of the inputs on
+        first use) and replayed after `inputs` are copied into them; -> run's outputs, in graph-owned buffers."""
         g = self._graphs.get(key)
         if g is None:
-            s_pts = [p.contiguous().clone() for p in points]
-            s_img = None if img_feats is None else [torch.empty_like(f).copy_(f) for f in img_feats]
-            s_l2i = None if lidar2img is None else lidar2img.clone()
+            s_in = statics()
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):          # warm-up off the capture: lazy kernel attributes, weight packing
                 for _ in range(2):
-                    self._infer_eager(s_pts, s_img, s_l2i, precision)
+                    run(*s_in)
             torch.cuda.current_stream().wait_stream(side)
             # the head memoises its img_convs outputs per input tensors: capture must record the convolutions themselves
             self.bbox_head._cache.pop('img_maps', None)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                out = self._infer_eager(s_pts, s_img, s_l2i, precision)
-            g = self._graphs[key] = (graph, s_pts, s_img, s_l2i, out)
-        graph, s_pts, s_img, s_l2i, out = g
-        for s, x in zip(s_pts + (s_img or []) + ([s_l2i] if s_l2i is not None else []),
-                        list(points) + list(img_feats or []) + ([lidar2img] if lidar2img is not None else [])):
-            if s.data_ptr() != x.data_ptr():
+                out = run(*s_in)
+            g = self._graphs[key] = (graph, s_in, out)
+        graph, s_in, out = g
+        for s, x in zip(s_in, inputs):
+            if s is not None and s.data_ptr() != x.data_ptr():
                 s.copy_(x, non_blocking=True)
         graph.replay()
         return out
+
+    # ------------------------------------------------------------------ test-time augmentation
+    def _check_aug(self):
+        """Before any device work: TTA runs LiDAR-only configs with the head's device NMS."""
+        self._check_eval()
+        if self.bbox_head.use_img:
+            raise NotImplementedError('test-time augmentation is built for LiDAR-only configs: camera fusion would need '
+                                      'flipped images and lidar2img (DESIGN.md §1)')
+        if not self.bbox_head.device_nms:
+            raise NotImplementedError('test-time augmentation merges the views\' NMS results: it needs test_cfg.use_nms=True '
+                                      'and the head\'s device NMS (no user nms_fn)')
+        if self.bbox_head.test_cfg.get('max_num') is None:
+            raise ValueError('test-time augmentation needs test_cfg.max_num (merge_aug_bboxes_3d keeps that many boxes)')
+
+    def _merge_views(self, out, bs, views):
+        """Per-view NMS outputs of a (bs * A)-cloud batch, sample-major -> merge_aug_bboxes_3d per sample."""
+        from .nms import merge_aug_device
+        boxes, scores, labels, counts = out
+        a, m = len(views), boxes.shape[1]
+        head, cfg = self.bbox_head, self.bbox_head.test_cfg
+        # Assumptions not checked against the reference source (one line each):
+        # SRFDet does not override mmdet3d's aug_test / aug_test_pts: views merged by merge_aug_bboxes_3d(test_cfg.pts).
+        # LiDARInstance3DBoxes.flip (rc6): yaw = -yaw (horizontal), yaw = -yaw + pi (vertical), with_yaw boxes.
+        # merge_aug_bboxes_3d uses nms_bev unless use_rotate_nms=False, like the head's get_bboxes.
+        return merge_aug_device(boxes.view(bs, a, m, -1), scores.view(bs, a, m), labels.view(bs, a, m), counts.view(bs, a),
+                                views, head.num_classes, cfg['nms_thr'], cfg.get('use_rotate_nms', True), cfg['max_num'])
+
+    @torch.no_grad()
+    def infer_aug(self, points, views, point_cloud_range=None, counts=None, precision=None):
+        """Test-time augmentation of B clouds on the device: every cloud becomes its augmented views (srf_augment_points:
+        scale, flips, then point_cloud_range -- the range filter of the test pipeline when it runs after the augmentation),
+        all B x A views run as one batch through the detector with the head's device NMS, and srf_merge_aug_bev maps
+        each view's boxes back and merges them per sample (mmdet3d merge_aug_bboxes_3d).  views: [(scale, horizontal flip,
+        vertical flip)] (PointAugmentation.views); duplicates are dropped first (they would only repeat detections that
+        the merge NMS removes again).  counts: (B,) int32 device numbers of valid rows (MultiSweepLoader), None: all rows.
+        -> boxes (B, max_num, dim-1), scores (B, max_num), labels (B, max_num) int32, counts (B,) int32; rows past a count
+        hold a zero box, score 0 and label -1.  No host synchronisation; use_graph=True: one graph per (shapes, views,
+        range, precision)."""
+        from .points import augment_points, distinct_views
+        self._check_aug()
+        self._check_inputs(points, None, None)
+        views = distinct_views(views)
+        if not 1 <= len(views) <= L.AUG_MAX_VIEWS:
+            raise ValueError(f'{len(views)} distinct views: 1 to {L.AUG_MAX_VIEWS} are supported')
+        precision = precision or registry.get_precision()
+        rng = None if point_cloud_range is None else [float(v) for v in point_cloud_range]
+        n = len(points)
+
+        def run(*s):
+            batch = []
+            for i, p in enumerate(s[:n]):
+                out, _ = augment_points(p, views, rng, None if s[n] is None else s[n][i:i + 1])
+                batch += list(out)
+            return self._merge_views(self._infer_eager(batch, None, None, precision), n, views)
+        inputs = list(points) + [counts]
+        if not self.use_graph:
+            return run(*inputs)
+        key = ('aug', tuple(tuple(p.shape) for p in points), tuple(views), None if rng is None else tuple(rng),
+               counts is None, precision)
+        return self._graph_call(key, lambda: [p.contiguous().clone() for p in points] + [None if counts is None else counts.clone()],
+                                run, inputs)
+
+    @torch.no_grad()
+    def aug_test(self, points, img_metas, img=None, img_feats=None, rescale=False):
+        """mmdet3d MVXTwoStageDetector.aug_test / aug_test_pts with SRFDet's head: points[a] / img_metas[a] are the
+        already augmented clouds of augmentation a, one per sample, with their metas (pcd_scale_factor,
+        pcd_horizontal_flip, pcd_vertical_flip).  All A x B clouds run as one batch, without dropping duplicates; the
+        views' NMS results are merged per sample by srf_merge_aug_bev.  -> [dict(pts_bbox=dict(boxes_3d, scores_3d,
+        labels_3d))] per sample, CPU tensors, boxes wrapped in box_type_3d when the metas give it; one read-back."""
+        self._check_aug()
+        if img is not None or img_feats is not None:
+            raise NotImplementedError('test-time augmentation is built for LiDAR-only configs')
+        a, bs = len(points), len(points[0])
+        if any(len(p) != bs for p in points) or any(len(m) != bs for m in img_metas):
+            raise ValueError('every augmentation needs the same number of clouds and metas')
+        views = []
+        for metas in img_metas:
+            v = {(float(m.get('pcd_scale_factor', 1.0)), bool(m.get('pcd_horizontal_flip', False)),
+                  bool(m.get('pcd_vertical_flip', False))) for m in metas}
+            if len(v) != 1:
+                raise ValueError(f'the samples of one augmentation have different flips / scales: {sorted(v)}')
+            views.append(v.pop())
+        clouds = [points[j][i] for i in range(bs) for j in range(a)]          # sample-major: the views of a sample together
+        self._check_inputs(clouds, None, None)
+        out = self._merge_views(self._infer_eager(clouds, None, None, registry.get_precision()), bs, views)
+        res = self.bbox_head.format_nms(*out, [m for m in img_metas[0]])
+        return [dict(pts_bbox=dict(boxes_3d=bx.to('cpu'), scores_3d=sc.cpu(), labels_3d=lb.cpu())) for bx, sc, lb in res]
 
     # ------------------------------------------------------------------ reference call contract
     @torch.no_grad()
@@ -355,7 +452,7 @@ class SRFDet(SRFDetPointPath):
         if len(points) != len(img_metas):
             raise ValueError(f'num of augmentations ({len(points)}) != num of image meta ({len(img_metas)})')
         if len(points) > 1:
-            raise NotImplementedError('test-time augmentation (aug_test) is not built: pass one augmentation')
+            return self.aug_test(points, img_metas, img=img, img_feats=img_feats, **kwargs)
         return self.simple_test(points[0], img_metas[0], img=None if img is None else img[0], img_feats=img_feats, **kwargs)
 
     def forward(self, return_loss=True, **kwargs):

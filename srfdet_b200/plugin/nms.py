@@ -6,6 +6,8 @@ ties between equal scores keep the lower box index (the reference's sorts leave 
 `nms_device` is the graph-capturable core shared with SRFDetHead.nms_bboxes; the drop-ins read the kept count back
 to the host, as their variable-length results require.
 """
+import ctypes
+
 import torch
 
 from .. import _lib as L
@@ -33,6 +35,34 @@ def nms_device(boxes, scores, score_thr, iou_thr, rotated, max_num, post_center_
                             int(max_num), rng, L.ptr(ws), ws.numel(), L.ptr(ob), L.ptr(osc), L.ptr(olab), L.ptr(oidx), L.ptr(cnt),
                             L.stream_ptr()), 'srf_nms_bev')
     return ob, osc, olab, oidx, cnt
+
+
+def merge_aug_device(boxes, scores, labels, counts, views, n_cls, iou_thr, rotated, max_num):
+    """srf_merge_aug_bev (mmdet3d merge_aug_bboxes_3d per sample): boxes (bs, A, m, dim), scores (bs, A, m), labels
+    (bs, A, m) int32 and counts (bs, A) int32 of A views, views [(scale, horizontal, vertical)] in concatenation order.
+    -> out_boxes (bs, max_num, dim), out_scores (bs, max_num), out_labels (bs, max_num) int32, counts (bs,) int32; rows past
+    the count: zero box, score 0, label -1.  No host synchronisation."""
+    boxes, scores = boxes.float().contiguous(), scores.float().contiguous()
+    labels, counts = labels.int().contiguous(), counts.int().contiguous()
+    bs, a, m, dim = boxes.shape
+    assert scores.shape == labels.shape == (bs, a, m) and counts.shape == (bs, a) and len(views) == a
+    lib = L.load()
+    inv = (ctypes.c_float * a)(*[1.0 / float(s) for s, _, _ in views])      # fl32(1 / scale): Python double, then fp32
+    flips = (ctypes.c_int32 * a)(*[(L.AUG_FLIP_HORIZONTAL if h else 0) | (L.AUG_FLIP_VERTICAL if v else 0) for _, h, v in views])
+    need = ctypes.c_size_t(0)
+    args = (bs, a, m, dim, inv, flips, int(n_cls), float(iou_thr), int(bool(rotated)), int(max_num))
+    L.check(lib.srf_merge_aug_bev(None, None, None, None, *args, None, ctypes.byref(need), None, None, None, None, None),
+            'srf_merge_aug_bev')
+    dev = boxes.device
+    ws = torch.empty(int(need.value), dtype=torch.uint8, device=dev)
+    ob = torch.empty((bs, max_num, dim), dtype=torch.float32, device=dev)
+    osc = torch.empty((bs, max_num), dtype=torch.float32, device=dev)
+    olab = torch.empty((bs, max_num), dtype=torch.int32, device=dev)
+    cnt = torch.empty((bs,), dtype=torch.int32, device=dev)
+    L.check(lib.srf_merge_aug_bev(L.ptr(boxes), L.ptr(scores), L.ptr(labels), L.ptr(counts), *args, L.ptr(ws),
+                                  ctypes.byref(ctypes.c_size_t(ws.numel())), L.ptr(ob), L.ptr(osc), L.ptr(olab), L.ptr(cnt),
+                                  L.stream_ptr()), 'srf_merge_aug_bev')
+    return ob, osc, olab, cnt
 
 
 def xywhr2xyxyr(boxes_xywhr):

@@ -50,28 +50,53 @@ def _is_identity_rot_scale_trans(step):
     return rot == [0, 0] and scale == [1, 1] and trans == [0, 0, 0] and not step.get('shift_height', False)
 
 
+def _point_step(step, acc):
+    """LoadPointsFromFile / LoadPointsFromMultiSweeps / PointsRangeFilter into acc ('load', 'sweeps', 'pcr');
+    -> True when the step was one of them."""
+    t = step['type']
+    if t == 'LoadPointsFromFile':
+        if step.get('shift_height', False) or step.get('use_color', False):
+            raise NotImplementedError('LoadPointsFromFile: shift_height / use_color are not supported')
+        acc['load'] = (int(step.get('load_dim', 6)), _as_dims(step.get('use_dim', [0, 1, 2])))
+    elif t == 'LoadPointsFromMultiSweeps':
+        sweeps = {k: step.get(k, v) for k, v in _SWEEP_DEFAULTS.items()}
+        sweeps['use_dim'] = _as_dims(sweeps['use_dim'])
+        acc['sweeps'] = sweeps
+    elif t == 'PointsRangeFilter':
+        acc['pcr'] = [float(v) for v in step['point_cloud_range']]
+    else:
+        return False
+    return True
+
+
+def _point_steps(acc):
+    load, sweeps, pcr = acc['load'], acc['sweeps'], acc['pcr']
+    if load is None:
+        raise ValueError('the test pipeline has no LoadPointsFromFile step')
+    if load[1][:3] != [0, 1, 2] or (sweeps and sweeps['use_dim'][:3] != [0, 1, 2]):
+        raise NotImplementedError('use_dim must start with the coordinates 0, 1, 2')
+    if sweeps and len(load[1]) != sweeps['load_dim']:
+        raise ValueError(f'LoadPointsFromFile keeps {len(load[1])} columns but LoadPointsFromMultiSweeps loads '
+                         f'{sweeps["load_dim"]}: the reference concatenates them, so they must agree')
+    if sweeps and sweeps['load_dim'] < 5:
+        raise ValueError('LoadPointsFromMultiSweeps writes the time lag into column 4: load_dim must be >= 5')
+    return PointSteps(load[0], load[1], sweeps, pcr)
+
+
 def parse_test_pipeline(pipeline):
     """-> PointSteps of a config's `test_pipeline` (a list of step dicts).  MultiScaleFlipAug3D's transforms are searched
     too.  Steps that leave the points bit-identical at test time are accepted: MultiScaleFlipAug3D(flip=False,
     pts_scale_ratio=1), GlobalRotScaleTrans(rot_range=[0, 0], scale_ratio_range=[1, 1], translation_std=[0, 0, 0]) and
     RandomFlip3D inside MultiScaleFlipAug3D(flip=False).  Image and formatting steps are ignored; any other step or
-    setting raises NotImplementedError naming it."""
-    load, sweeps, pcr = None, None, None
+    setting raises NotImplementedError naming it.  Test-time augmentation: parse_test_augmentations."""
+    acc = dict(load=None, sweeps=None, pcr=None)
 
     def walk(steps, in_noflip_aug):
-        nonlocal load, sweeps, pcr
         for step in steps:
             t = step['type']
-            if t == 'LoadPointsFromFile':
-                if step.get('shift_height', False) or step.get('use_color', False):
-                    raise NotImplementedError('LoadPointsFromFile: shift_height / use_color are not supported')
-                load = (int(step.get('load_dim', 6)), _as_dims(step.get('use_dim', [0, 1, 2])))
-            elif t == 'LoadPointsFromMultiSweeps':
-                sweeps = {k: step.get(k, v) for k, v in _SWEEP_DEFAULTS.items()}
-                sweeps['use_dim'] = _as_dims(sweeps['use_dim'])
-            elif t == 'PointsRangeFilter':
-                pcr = [float(v) for v in step['point_cloud_range']]
-            elif t == 'MultiScaleFlipAug3D':
+            if _point_step(step, acc):
+                continue
+            if t == 'MultiScaleFlipAug3D':
                 ratio = step.get('pts_scale_ratio', 1)
                 ratio = list(ratio) if isinstance(ratio, (list, tuple)) else [ratio]
                 if step.get('flip', False) or ratio != [1]:
@@ -90,16 +115,107 @@ def parse_test_pipeline(pipeline):
                 raise NotImplementedError(f'{t}: this test-pipeline step is not supported by the point loader')
 
     walk(pipeline, False)
-    if load is None:
-        raise ValueError('the test pipeline has no LoadPointsFromFile step')
-    if load[1][:3] != [0, 1, 2] or (sweeps and sweeps['use_dim'][:3] != [0, 1, 2]):
-        raise NotImplementedError('use_dim must start with the coordinates 0, 1, 2')
-    if sweeps and len(load[1]) != sweeps['load_dim']:
-        raise ValueError(f'LoadPointsFromFile keeps {len(load[1])} columns but LoadPointsFromMultiSweeps loads '
-                         f'{sweeps["load_dim"]}: the reference concatenates them, so they must agree')
-    if sweeps and sweeps['load_dim'] < 5:
-        raise ValueError('LoadPointsFromMultiSweeps writes the time lag into column 4: load_dim must be >= 5')
-    return PointSteps(load[0], load[1], sweeps, pcr)
+    return _point_steps(acc)
+
+
+IDENTITY_VIEW = (1.0, False, False)
+
+
+class PointAugmentation(collections.namedtuple('PointAugmentation', ['steps', 'views', 'range_position'])):
+    """Test-time augmentation of a config's `test_pipeline` (parse_test_augmentations).
+    steps: the single-view PointSteps (point_cloud_range: the PointsRangeFilter's range wherever it sits);
+    views: [(pcd_scale_factor, horizontal flip, vertical flip)] in MultiScaleFlipAug3D's order, duplicates included;
+    range_position: 'before' or 'after' the augmentation, None without a range filter."""
+    __slots__ = ()
+
+    @property
+    def loader_steps(self):
+        """Steps of the point loader: without the range filter when it runs after the augmentation
+        (srf_augment_points applies it to each view)."""
+        return self.steps._replace(point_cloud_range=None) if self.range_position == 'after' else self.steps
+
+    @property
+    def view_range(self):
+        """The range srf_augment_points tests each view against, or None."""
+        return self.steps.point_cloud_range if self.range_position == 'after' else None
+
+    @property
+    def augments(self):
+        """The reference runs aug_test (more than one view, or one that changes the points)."""
+        return list(self.views) != [IDENTITY_VIEW]
+
+
+def distinct_views(views):
+    """The distinct views in first-occurrence order."""
+    return list(dict.fromkeys((float(s), bool(h), bool(v)) for s, h, v in views))
+
+
+def parse_test_augmentations(pipeline):
+    """-> PointAugmentation of a config's `test_pipeline`, with mmdet3d 1.0.0rc6's MultiScaleFlipAug3D expansion: loops
+    img_scale -> pts_scale_ratio (a list) -> flip in [False, True] if flip else [False] -> pcd_horizontal_flip in
+    [False, True] if flip and pcd_horizontal_flip else [False] -> the same for pcd_vertical_flip -> flip_direction.
+    RandomFlip3D with sync_2d=True (its default) flips horizontally when `flip` and never vertically; with
+    sync_2d=False it takes the wrapper's pcd flags.  Inside the wrapper GlobalRotScaleTrans must have the identity
+    rotation and translation (its scale_ratio_range is ignored: the wrapper sets pcd_scale_factor).  NotImplementedError
+    for scale ratios other than 1 without GlobalRotScaleTrans and for flip=True without RandomFlip3D (the reference would
+    map boxes back that were never augmented), and for the steps parse_test_pipeline refuses."""
+    acc = dict(load=None, sweeps=None, pcr=None)
+    aug, state = None, dict(range_position=None, augmenting_seen=False, scale=False, flip3d=None)
+
+    def walk(steps, in_aug):
+        nonlocal aug
+        for step in steps:
+            t = step['type']
+            if _point_step(step, acc):
+                if t == 'PointsRangeFilter':
+                    state['range_position'] = 'after' if state['augmenting_seen'] else 'before'
+                continue
+            if t == 'MultiScaleFlipAug3D':
+                if aug is not None:
+                    raise NotImplementedError('MultiScaleFlipAug3D: one wrapper per test pipeline is supported')
+                aug = step
+                walk(step['transforms'], True)
+            elif t == 'GlobalRotScaleTrans':
+                if not in_aug:
+                    if not _is_identity_rot_scale_trans(step):
+                        raise NotImplementedError(f'GlobalRotScaleTrans outside MultiScaleFlipAug3D: only the identity is '
+                                                  f'supported, got {step}')
+                    continue
+                if not _is_identity_rot_scale_trans(dict(step, scale_ratio_range=[1, 1])):
+                    raise NotImplementedError(f'GlobalRotScaleTrans: only the identity rotation and translation (rot_range='
+                                              f'[0, 0], translation_std=[0, 0, 0]) are supported, got {step}')
+                state['scale'] = state['augmenting_seen'] = True
+            elif t == 'RandomFlip3D':
+                if not in_aug:
+                    raise NotImplementedError('RandomFlip3D is supported only inside MultiScaleFlipAug3D')
+                state['flip3d'] = step
+                state['augmenting_seen'] = True
+            elif t not in _IGNORED:
+                raise NotImplementedError(f'{t}: this test-pipeline step is not supported by the point loader')
+
+    walk(pipeline, False)
+    steps = _point_steps(acc)
+    if aug is None:
+        return PointAugmentation(steps, [IDENTITY_VIEW], state['range_position'])
+    ratio = aug.get('pts_scale_ratio', 1)
+    ratios = [float(r) for r in ratio] if isinstance(ratio, (list, tuple)) else [float(ratio)]
+    flip = bool(aug.get('flip', False))
+    if any(r != 1 for r in ratios) and not state['scale']:
+        raise NotImplementedError(f'MultiScaleFlipAug3D(pts_scale_ratio={ratio}) without GlobalRotScaleTrans in its '
+                                  'transforms: the points would not be scaled while the boxes are mapped back')
+    if flip and state['flip3d'] is None:
+        raise NotImplementedError('MultiScaleFlipAug3D(flip=True) without RandomFlip3D in its transforms: the points would '
+                                  'not be flipped while the boxes are mapped back')
+    img_scale, direction = aug.get('img_scale'), aug.get('flip_direction', 'horizontal')
+    n_img = len(img_scale) if isinstance(img_scale, list) else 1
+    n_dir = len(direction) if isinstance(direction, list) else 1
+    hs = [False, True] if flip and aug.get('pcd_horizontal_flip', False) else [False]
+    vs = [False, True] if flip and aug.get('pcd_vertical_flip', False) else [False]
+    sync_2d = state['flip3d'] is None or state['flip3d'].get('sync_2d', True)
+    views = [(s, f, False) if sync_2d else (s, h, v)
+             for _ in range(n_img) for s in ratios for f in ([False, True] if flip else [False]) for h in hs for v in vs
+             for _ in range(n_dir)]
+    return PointAugmentation(steps, views, state['range_position'])
 
 
 def choose_sweeps(n_sweeps, sweeps_num, test_mode):
@@ -317,3 +433,26 @@ class MultiSweepLoader:
                                          d['out'][b].data_ptr(), d['total'][b:b + 1].data_ptr(), self._ws[b].data_ptr(),
                                          self._ws.shape[1], L.stream_ptr()), 'srf_merge_sweeps')
         return [d['out'][b] for b in range(self.batch_size)], d['total']
+
+
+def augment_points(points, views, point_cloud_range=None, count=None):
+    """srf_augment_points: one (cap, C) float32 CUDA cloud (first `count` rows valid, a (1,) int32 device tensor; None:
+    all) -> (views (A, cap, C), counts (A,) int32 device).  View a = views[a] = (scale, horizontal, vertical): xyz scaled
+    in float32, y negated (horizontal), x negated (vertical), then the strict point_cloud_range test when given; kept
+    rows first in row order, NaN rows after.  No host synchronisation."""
+    pts = points.float().contiguous()
+    cap, c = pts.shape
+    n = len(views)
+    lib = L.load()
+    scales = (ctypes.c_float * n)(*[float(s) for s, _, _ in views])
+    flips = (ctypes.c_int32 * n)(*[(L.AUG_FLIP_HORIZONTAL if h else 0) | (L.AUG_FLIP_VERTICAL if v else 0) for _, h, v in views])
+    need = ctypes.c_size_t(0)
+    L.check(lib.srf_augment_points(None, cap, c, None, n, scales, flips, None, None, None, None, ctypes.byref(need), None),
+            'srf_augment_points')
+    ws = torch.empty(max(int(need.value), 1), dtype=torch.uint8, device=pts.device)
+    out = torch.empty((n, cap, c), dtype=torch.float32, device=pts.device)
+    counts = torch.empty((n,), dtype=torch.int32, device=pts.device)
+    rng = L.f6(point_cloud_range) if point_cloud_range is not None else None
+    L.check(lib.srf_augment_points(L.ptr(pts), cap, c, L.ptr(count), n, scales, flips, rng, L.ptr(out), L.ptr(counts),
+                                   L.ptr(ws), ctypes.byref(ctypes.c_size_t(ws.numel())), L.stream_ptr()), 'srf_augment_points')
+    return out, counts

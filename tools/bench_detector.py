@@ -1,6 +1,6 @@
 """Detector-level timings (CUDA events on the launching stream, 512 MiB L2 flush between steps, median of `--iters`):
 
-    python tools/bench_detector.py [--kinds nusc waymo pillar] [--iters 20]
+    python tools/bench_detector.py [--kinds nusc waymo pillar tta] [--iters 20]
 
 Per configuration (nusc_L, waymo_L; calibrated synthetic weights of RegionFeaturePipeline, production-size clouds,
 the configs' rotated NMS on) one JSON line per case:
@@ -21,6 +21,10 @@ pillar (the restated srfdet_pillar_nusc_L config, seeded synthetic weights, rota
                      (up to 40000 pillars), fp16 rows; algorithmic bytes = pillars read (voxels, num_points, coors) +
                      rows written, GB/s against that;
   infer B=1/2/4      one CUDA graph over the batch, plain clouds and MultiSweepLoader clouds (stage + merge + graph).
+tta (nusc_L weights as above, the restated double-flip config's range; one 300k-point cloud):
+  infer_aug B=1      one CUDA graph over augment + the views' batch + merge, at 1, 2 and 4 distinct flip views, next to
+                     plain infer on the same cloud (frames/s);
+  kernels            srf_augment_points (4 views) and srf_merge_aug_bev (8 views x 300 rows, 10 classes) alone (us).
 The first line names the GPU and its power limit.
 """
 import argparse
@@ -217,9 +221,48 @@ def bench_pillar(iters, flush):
     det.reset_graphs()
 
 
+def bench_tta(iters, flush):
+    from srfdet_b200 import synth
+    from srfdet_b200.pipeline import RegionFeaturePipeline, backbone_cfg, head_cfg, MODEL_CFG
+    from srfdet_b200.plugin import SRFDet
+    from srfdet_b200.plugin.nms import merge_aug_device
+    from srfdet_b200.plugin.points import augment_points
+    pipe = RegionFeaturePipeline('nusc', fusion=False, scope='full', use_nms=True)
+    pipe.calibrate(torch.as_tensor(synth.cloud('nusc', 44)).cuda())
+    head = head_cfg('nusc', False, use_nms=True)
+    test_cfg = dict(pts=dict(head.pop('test_cfg'), max_num=500))
+    det = SRFDet(**MODEL_CFG['nusc'], **backbone_cfg('nusc'), bbox_head=head, test_cfg=test_cfg, use_graph=True).cuda()
+    sd = dict(pipe.detector.state_dict())
+    for prefix, m in (('pts_backbone.', pipe.backbone), ('pts_neck.', pipe.neck), ('bbox_head.', pipe.head)):
+        sd.update({prefix + k: v for k, v in m.state_dict().items()})
+    det.load_checkpoint(sd)
+    name, prec = 'nusc_L', pipe.precision
+    pcr = [-55.2, -55.2, -5.0, 55.2, 55.2, 3.0]
+    cloud = torch.as_tensor(synth.cloud('nusc', 1000)).cuda()
+
+    def out(case, ms, frames_n, **extra):
+        print(json.dumps(dict(config=name, case=case, precision=prec, ms=round(ms, 4),
+                              frames_per_s=round(frames_n / ms * 1e3, 1) if frames_n else None, **extra)), flush=True)
+    out('infer B=1 (one graph, no augmentation)', timed(lambda: det.infer([cloud]), iters, flush), 1, points=int(cloud.shape[0]))
+    flips = [(1.0, False, False), (1.0, True, False), (1.0, False, True), (1.0, True, True)]
+    for a in (1, 2, 4):
+        out(f'infer_aug B=1, {a} distinct views (one graph: augment + batch of {a} + merge)',
+            timed(lambda: det.infer_aug([cloud], flips[:a], pcr), iters, flush), 1)
+    ms = timed(lambda: augment_points(cloud, flips, pcr), iters * 5, flush)
+    out('kernel srf_augment_points (4 views)', ms, 0, us=round(ms * 1e3, 1), input_rows=int(cloud.shape[0]),
+        algorithmic_bytes=int(cloud.numel() * 4 * (1 + 4)))
+    views = [cloud] + [augment_points(cloud, [v], pcr)[0][0] for v in flips[1:]]
+    b, s, l, c = [t.clone() for t in det.infer(views)]
+    b8, s8, l8, c8 = b.repeat(2, 1, 1)[None], s.repeat(2, 1)[None], l.repeat(2, 1)[None], c.repeat(2)[None]
+    ms = timed(lambda: merge_aug_device(b8, s8, l8, c8, flips * 2, det.bbox_head.num_classes, 0.4, True, 500), iters * 5, flush)
+    out('kernel srf_merge_aug_bev (8 views x 300 rows, 10 classes)', ms, 0, us=round(ms * 1e3, 1),
+        candidates=int(c8.sum()))
+    det.reset_graphs()
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar'])
+    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar', 'tta'])
     ap.add_argument('--iters', type=int, default=20)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -229,6 +272,8 @@ def main():
     for kind in a.kinds:
         if kind == 'pillar':
             bench_pillar(a.iters, flush)
+        elif kind == 'tta':
+            bench_tta(a.iters, flush)
         else:
             bench_kind(kind, a.iters, flush)
 

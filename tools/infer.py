@@ -26,6 +26,10 @@ sweeps moved into the key frame's LiDAR frame, with the time lag column) and Poi
 into a fixed-capacity cloud, so one CUDA graph serves every frame.  --data-root re-roots the infos' paths at their
 samples/ or sweeps/ component; --max-points is the capacity per point file (a larger file is an error).  LiDAR-only
 configs.  The image pipeline is not part of this tool.
+Test-time augmentation: when the config's test_pipeline augments (MultiScaleFlipAug3D with flip=True or scale ratios
+other than 1), --info and --points run SRFDet.infer_aug with its distinct views -- the clouds flipped and scaled on the
+GPU, all views as one batch, the views' boxes mapped back and merged by class-wise rotated BEV NMS
+(merge_aug_bboxes_3d, test_cfg.max_num boxes) -- one CUDA graph for the whole --info sequence.  LiDAR-only configs.
 --out writes <i>.boxes_3d, <i>.scores_3d and <i>.labels_3d per sample i.
 """
 
@@ -80,7 +84,11 @@ def main(argv=None):
         img_feats = [torch.as_tensor(z[k]).float().cuda() for k in z.files]
         img_feats = [f.unsqueeze(0) if f.dim() == 4 else f for f in img_feats]
         metas[0]['lidar2img'] = np.load(a.lidar2img)
-    results = det.simple_test(clouds, metas, img_feats=img_feats)
+    aug = test_augmentation(a.config)
+    if aug is not None:
+        results = aug_results(det, det.infer_aug(clouds, aug.views, aug.view_range))
+    else:
+        results = det.simple_test(clouds, metas, img_feats=img_feats)
     out = {}
     for i, (path, r) in enumerate(zip(a.points, results)):
         report(out, i, path, clouds[i].shape[0], r)
@@ -97,6 +105,30 @@ def report(out, i, name, n_points, r):
     print(f'{name}: {n_points} points, {n} boxes{top}, labels {np.bincount(b["labels_3d"].numpy()).tolist()}')
 
 
+def test_augmentation(config):
+    """PointAugmentation of the config's test_pipeline when it augments (flip=True or scale ratios other than 1), else
+    None."""
+    from srfdet_b200.plugin import registry
+    from srfdet_b200.plugin.points import parse_test_augmentations
+    cfg = registry.load_config(config)
+
+    def augments(steps):
+        for st in steps:
+            if st.get('type') == 'MultiScaleFlipAug3D':
+                r = st.get('pts_scale_ratio', 1)
+                if st.get('flip', False) or (list(r) if isinstance(r, (list, tuple)) else [r]) != [1]:
+                    return True
+        return False
+    if not augments(cfg.get('test_pipeline') or []):
+        return None
+    return parse_test_augmentations(cfg['test_pipeline'])
+
+
+def aug_results(det, out):
+    """infer_aug outputs -> simple_test-style results (one read-back)."""
+    return [dict(pts_bbox=dict(boxes_3d=bx.cpu(), scores_3d=sc.cpu(), labels_3d=lb.cpu())) for bx, sc, lb in det.bbox_head.format_nms(*out)]
+
+
 def run_infos(det, a):
     from srfdet_b200.plugin import registry
     from srfdet_b200.plugin.points import MultiSweepLoader, load_nuscenes_infos
@@ -107,7 +139,11 @@ def run_infos(det, a):
     if det.bbox_head.use_img:
         sys.exit('--info runs LiDAR-only configs (the image pipeline is not part of this tool)')
     infos = load_nuscenes_infos(a.info, data_root=a.data_root)
-    loader = MultiSweepLoader.from_config(cfg, batch_size=1, max_points=a.max_points)
+    aug = test_augmentation(a.config)
+    if aug is not None:
+        loader = MultiSweepLoader(aug.loader_steps, batch_size=1, max_points=a.max_points)
+    else:
+        loader = MultiSweepLoader.from_config(cfg, batch_size=1, max_points=a.max_points)
     det.use_graph = True
     out = {}
     for i, idx in enumerate(a.index):
@@ -115,7 +151,10 @@ def run_infos(det, a):
             sys.exit(f'--index {idx}: {a.info} has {len(infos)} frames')
         loader.stage([infos[idx]])
         clouds, counts = loader()
-        results = det.simple_test(clouds, [{}])
+        if aug is not None:
+            results = aug_results(det, det.infer_aug(clouds, aug.views, aug.view_range, counts=counts))
+        else:
+            results = det.simple_test(clouds, [{}])
         report(out, i, infos[idx]['lidar_path'], int(counts[0]), results[0])
     if a.out:
         np.savez(a.out, **out)
