@@ -419,11 +419,16 @@ int srf_bev_roi_features(const srf_pyramid* p_host, float* boxes, int32_t batch,
                          int32_t box_dim, const float pc_range_host[6], const float voxel_size_host[3],
                          int32_t mutate, const srf_roi_out* out_host, float* rois_out, void* stream);
 
-/* Fused img_feats_sampling_bboxes_roi (srfdet_head.py:2424-2565 / 1963-2099), B = 1
- * semantics (SURVEY.md 3.4): projection by lidar2img (n_cam,4,4), per-camera rectangle,
- * level map, RoIAlign, sum over cameras in registers.  Maps are (n_cam, C, H_l, W_l).
- * boxes (P, box_dim) normalised centres, NOT mutated.  rois_out (n_cam*P,5) nullable. */
-int srf_img_roi_features(const srf_pyramid* p_host, const float* boxes, int32_t n_prop, int32_t box_dim,
+/* Fused img_feats_sampling_bboxes_roi (srfdet_head.py:2424-2565 / 1963-2099) over a batch of
+ * B independent samples, each with the batch-1 semantics of SURVEY.md 3.4 (the reference itself is
+ * only defined at B = 1): projection by its own lidar2img[b] (n_cam,4,4), per-camera rectangle,
+ * level map, RoIAlign, sum over that sample's cameras in registers.  Maps are
+ * (B*n_cam, C, H_l, W_l) (NCHW or channels_last); image b*n_cam + cam is camera cam of sample b.
+ * boxes (B, P, box_dim) normalised centres, NOT mutated.  lidar2img (B, n_cam, 4, 4).  Output row
+ * k = b*P + p (as in srf_roi_extract, every srf_roi_out form).  rois_out (B*n_cam*P, 5) nullable:
+ * row (b*n_cam + cam)*P + p, column 0 = b*n_cam + cam, the image index srf_roi_extract reads.
+ * batch < 1 is SRF_ERR_ARG. */
+int srf_img_roi_features(const srf_pyramid* p_host, const float* boxes, int32_t batch, int32_t n_prop, int32_t box_dim,
                          const float* lidar2img, int32_t n_cam, const float pc_range_host[6],
                          const srf_roi_out* out_host, float* rois_out, void* stream);
 

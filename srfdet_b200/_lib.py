@@ -97,6 +97,7 @@ SWEEP_TRANSFORM, SWEEP_TIME_LAG, SWEEP_REMOVE_CLOSE = 1, 2, 4      # include/srf
 SWEEP_MAX_SOURCES, SWEEP_MAX_COLS = 64, 8
 AUG_FLIP_HORIZONTAL, AUG_FLIP_VERTICAL = 1, 2                       # include/srfdet_b200.h srf_augment_points flips
 AUG_MAX_VIEWS, AUG_MAX_COLS, MERGE_AUG_MAX_K = 32, 8, 4096
+GEMV_MAX_ROWS = 8                 # srf_gemv_f32 rows: the samples one DPG projection takes
 
 
 class Map(Structure):
@@ -194,7 +195,7 @@ PROTOTYPES = {
     'srf_roi_extract': (c_int32, [POINTER(Pyramid), c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
     'srf_bev_roi_features': (c_int32, [POINTER(Pyramid), c_void_p, c_int32, c_int32, c_int32, POINTER(c_float),
                                        POINTER(c_float), c_int32, POINTER(RoiOut), c_void_p, c_void_p]),
-    'srf_img_roi_features': (c_int32, [POINTER(Pyramid), c_void_p, c_int32, c_int32, c_void_p, c_int32,
+    'srf_img_roi_features': (c_int32, [POINTER(Pyramid), c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32,
                                        POINTER(c_float), POINTER(RoiOut), c_void_p, c_void_p]),
     'srf_dynconv_interact': (c_int32, [c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),

@@ -3,7 +3,7 @@
 // 2x2 samples, bilinear, avg, aligned=True), fused so that no RoI list, per-level
 // nonzero()/index round trip or (n_cam,P,C,7,7) intermediate ever reaches HBM.
 //
-// Work split: one CTA per proposal; lanes own output bins (bin = lane, lane+32) and keep
+// Work split: one CTA per proposal (per (sample, proposal) for a batch); lanes own output bins (bin = lane, lane+32) and keep
 // their 2x16 bilinear taps (offset, weight) in registers, warps stride over channels, so
 // the taps are computed once per (proposal, camera) and each channel costs 32 coalesced-
 // in-plane loads per lane.  The image variant accumulates the camera sum in registers.
@@ -183,12 +183,15 @@ __global__ void __launch_bounds__(256) bev_roi_kernel(Pyr p, float* __restrict__
   roi_forward(p, img, x1, y1, x2, y2, out, k, channel_last);
 }
 
-// image branch: CPW = channels per warp held as register accumulators (camera sum)
+// image branch: CPW = channels per warp held as register accumulators (camera sum).
+// One CTA per (sample, proposal): k = b * n_prop + proposal.  Sample b sums its own cameras only: images
+// b * n_cam + cam of the flattened pyramid, projected by lidar2img[b][cam] (B independent batch-1 calls, SURVEY.md 3.4).
 template <int CPW>
 __global__ void __launch_bounds__(256) img_roi_kernel(Pyr p, const float* __restrict__ boxes, int n_prop, int box_dim,
                                                      const float* __restrict__ lidar2img, int n_cam, Range rg,
                                                      float* __restrict__ out, int channel_last, float* __restrict__ rois_out) {
   const int k = blockIdx.x;
+  const int smp = k / n_prop, prop = k - smp * n_prop, img0 = smp * n_cam;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   const float* b = boxes + (size_t)k * box_dim;
   const float cx = b[0] * rg.span[0] + rg.lo[0], cy = b[1] * rg.span[1] + rg.lo[1], cz = b[2] * rg.span[2] + rg.lo[2];
@@ -199,7 +202,8 @@ __global__ void __launch_bounds__(256) img_roi_kernel(Pyr p, const float* __rest
   for (int i = 0; i < CPW; ++i) { acc0[i] = 0.f; acc1[i] = 0.f; }
   const bool has2 = lane + 32 < NBIN;
   for (int cam = 0; cam < n_cam; ++cam) {
-    const float* L = lidar2img + (size_t)cam * 16;
+    const int img = img0 + cam;
+    const float* L = lidar2img + (size_t)img * 16;
     float x1 = INFINITY, y1 = INFINITY, x2 = -INFINITY, y2 = -INFINITY;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -212,8 +216,8 @@ __global__ void __launch_bounds__(256) img_roi_kernel(Pyr p, const float* __rest
       x1 = fminf(x1, u); x2 = fmaxf(x2, u); y1 = fminf(y1, v); y2 = fmaxf(y2, v);
     }
     if (rois_out && threadIdx.x == 0) {
-      float* r = rois_out + ((size_t)cam * n_prop + k) * 5;
-      r[0] = (float)cam; r[1] = x1; r[2] = y1; r[3] = x2; r[4] = y2;
+      float* r = rois_out + ((size_t)img * n_prop + prop) * 5;
+      r[0] = (float)img; r[1] = x1; r[2] = y1; r[3] = x2; r[4] = y2;
     }
     const int lvl = roi_level(x1, y1, x2, y2, p.n_levels);
     const int H = p.h[lvl], W = p.w[lvl];
@@ -226,7 +230,7 @@ __global__ void __launch_bounds__(256) img_roi_kernel(Pyr p, const float* __rest
     Taps t0, t1;
     bin_taps(lane, x1s, y1s, bw, bh, H, W, t0);
     bin_taps(has2 ? lane + 32 : 0, x1s, y1s, bw, bh, H, W, t1);
-    const float* base = p.feat[lvl] + (size_t)cam * p.channels * H * W;
+    const float* base = p.feat[lvl] + (size_t)img * p.channels * H * W;
 #pragma unroll
     for (int i = 0; i < CPW; ++i) {
       int c = warp + i * nwarps;
@@ -453,7 +457,7 @@ __global__ void __launch_bounds__(256, NP == 1 ? SRF_ROI_MINB : 1) img_roi_cl_ke
   float* s_wt = reinterpret_cast<float*>(s_off + n_cam * NTAP);
   __shared__ RoiGeom sg[IMG_MAX_CAM];
   __shared__ const float* s_base[IMG_MAX_CAM];     // camera image of the RoI's level (resolved once: p.feat[] is indexed dynamically)
-  const int k = blockIdx.x;
+  const int k = blockIdx.x;   // b * n_prop + proposal (as img_roi_kernel)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // warp 0: lane = camera projects the box, resolves its level geometry, and the live cameras of this proposal are compacted
   // (1.2 of 6 on the bench frame): the tap staging and the bin loops only see those
@@ -463,11 +467,12 @@ __global__ void __launch_bounds__(256, NP == 1 ? SRF_ROI_MINB : 1) img_roi_cl_ke
     bool live = false;
     if (lane < n_cam) {
       const int cam = lane;
+      const int smp = k / n_prop, img = smp * n_cam + cam;
       const float* b = boxes + (size_t)k * box_dim;
       const float cx = b[0] * rg.span[0] + rg.lo[0], cy = b[1] * rg.span[1] + rg.lo[1], cz = b[2] * rg.span[2] + rg.lo[2];
       float cor[8][3];
       box_corners(cx, cy, cz, b[3], b[4], b[5], b[6], b[7], cor);
-      const float* L = lidar2img + (size_t)cam * 16;
+      const float* L = lidar2img + (size_t)img * 16;
       float x1 = INFINITY, y1 = INFINITY, x2 = -INFINITY, y2 = -INFINITY;
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
@@ -480,12 +485,12 @@ __global__ void __launch_bounds__(256, NP == 1 ? SRF_ROI_MINB : 1) img_roi_cl_ke
         x1 = fminf(x1, u); x2 = fmaxf(x2, u); y1 = fminf(y1, v); y2 = fmaxf(y2, v);
       }
       if (rois_out) {
-        float* r = rois_out + ((size_t)cam * n_prop + k) * 5;
-        r[0] = (float)cam; r[1] = x1; r[2] = y1; r[3] = x2; r[4] = y2;
+        float* r = rois_out + ((size_t)img * n_prop + (k - smp * n_prop)) * 5;
+        r[0] = (float)img; r[1] = x1; r[2] = y1; r[3] = x2; r[4] = y2;
       }
       const RoiGeom g = roi_geom(p, x1, y1, x2, y2);
       sg[cam] = g;
-      s_base[cam] = p.feat[g.lvl] + (size_t)cam * g.H * g.W * p.channels;
+      s_base[cam] = p.feat[g.lvl] + (size_t)img * g.H * g.W * p.channels;   // per-image base in size_t; taps stay 32-bit inside it
       live = g.live != 0;
     }
     const unsigned m = __ballot_sync(0xffffffffu, live);
@@ -617,12 +622,15 @@ int srf_bev_roi_features(const srf_pyramid* p, float* boxes, int32_t batch, int3
   return SRF_OK;
 }
 
-int srf_img_roi_features(const srf_pyramid* p, const float* boxes, int32_t n_prop, int32_t box_dim,
+int srf_img_roi_features(const srf_pyramid* p, const float* boxes, int32_t batch, int32_t n_prop, int32_t box_dim,
                          const float* lidar2img, int32_t n_cam, const float pc_range[6], const srf_roi_out* out_spec,
                          float* rois_out, void* stream) {
   Pyr d;
   SRF_CHECK_ARG(make_pyr(&d, p) == 0, "srf_img_roi_features: bad pyramid");
+  SRF_CHECK_ARG(batch >= 1, "srf_img_roi_features: batch must be >= 1 (got %d)", batch);
   SRF_CHECK_ARG(boxes && lidar2img && pc_range && n_prop >= 0 && box_dim >= 8 && n_cam >= 1, "srf_img_roi_features: bad args");
+  SRF_CHECK_ARG((long long)batch * n_prop <= 0x7fffffffLL && (long long)batch * n_cam <= 0x7fffffffLL,
+                "srf_img_roi_features: batch %d x %d proposals / %d cameras overflows", batch, n_prop, n_cam);
   OutSpec o;
   { int rc = make_out(&o, out_spec, d.channels, d.channels_last != 0, "srf_img_roi_features"); if (rc) return rc; }
   float* out = (float*)o.ptr;
@@ -640,15 +648,15 @@ int srf_img_roi_features(const srf_pyramid* p, const float* boxes, int32_t n_pro
       SRF_CUDA(cudaFuncSetAttribute(img_roi_cl_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       SRF_CUDA(cudaFuncSetAttribute(img_roi_cl_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
-    if (d.channels <= 128) img_roi_cl_kernel<1><<<n_prop, 256, smem, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, o, rois_out);
-    else img_roi_cl_kernel<2><<<n_prop, 256, smem, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, o, rois_out);
+    if (d.channels <= 128) img_roi_cl_kernel<1><<<batch * n_prop, 256, smem, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, o, rois_out);
+    else img_roi_cl_kernel<2><<<batch * n_prop, 256, smem, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, o, rois_out);
     SRF_LAUNCH_CHECK();
     return SRF_OK;
   }
   if (d.channels <= 128)
-    img_roi_kernel<16><<<n_prop, 256, 0, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, out, channel_last, rois_out);
+    img_roi_kernel<16><<<batch * n_prop, 256, 0, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, out, channel_last, rois_out);
   else
-    img_roi_kernel<32><<<n_prop, 256, 0, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, out, channel_last, rois_out);
+    img_roi_kernel<32><<<batch * n_prop, 256, 0, st>>>(d, boxes, n_prop, box_dim, lidar2img, n_cam, rg, out, channel_last, rois_out);
   SRF_LAUNCH_CHECK();
   return SRF_OK;
 }

@@ -7,7 +7,9 @@ builds; `pillar_rows` takes them straight to the backbone's input rows (srf_pill
 detector above it -- point path, SECONDCustom + FPN (`pts_backbone`, `pts_neck`) and SRFDetHead (`bbox_head`) --
 with the reference's test-time call contract (`forward_test` / `simple_test`), checkpoint loading by the reference's
 attribute names and a device-resident, optionally graph-captured `infer`.  The image backbone and image neck are not
-built: callers pass the image-neck outputs (DESIGN.md §1).
+built: callers pass the image-neck outputs (DESIGN.md §1).  Camera-fusion configs take batches too: a batch of B fusion
+samples is B independent batch-1 calls of the reference (SURVEY.md §3.4), each sample with its own image maps and its own
+lidar2img.
 """
 import collections
 import os
@@ -153,8 +155,8 @@ class SRFDet(SRFDetPointPath):
     Attributes keep the reference's names, so its checkpoints load unchanged: pts_voxel_layer, pts_voxel_encoder,
     pts_middle_encoder, pts_backbone, pts_neck, bbox_head.  img_backbone / img_neck configs are kept (not built) in
     `img_backbone_cfg` / `img_neck_cfg`.  use_graph=True: `infer` is captured into one CUDA graph per
-    (batch size, point counts, precision, image-map shapes) and replayed; outputs then live in graph-owned buffers that
-    the next replay overwrites.  A graph bakes in the weights it was captured with: loading weights through this
+    (batch size, point counts, precision, image-map shapes and strides, lidar2img shape) and replayed; outputs then live
+    in graph-owned buffers that the next replay overwrites.  A graph bakes in the weights it was captured with: loading weights through this
     module (load_checkpoint / load_state_dict) drops the captured graphs, any other weight change needs reset_graphs()."""
 
     def __init__(self, pts_voxel_layer=None, pts_voxel_encoder=None, pts_middle_encoder=None, pts_backbone=None,
@@ -270,16 +272,39 @@ class SRFDet(SRFDetPointPath):
         return img_feats, self.extract_pts_feat(points, precision)
 
     def _check_inputs(self, points, img_feats, lidar2img):
+        """Host-side checks of an infer call, before any device work."""
         self._check_eval()
         if not isinstance(points, (list, tuple)) or not points:
             raise ValueError('points must be a non-empty list of (N_i, C) CUDA tensors')
         if self.bbox_head.use_img:
             if img_feats is None or lidar2img is None:
                 raise ValueError('this fusion config needs img_feats (the image-neck outputs, one (B, n_cam, C, H, W) map per '
-                                 'level) and lidar2img (n_cam, 4, 4)')
-            if len(points) > 1:
-                raise NotImplementedError('the camera fusion branch keeps the reference\'s batch-size-1 semantics '
-                                          '(one lidar2img for the batch): pass one cloud per call with images')
+                                 'level) and lidar2img (B, n_cam, 4, 4)')
+            self._check_fusion_batch(len(points), img_feats, lidar2img)
+
+    def _check_fusion_batch(self, n, img_feats, lidar2img):
+        """n clouds need n samples of image maps and n camera sets (SURVEY.md §3.4: a batch of B fusion samples is B
+        independent batch-1 calls).  One camera set for several clouds is the reference's own B > 1 case, which it does not
+        define consistently (its RoI batch index and its feature flattening disagree): refused as such."""
+        if not img_feats or any(f.dim() != 5 for f in img_feats):
+            raise ValueError('img_feats: one (B, n_cam, C, H, W) image-neck map per level')
+        batches, cams = {f.shape[0] for f in img_feats}, {f.shape[1] for f in img_feats}
+        if len(batches) != 1 or len(cams) != 1:
+            raise ValueError(f'every image level needs the same batch and camera count, got {[tuple(f.shape[:2]) for f in img_feats]}')
+        mb, n_cam = batches.pop(), cams.pop()
+        l2i = tuple(lidar2img.shape)
+        if n > 1 and mb == 1 and l2i in ((n_cam, 4, 4), (1, n_cam, 4, 4)):
+            raise NotImplementedError(
+                f'the camera fusion branch has the reference\'s batch-size-1 semantics per sample: one camera set (image maps '
+                f'of batch 1, lidar2img {l2i}) for {n} clouds is undefined there; pass each sample\'s maps as '
+                f'({n}, {n_cam}, C, H, W) per level and lidar2img as ({n}, {n_cam}, 4, 4)')
+        if mb != n:
+            raise ValueError(f'image maps of batch {mb} for {n} clouds: the maps need one sample per cloud')
+        if l2i != (n, n_cam, 4, 4) and not (n == 1 and l2i == (n_cam, 4, 4)):
+            raise ValueError(f'lidar2img {l2i} does not match {n} sample(s) of {n_cam} cameras: pass ({n}, {n_cam}, 4, 4)')
+        if getattr(self.bbox_head, 'with_dpg', False) and n > L.GEMV_MAX_ROWS:
+            raise ValueError(f'{n} samples: the dynamic proposal generation projections (srf_gemv_f32) take at most '
+                             f'{L.GEMV_MAX_ROWS} samples per call')
 
     @torch.no_grad()
     def _infer_eager(self, points, img_feats, lidar2img, precision):
@@ -294,7 +319,9 @@ class SRFDet(SRFDetPointPath):
     @torch.no_grad()
     def infer(self, points, img_feats=None, lidar2img=None, precision=None):
         """points: list of B (N_i, C) fp32 CUDA clouds; img_feats (fusion configs): per level (B, n_cam, C, H, W) image-neck
-        maps, C = feat_channels_img (reduced by the head's img_convs) or hidden_dim; lidar2img (n_cam, 4, 4).
+        maps, C = feat_channels_img (reduced by the head's img_convs) or hidden_dim; lidar2img (B, n_cam, 4, 4), or
+        (n_cam, 4, 4) for one cloud.  Sample b is fused with its own maps img_feats[l][b] and projections lidar2img[b]: the
+        B samples are B independent batch-1 calls of the reference (SURVEY.md §3.4).
         -> with the head's device NMS: boxes (B, max_per_img, dim-1), scores (B, max_per_img), labels (B, max_per_img)
         int32, counts (B,) int32 (SRFDetHead.nms_bboxes); otherwise the decoded (scores (B, P, #cls), boxes (B, P, dim-1)).
         No host synchronisation."""
@@ -303,7 +330,8 @@ class SRFDet(SRFDetPointPath):
         if not self.use_graph:
             return self._infer_eager(points, img_feats, lidar2img, precision)
         key = (tuple(tuple(p.shape) for p in points), precision,
-               None if img_feats is None else tuple((tuple(f.shape), f.stride()) for f in img_feats))
+               None if img_feats is None else tuple((tuple(f.shape), f.stride()) for f in img_feats),
+               None if lidar2img is None else tuple(lidar2img.shape))
         n, n_img = len(points), len(img_feats or [])
 
         def statics():
@@ -430,7 +458,8 @@ class SRFDet(SRFDetPointPath):
     @torch.no_grad()
     def simple_test(self, points, img_metas, img=None, img_feats=None, rescale=False):
         """srfdet.py:326-340 -> [dict(pts_bbox=dict(boxes_3d, scores_3d, labels_3d))] per sample, CPU tensors (mmdet3d
-        bbox3d2result); boxes wrapped in img_metas[i]['box_type_3d'] when given.  One host read-back per call."""
+        bbox3d2result); boxes wrapped in img_metas[i]['box_type_3d'] when given.  One host read-back per call.
+        Fusion configs: img_feats per level (B, n_cam, C, H, W); sample i is projected by img_metas[i]['lidar2img']."""
         self._check_eval()
         if img is not None and img_feats is None:
             raise ValueError('img= needs the image backbone and image neck, which are not built here '
@@ -438,7 +467,12 @@ class SRFDet(SRFDetPointPath):
                              f'{(self.img_neck_cfg or {}).get("type")}): run them outside and pass their outputs as img_feats=')
         lidar2img = None
         if self.bbox_head.use_img and img_feats is not None:
-            lidar2img = torch.as_tensor(np.asarray(img_metas[0]['lidar2img']), dtype=torch.float32, device=points[0].device)
+            if len(img_metas) != len(points):
+                raise ValueError(f'{len(points)} clouds with {len(img_metas)} img_metas: each sample needs its own meta')
+            # one sample: its meta's (n_cam, 4, 4) as given; B samples: each from its own meta -> (B, n_cam, 4, 4)
+            l2i = (np.asarray(img_metas[0]['lidar2img']) if len(img_metas) == 1
+                   else np.stack([np.asarray(m['lidar2img']) for m in img_metas]))
+            lidar2img = torch.as_tensor(l2i, dtype=torch.float32, device=points[0].device)
         out = self.infer(points, img_feats, lidar2img)
         head = self.bbox_head
         res = head.format_nms(*out, img_metas) if head.device_nms else head.select_decoded(*out, img_metas)

@@ -18,7 +18,7 @@ from torch import nn
 from .. import _lib as L
 from . import registry
 from .registry import HEADS
-from .roi import img_feats_sampling_bboxes_roi, maps_channels_last, points_feats_sampling_bboxes_roi
+from .roi import flat_image_maps, img_feats_sampling_bboxes_roi, maps_channels_last, points_feats_sampling_bboxes_roi
 
 _DEFAULT_SCALE_CLAMP = math.log(100000.0 / 16)
 
@@ -434,12 +434,12 @@ class SingleSRFDetHead(_SingleHeadBase):
         self._cache = {}
 
     def region_features(self, img_feats, point_feats, bboxes, pooler, pooler_img, lidar2img, precision=None):
-        """Fused RoI features (bs*n_p, 49, C) channel-last: image RoIs (camera sum), BEV RoIs,
-        concat + Linear(2C->C) (srfdet_head.py:2236-2264)."""
+        """Fused RoI features (bs*n_p, 49, C) channel-last: image RoIs (each sample's own camera sum), BEV RoIs,
+        concat + Linear(2C->C) (srfdet_head.py:2236-2264).  lidar2img (bs, n_cam, 4, 4), or (n_cam, 4, 4) at bs = 1."""
         precision = precision or registry.get_precision()
         img_roi = pts_roi = None
         if (self.use_fusion and img_feats is not None and point_feats is not None
-                and maps_channels_last([f[0] for f in img_feats], pooler_img.num_inputs)
+                and maps_channels_last(flat_image_maps(img_feats), pooler_img.num_inputs)
                 and maps_channels_last(point_feats, pooler.num_inputs)):
             # both samplers write their half of cat(img, pts) (srfdet_head.py:2257) in the GEMM's dtype
             k, c = bboxes.shape[0] * bboxes.shape[1], point_feats[0].shape[1]

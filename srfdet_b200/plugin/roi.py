@@ -133,20 +133,40 @@ def points_feats_sampling_bboxes_roi(points_feats, bboxes, pooler, pc_range, vox
     return (out, rois) if return_rois else out
 
 
+def flat_image_maps(img_feats):
+    """(B, n_cam, C, H, W) image maps per level -> (B*n_cam, C, H, W): image b*n_cam + cam is camera cam of sample b.
+    A view where the strides allow one (the head's img_convs outputs and any densely packed level); a level whose images
+    are not evenly spaced is copied."""
+    for f in img_feats:
+        if f.dim() != 5:
+            raise ValueError(f'image maps must be (B, n_cam, C, H, W) per level, got {tuple(f.shape)}')
+    return [f.reshape(-1, *f.shape[2:]) for f in img_feats]
+
+
 def img_feats_sampling_bboxes_roi(img_feats, bboxes, pooler, lidar2img, pc_range, channel_last=False,
                                   return_rois=False, out=None, ch_offset=0, out_enc=None):
-    """Fused srfdet_head.py:2424-2565 (B = 1 semantics, SURVEY.md 3.4).  img_feats: list of
-    (1, n_cam, C, H, W); bboxes (1, n_p, >=8) (not mutated); lidar2img (n_cam,4,4) tensor."""
-    assert bboxes.shape[0] == 1 and img_feats[0].shape[0] == 1, 'image branch is built for batch size 1 (as the reference is)'
-    b = bboxes[0].contiguous().float()
-    n_p, d = b.shape
-    flat = [f[0] for f in img_feats]
+    """Fused srfdet_head.py:2424-2565 over B samples, each with the reference's batch-1 semantics (SURVEY.md 3.4: a
+    batch of B fusion samples is B independent batch-1 calls): sample b sums its own cameras, projected by its own
+    lidar2img[b].  img_feats: list of (B, n_cam, C, H, W); bboxes (B, n_p, >=8) (not mutated); lidar2img
+    (B, n_cam, 4, 4) tensor, or (n_cam, 4, 4) at B = 1.  -> (B*n_p, C, 7, 7) (or channel-last (B*n_p, 49, C); `out` /
+    `ch_offset`: write into a slice of a caller buffer); return_rois: also the (B*n_cam*n_p, 5) image RoIs, row
+    (b*n_cam + cam)*n_p + p with column 0 = b*n_cam + cam (srf_roi_extract on the flattened maps reads them)."""
+    bs, n_p, d = bboxes.shape
+    flat = flat_image_maps(img_feats)
+    if any(f.shape[0] != bs for f in img_feats):
+        raise ValueError(f'image maps of batch {[f.shape[0] for f in img_feats]} for {bs} samples of boxes')
+    n_cam = img_feats[0].shape[1]
+    if any(f.shape[1] != n_cam for f in img_feats):
+        raise ValueError('every image level needs the same number of cameras')
+    if tuple(lidar2img.shape) not in ((bs, n_cam, 4, 4),) + (((n_cam, 4, 4),) if bs == 1 else ()):
+        raise ValueError(f'lidar2img {tuple(lidar2img.shape)} does not match {bs} sample(s) of {n_cam} cameras: '
+                         f'pass ({bs}, {n_cam}, 4, 4)')
+    b = bboxes.contiguous().float()
     p, keep = _pyramid(flat, pooler.featmap_strides, pooler.num_inputs)
-    n_cam = flat[0].shape[0]
-    l2i = lidar2img.reshape(n_cam, 4, 4).contiguous().float()
+    l2i = lidar2img.reshape(bs, n_cam, 4, 4).contiguous().float()
     c = p.channels
-    out, spec = _roi_out(n_p, c, channel_last, b.device, out, ch_offset, out_enc)
-    rois = torch.empty((n_cam * n_p, 5), dtype=torch.float32, device=b.device) if return_rois else None
-    L.check(L.load().srf_img_roi_features(ctypes.byref(p), L.ptr(b), n_p, d, L.ptr(l2i), n_cam, L.f6(pc_range),
+    out, spec = _roi_out(bs * n_p, c, channel_last, b.device, out, ch_offset, out_enc)
+    rois = torch.empty((bs * n_cam * n_p, 5), dtype=torch.float32, device=b.device) if return_rois else None
+    L.check(L.load().srf_img_roi_features(ctypes.byref(p), L.ptr(b), bs, n_p, d, L.ptr(l2i), n_cam, L.f6(pc_range),
                                           ctypes.byref(spec), L.ptr(rois), L.stream_ptr()), 'srf_img_roi_features')
     return (out, rois) if return_rois else out

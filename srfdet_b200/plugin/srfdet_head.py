@@ -186,8 +186,9 @@ class SRFDetHead(nn.Module):
     def forward(self, img_feats, point_feats, img_metas=None, lidar2img=None, precision=None, dpg_img_logits=None):
         """img_feats: list of (bs, n_cam, C, H, W) | None; point_feats: list of (bs, C, H, W) BEV maps (NCHW or
         torch.channels_last).  -> (pred_logits (#stages, bs, n_p, #cls), pred_bboxes (#stages, bs, n_p, dim)) with
-        absolute centres and log sizes, like the reference (:474-498).  lidar2img (n_cam,4,4) tensor may replace
-        img_metas[*]['lidar2img'] (keeps the call free of host work)."""
+        absolute centres and log sizes, like the reference (:474-498).  A lidar2img (bs, n_cam, 4, 4) tensor ((n_cam, 4, 4)
+        at bs = 1) may replace img_metas[*]['lidar2img'] (keeps the call free of host work).  Sample b uses its own camera
+        maps and lidar2img[b] only (SURVEY.md §3.4: B fusion samples are B independent batch-1 calls)."""
         img_feats = self._image_maps(img_feats, precision)
         bboxes, prop = self._get_init_proposals(img_feats, point_feats, sigmoid_centres=True, dpg_img_logits=dpg_img_logits)
         if self.use_img and lidar2img is None:

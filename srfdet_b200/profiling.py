@@ -146,9 +146,10 @@ def _work(name, a, s, ctx):
         # (379 MB) as an upper bound; what 900 car-sized proposals touch is data dependent and ~6x smaller: the
         # per-launch DRAM read of this kernel in the committed ncu capture is used when bench.py passes it
         # (ctx['img_roi_input_bytes']), otherwise the upper bound.
+        # (a batch of B samples touches B such camera sets)
         c = s['channels']
-        k, n_cam = a[2], a[5]
-        touched = ctx.get('img_roi_input_bytes') or n_cam * sum(h * w for h, w in s['hw']) * c * 4
+        batch, k, n_cam = a[2], a[2] * a[3], a[6]
+        touched = batch * (ctx.get('img_roi_input_bytes') or n_cam * sum(h * w for h, w in s['hw']) * c * 4)
         return 0.0, k * 49 * c * ES[s.get('out_enc', L.F32)] + touched
     if name == 'srf_linear':
         es = ES[s['enc']]

@@ -141,9 +141,20 @@ def proposals(seed, n=900, dims=10, batch=1):
     return b
 
 
-def lidar2img(n_cam=6, batch=1):
+def lidar2img(n_cam=6, batch=1, yaw_offsets=None):
     """nuScenes-like projection matrices built by the recipe of
-    datasets/nuscenes_dataset.py:53-65: lidar2img = viewpad(K) @ [R^T | -R^T t]^T."""
+    datasets/nuscenes_dataset.py:53-65: lidar2img = viewpad(K) @ [R^T | -R^T t]^T.
+    yaw_offsets: one angle (radians) per sample that turns its whole camera rig about the LiDAR z axis, so the
+    samples of a batch see different projections; None: every sample has the same rig."""
+    if yaw_offsets is not None:
+        assert len(yaw_offsets) == batch
+        base = lidar2img(n_cam, 1)[0].astype(np.float64)
+        out = np.zeros((batch, n_cam, 4, 4), np.float32)
+        for b, a in enumerate(yaw_offsets):
+            rz = np.eye(4)      # a rig turned by a sees the LiDAR frame turned by -a
+            rz[:2, :2] = [[math.cos(a), math.sin(a)], [-math.sin(a), math.cos(a)]]
+            out[b] = (base @ rz).astype(np.float32)
+        return out
     yaws = np.deg2rad([0.0, 55.0, -55.0, 110.0, -110.0, 180.0])[:n_cam]
     K = np.array([[1266.0, 0, 816.0], [0, 1266.0, 491.0], [0, 0, 1.0]])
     out = np.zeros((batch, n_cam, 4, 4), np.float32)

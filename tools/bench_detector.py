@@ -1,6 +1,6 @@
 """Detector-level timings (CUDA events on the launching stream, 512 MiB L2 flush between steps, median of `--iters`):
 
-    python tools/bench_detector.py [--kinds nusc waymo pillar tta] [--iters 20]
+    python tools/bench_detector.py [--kinds nusc waymo pillar tta nusc_lc] [--iters 20]
 
 Per configuration (nusc_L, waymo_L; calibrated synthetic weights of RegionFeaturePipeline, production-size clouds,
 the configs' rotated NMS on) one JSON line per case:
@@ -25,6 +25,14 @@ tta (nusc_L weights as above, the restated double-flip config's range; one 300k-
   infer_aug B=1      one CUDA graph over augment + the views' batch + merge, at 1, 2 and 4 distinct flip views, next to
                      plain infer on the same cloud (frames/s);
   kernels            srf_augment_points (4 views) and srf_merge_aug_bev (8 views x 300 rows, 10 classes) alone (us).
+nusc_lc (camera fusion, tests/golden/configs/model/srfdet_nusc_LC.py with RegionFeaturePipeline(fusion=True)'s calibrated
+weights, rotated NMS on; 300k-point clouds, per sample synthetic 6-camera channels_last maps and its own lidar2img, the
+camera rig turned about z per sample):
+  infer B=1/2/4      one CUDA graph over the batch, 128-channel maps (frames/s);
+  infer B=4 256ch    the same with 256-channel image-neck maps reduced by the head's img_convs inside the graph;
+  run_frames x4      RegionFeaturePipeline(fusion=True).run_frames: 4 single-frame graphs in flight (frames/s);
+  kernel             srf_img_roi_features alone at B = 1 and B = 4 (900 proposals per sample, 128 channels, fp32
+                     channel-last output; us per call).
 The first line names the GPU and its power limit.
 """
 import argparse
@@ -260,9 +268,59 @@ def bench_tta(iters, flush):
     det.reset_graphs()
 
 
+def _camera_maps(seed, b, c, n_cam=6):
+    """(b, n_cam, c, H, W) synthetic image-neck maps per level, channels_last in memory (as the img_convs emit them)."""
+    from srfdet_b200 import synth
+    return [torch.as_tensor(f.reshape(b * n_cam, *f.shape[2:])).cuda().contiguous(memory_format=torch.channels_last).view(f.shape)
+            for f in synth.feature_pyramid(seed, c, (232, 400), 4, lead=(b, n_cam))]
+
+
+def bench_nusc_lc(iters, flush):
+    from srfdet_b200 import synth
+    from srfdet_b200.pipeline import N_PROP, RegionFeaturePipeline
+    from srfdet_b200.plugin import SRFDet, img_feats_sampling_bboxes_roi
+    cfg = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'tests', 'golden', 'configs', 'model', 'srfdet_nusc_LC.py')
+    pipe = RegionFeaturePipeline('nusc', fusion=True, scope='full', use_nms=True, use_graph=True)
+    pipe.calibrate(torch.as_tensor(synth.cloud('nusc', 44)).cuda())
+    det = SRFDet.from_config(cfg).cuda()
+    sd = dict(pipe.detector.state_dict())
+    for prefix, m in (('pts_backbone.', pipe.backbone), ('pts_neck.', pipe.neck), ('bbox_head.', pipe.head)):
+        sd.update({prefix + k: v for k, v in m.state_dict().items()})
+    det.load_checkpoint(sd)
+    det.use_graph = True
+    name, prec = 'nusc_LC', pipe.precision
+    clouds = [torch.as_tensor(synth.cloud('nusc', 1000 + i)).cuda() for i in range(4)]
+    l2i = torch.as_tensor(synth.lidar2img(6, 4, yaw_offsets=[0.0, 0.4, -0.7, 1.3])).cuda()
+    maps = _camera_maps(1100, 4, 128)
+
+    def out(case, ms, frames_n, **extra):
+        print(json.dumps(dict(config=name, case=case, precision=prec, ms=round(ms, 4),
+                              frames_per_s=round(frames_n / ms * 1e3, 1) if frames_n else None, **extra)), flush=True)
+    for b in (1, 2, 4):
+        mb = [f[:b] for f in maps]
+        out(f'infer B={b} (one graph, 6 cameras x 128 channels per sample)',
+            timed(lambda: det.infer(clouds[:b], img_feats=mb, lidar2img=l2i[:b]), iters, flush), b,
+            points=[int(x.shape[0]) for x in clouds[:b]])
+    wide = _camera_maps(1200, 4, 256)
+    out('infer B=4 (one graph, 6 cameras x 256 channels per sample through img_convs)',
+        timed(lambda: det.infer(clouds, img_feats=wide, lidar2img=l2i), iters, flush), 4)
+    del wide
+    det.reset_graphs()
+    out('run_frames x4 (RegionFeaturePipeline(fusion=True): 4 single-frame graphs in flight)',
+        timed(lambda: pipe.run_frames(clouds), iters, flush), 4)
+    pooler = det.bbox_head.roi_extractor_img
+    pc = det.bbox_head.head_series_lidar[0].pc_range_lidar
+    boxes = torch.as_tensor(synth.proposals(1300, N_PROP, 10, 4)).cuda()
+    for b in (1, 4):
+        mb, bb = [f[:b] for f in maps], boxes[:b].contiguous()
+        ms = timed(lambda: img_feats_sampling_bboxes_roi(mb, bb, pooler, l2i[:b], pc, channel_last=True), iters * 5, flush)
+        out(f'kernel srf_img_roi_features B={b} ({N_PROP} proposals x 6 cameras per sample, 128 channels, fp32 out)', ms, 0,
+            us=round(ms * 1e3, 1), us_per_sample=round(ms * 1e3 / b, 1))
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar', 'tta'])
+    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar', 'tta', 'nusc_lc'])
     ap.add_argument('--iters', type=int, default=20)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -274,6 +332,8 @@ def main():
             bench_pillar(a.iters, flush)
         elif kind == 'tta':
             bench_tta(a.iters, flush)
+        elif kind == 'nusc_lc':
+            bench_nusc_lc(a.iters, flush)
         else:
             bench_kind(kind, a.iters, flush)
 

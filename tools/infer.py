@@ -16,10 +16,11 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..'
 EPILOG = """\
 --points: point files are raw float32 arrays of load-dim values per point (mmdet3d LoadPointsFromFile); use-dim selects
 the columns the model reads.  Each file is one cloud, used as it is, so pass clouds that already hold what the config's
-pipeline would have produced.  LiDAR-only configs run all clouds as one batch; camera-fusion
-configs take one cloud plus the image-neck outputs (the image backbone and neck are not built here): --img-feats is an
-.npz with one (n_cam, C, H, W) or (1, n_cam, C, H, W) float32 array per FPN level, in level order, and --lidar2img an
-(n_cam, 4, 4) .npy.
+pipeline would have produced.  All clouds run as one batch.  Camera-fusion configs also take the image-neck outputs
+(the image backbone and neck are not built here): --img-feats is an .npz with one float32 array per FPN level, in level
+order, each (B, n_cam, C, H, W) with one sample per --points file in the same order (or (n_cam, C, H, W) for one cloud),
+and --lidar2img a (B, n_cam, 4, 4) .npy (or (n_cam, 4, 4) for one cloud).  Sample i is fused with its own maps and
+projections only, as B separate runs of one cloud would be.
 --info: frames --index of an mmdet3d nuscenes_infos_*.pkl (read without running any pickled code) go through the point
 steps of the config's test_pipeline on the GPU -- LoadPointsFromFile, LoadPointsFromMultiSweeps (the key frame and its
 sweeps moved into the key frame's LiDAR frame, with the time lag column) and PointsRangeFilter -- one frame at a time
@@ -48,7 +49,7 @@ def main(argv=None):
     ap.add_argument('--load-dim', type=int, default=5, help='float32 values per point in the files (default 5)')
     ap.add_argument('--use-dim', type=int, nargs='+', default=None, help='columns passed to the model (default: all)')
     ap.add_argument('--img-feats', help='.npz of image-neck maps, one array per level (fusion configs)')
-    ap.add_argument('--lidar2img', help='.npy (n_cam, 4, 4) LiDAR-to-image projections (fusion configs)')
+    ap.add_argument('--lidar2img', help='.npy (B, n_cam, 4, 4) LiDAR-to-image projections, one set per cloud (fusion configs)')
     ap.add_argument('--precision', choices=['fp16', 'fp32'], default=None, help='default: the library default (fp16)')
     ap.add_argument('--trusted', action='store_true',
                     help='allow pickled Python objects in the checkpoint (mmcv checkpoints carry them); only for trusted files')
@@ -78,12 +79,10 @@ def main(argv=None):
     if det.bbox_head.use_img:
         if not (a.img_feats and a.lidar2img):
             sys.exit('this is a camera-fusion config: pass --img-feats and --lidar2img')
-        if len(clouds) != 1:
-            sys.exit('camera-fusion configs take one cloud per run')
-        z = np.load(a.img_feats)
-        img_feats = [torch.as_tensor(z[k]).float().cuda() for k in z.files]
-        img_feats = [f.unsqueeze(0) if f.dim() == 4 else f for f in img_feats]
-        metas[0]['lidar2img'] = np.load(a.lidar2img)
+        maps, l2i = camera_inputs(np.load(a.img_feats), np.load(a.lidar2img), len(clouds))
+        img_feats = [torch.as_tensor(f).float().cuda() for f in maps]
+        for m, p in zip(metas, l2i):
+            m['lidar2img'] = p
     aug = test_augmentation(a.config)
     if aug is not None:
         results = aug_results(det, det.infer_aug(clouds, aug.views, aug.view_range))
@@ -94,6 +93,29 @@ def main(argv=None):
         report(out, i, path, clouds[i].shape[0], r)
     if a.out:
         np.savez(a.out, **out)
+
+
+def camera_inputs(z, lidar2img, n_clouds):
+    """--img-feats levels and --lidar2img for n_clouds samples -> ((B, n_cam, C, H, W) arrays, (B, n_cam, 4, 4)); exits
+    with a message when the counts do not match."""
+    maps = [np.asarray(z[k]) for k in z.files]
+    if not maps:
+        sys.exit('--img-feats holds no arrays')
+    if any(f.ndim not in (4, 5) for f in maps):
+        sys.exit(f'--img-feats: each level must be (B, n_cam, C, H, W) or (n_cam, C, H, W), got {[f.shape for f in maps]}')
+    maps = [f[None] if f.ndim == 4 else f for f in maps]
+    if any(f.shape[:2] != maps[0].shape[:2] for f in maps):
+        sys.exit(f'--img-feats: every level needs the same (B, n_cam), got {[f.shape[:2] for f in maps]}')
+    b, n_cam = maps[0].shape[:2]
+    if b != n_clouds:
+        sys.exit(f'--img-feats holds maps of {b} sample(s) for {n_clouds} --points file(s): pass one sample per cloud')
+    lidar2img = np.asarray(lidar2img, np.float32)
+    shape = lidar2img.shape
+    if shape == (n_cam, 4, 4) and n_clouds == 1:
+        lidar2img = lidar2img[None]
+    elif shape != (n_clouds, n_cam, 4, 4):
+        sys.exit(f'--lidar2img {shape} does not match {n_clouds} cloud(s) of {n_cam} cameras: pass ({n_clouds}, {n_cam}, 4, 4)')
+    return maps, lidar2img
 
 
 def report(out, i, name, n_points, r):
