@@ -88,6 +88,29 @@ int srf_hard_voxelize(const float* points, int32_t n, int32_t c, const srf_geom*
                       int32_t* coors, int32_t* num_points, float* mean, int32_t* point2voxel,
                       int32_t* d_voxel_num, void* ws, size_t ws_bytes, void* stream);
 
+/* Hard voxelization of B clouds in one launch sequence (the number of launches does not depend
+ * on B).  Cloud b is points_host[b] (n_host[b], c) on the device; host arrays of B entries.
+ * Block b of every output equals, bit for bit, what srf_hard_voxelize(..., batch_idx = b)
+ * writes for cloud b alone (its first-come voxel order, slots, counts, coordinates and means):
+ *  voxels      (B, max_voxels, max_points, c) f32, zero padded   [nullable]
+ *  coors       (B, max_voxels, 4) bzyx, b = block index
+ *  num_points  (B, max_voxels)
+ *  mean        (B, max_voxels, c) f32                            [nullable]
+ *  d_counts    (B) device: voxels of each block (<= max_voxels)
+ * Rows of block b at and past d_counts[b] are left untouched.  Limits (SRF_ERR_ARG, before any
+ * launch): 1 <= B <= SRF_HV_BATCH_MAX, 3 <= c <= 8, the row counts sum to < 2^31, and
+ * B x max_voxels and B x table capacity (the power of two >= max(1024, 2 max n)) < 2^31.
+ * Workspace: srf_hard_voxelize_batch_ws_bytes(n_host, B, ...) bytes, 0 for bad arguments; one
+ * hash table per cloud, so it is about B times the largest cloud's srf_hard_voxelize workspace
+ * (B = 32 clouds of 300k points, max_points 10, 160k voxels: 723 MB).  No allocation, no host
+ * synchronisation: a captured call replays.  11 launches (10 without voxels), 2 of them memsets. */
+#define SRF_HV_BATCH_MAX 1024
+size_t srf_hard_voxelize_batch_ws_bytes(const int32_t* n_host, int32_t batch, int32_t max_points, int32_t max_voxels);
+int srf_hard_voxelize_batch(const float* const* points_host, const int32_t* n_host, int32_t batch, int32_t c,
+                            const srf_geom* g_host, int32_t max_points, int32_t max_voxels, float* voxels,
+                            int32_t* coors, int32_t* num_points, float* mean, int32_t* d_counts, void* ws,
+                            size_t ws_bytes, void* stream);
+
 /* Batched hard voxelization without a host read of the per-sample voxel counts: the
  * reference voxelizes each sample alone and concatenates the valid rows (srfdet.py:218-232);
  * here every sample writes a fixed block of block_rows rows (srf_hard_voxelize with its own
@@ -477,7 +500,8 @@ int srf_dwconv3x3_s2(const srf_map* a_host, const srf_map* b_host, int32_t n, in
  * F.interpolate + sum over the cameras of a sample (:584-590).  out (n_samples, ho*wo). */
 int srf_channel_sum(const srf_map* a_host, const srf_map* b_host, int32_t n_samples, int32_t group, int32_t h,
                     int32_t w, int32_t ho, int32_t wo, float* out, void* stream);
-/* out (m,n) = act(x (m,k) . W (n,k)^T + bias), m <= 8 rows (dpg_fc1 / dpg_fc2, :537-543) */
+/* out (m,n) = act(x (m,k) . W (n,k)^T + bias), 1 <= m <= 524280 rows (dpg_fc1 / dpg_fc2, :537-543; one row per
+ * sample).  Rows run in groups of 8, one launch; each row is bit-identical to a call with that row alone. */
 int srf_gemv_f32(const float* x, int32_t m, int32_t k, const float* w, int32_t n, const float* bias,
                  int32_t relu, float* out, void* stream);
 /* (logits_a (+ logits_b)/2) (B,E,P) -> softmax over E -> boxes (B,P,dim) = sum_e w emb_boxes[e,p] with the

@@ -97,7 +97,7 @@ SWEEP_TRANSFORM, SWEEP_TIME_LAG, SWEEP_REMOVE_CLOSE = 1, 2, 4      # include/srf
 SWEEP_MAX_SOURCES, SWEEP_MAX_COLS = 64, 8
 AUG_FLIP_HORIZONTAL, AUG_FLIP_VERTICAL = 1, 2                       # include/srfdet_b200.h srf_augment_points flips
 AUG_MAX_VIEWS, AUG_MAX_COLS, MERGE_AUG_MAX_K = 32, 8, 4096
-GEMV_MAX_ROWS = 8                 # srf_gemv_f32 rows: the samples one DPG projection takes
+HV_BATCH_MAX = 1024               # include/srfdet_b200.h SRF_HV_BATCH_MAX: clouds of one srf_hard_voxelize_batch call
 
 
 class Map(Structure):
@@ -129,6 +129,9 @@ PROTOTYPES = {
     'srf_hard_voxelize_ws_bytes': (c_size_t, [c_int32, c_int32, c_int32]),
     'srf_hard_voxelize': (c_int32, [c_void_p, c_int32, c_int32, POINTER(Geom), c_int32, c_int32, c_int32, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    'srf_hard_voxelize_batch_ws_bytes': (c_size_t, [POINTER(c_int32), c_int32, c_int32, c_int32]),
+    'srf_hard_voxelize_batch': (c_int32, [POINTER(c_void_p), POINTER(c_int32), c_int32, c_int32, POINTER(Geom), c_int32, c_int32,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     'srf_concat_counted_rows': (c_int32, [c_void_p, c_int32, c_int32, POINTER(Rows), c_int32, c_void_p, c_void_p]),
     'srf_index_bytes': (c_size_t, [c_int64]),
     'srf_index_clear': (c_int32, [c_void_p, c_int64, c_void_p]),

@@ -292,12 +292,18 @@ __global__ void channel_sum_kernel(MapView a, MapView b, int n_samples, int grou
   }
 }
 
-// out (m, n) = act(x (m, k) . W (n, k)^T + bias): one warp per output column, every row of x (m <= 8) at once
+// out (m, n) = act(x (m, k) . W (n, k)^T + bias): one warp per output column, GEMV_MAXM rows of x at once; blockIdx.y
+// picks the group of rows [8y, 8y + 8).  A row's sum does not depend on the other rows of its group or on the group, so
+// every row comes out as it does in a call of that row alone.
 constexpr int GEMV_MAXM = 8;
 __global__ void __launch_bounds__(256) gemv_kernel(const float* __restrict__ x, int m, int k, const float* __restrict__ w, int n,
                                                    const float* __restrict__ bias, int relu, float* __restrict__ out) {
   const int col = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (col >= n) return;
+  const int r0 = blockIdx.y * GEMV_MAXM;
+  x += (size_t)r0 * k;
+  out += (size_t)r0 * n;
+  m = min(m - r0, GEMV_MAXM);
   float acc[GEMV_MAXM];
 #pragma unroll
   for (int r = 0; r < GEMV_MAXM; ++r) acc[r] = 0.f;
@@ -461,9 +467,10 @@ int srf_channel_sum(const srf_map* a, const srf_map* b, int32_t n_samples, int32
 
 int srf_gemv_f32(const float* x, int32_t m, int32_t k, const float* w, int32_t n, const float* bias, int32_t relu, float* out,
                  void* stream) {
-  SRF_CHECK_ARG(x && w && out && m >= 1 && m <= GEMV_MAXM && k >= 1 && n >= 1, "srf_gemv_f32: need 1 <= m <= %d rows", GEMV_MAXM);
+  SRF_CHECK_ARG(x && w && out && m >= 1 && m <= 65535 * GEMV_MAXM && k >= 1 && n >= 1, "srf_gemv_f32: need 1 <= m <= %d rows",
+                65535 * GEMV_MAXM);
   SRF_COUNT(1);
-  gemv_kernel<<<cdiv(n, 8), 256, 0, (cudaStream_t)stream>>>(x, m, k, w, n, bias, relu, out);
+  gemv_kernel<<<dim3(cdiv(n, 8), cdiv(m, GEMV_MAXM)), 256, 0, (cudaStream_t)stream>>>(x, m, k, w, n, bias, relu, out);
   SRF_LAUNCH_CHECK();
   return SRF_OK;
 }

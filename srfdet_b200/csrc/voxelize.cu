@@ -71,35 +71,111 @@ __device__ __forceinline__ uint32_t hash32(uint32_t k) {
   return k;
 }
 
+// Per-point / per-voxel bodies of the passes below, shared by srf_hard_voxelize (one cloud) and
+// srf_hard_voxelize_batch (B clouds, each with its own table, voxel block and list block).
+
+// pass 1 body: slot of point p's voxel in `table` (cap_mask + 1 entries), entry = key<<32 | min(idx);
+// -1 when p is out of range.  idx is the point's index in the scan's numbering.
+__device__ __forceinline__ int hv_insert_point(const float* __restrict__ p, uint32_t idx, const GeomDev& g,
+                                               unsigned long long* __restrict__ table, uint32_t cap_mask) {
+  float xyz[3] = {__ldg(p), __ldg(p + 1), __ldg(p + 2)};
+  int cx, cy, cz;
+  if (!point_cell(xyz, g, cx, cy, cz)) return -1;
+  uint32_t key = (uint32_t)((cz * g.grid[1] + cy) * g.grid[0] + cx);
+  unsigned long long mine = ((unsigned long long)key << 32) | idx;
+  uint32_t h = hash32(key) & cap_mask;
+  while (true) {
+    unsigned long long cur = table[h];
+    if (cur == HASH_EMPTY) {
+      unsigned long long old = atomicCAS(table + h, HASH_EMPTY, mine);
+      if (old == HASH_EMPTY) return (int)h;
+      cur = old;
+    }
+    if ((uint32_t)(cur >> 32) == key) {
+      atomicMin(table + h, mine);
+      return (int)h;
+    }
+    h = (h + 1) & cap_mask;
+  }
+}
+
+// pass 2c body: the first point of voxel v (slot s) publishes list row row0 + v and the coordinates (row v of coors)
+__device__ __forceinline__ void hv_assign_voxel(const unsigned long long* __restrict__ table, int s, int v, int max_voxels,
+                                                int row0, const GeomDev& g, int batch_idx, int32_t* __restrict__ slot2voxel,
+                                                int32_t* __restrict__ coors) {
+  if (v >= max_voxels) { slot2voxel[s] = -1; return; }
+  slot2voxel[s] = row0 + v;
+  uint32_t key = (uint32_t)(table[s] >> 32);
+  int cx = key % g.grid[0];
+  key /= g.grid[0];
+  int cy = key % g.grid[1];
+  int cz = key / g.grid[1];
+  if (batch_idx >= 0) {
+    reinterpret_cast<int4*>(coors)[v] = make_int4(batch_idx, cz, cy, cx);
+  } else {
+    coors[(size_t)v * 3 + 0] = cz;
+    coors[(size_t)v * 3 + 1] = cy;
+    coors[(size_t)v * 3 + 2] = cx;
+  }
+}
+
+// pass 3 body: sorted insertion of point index i into the slot list L (init 0x7f7f7f7f)
+__device__ __forceinline__ void hv_rank_insert(int32_t* __restrict__ L, int max_points, int i) {
+  int carry = i;
+  for (int t = 0; t < max_points; ++t) {
+    // cheap pre-check: a slot already holding a smaller index cannot take the carry
+    int seen = *((volatile int32_t*)(L + t));
+    if (seen < carry) continue;
+    int old = atomicMin(L + t, carry);
+    if (old == 0x7f7f7f7f) break;       // landed in a free slot
+    if (old > carry) carry = old;        // displaced a larger index: keep bubbling it
+  }
+}
+
+// pass 4 body: voxel v with slot list L: num_points[v], mean row v, point2voxel
+__device__ __forceinline__ void hv_gather_voxel(const float* __restrict__ pts, int c, const int32_t* __restrict__ L,
+                                                int max_points, int v, int32_t* __restrict__ num_points,
+                                                float* __restrict__ mean, int32_t* __restrict__ point2voxel) {
+  float acc[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+  int cnt = 0;
+  for (int t = 0; t < max_points; ++t) {
+    int i = L[t];
+    if (i == 0x7f7f7f7f) break;
+    ++cnt;
+    if (point2voxel) point2voxel[i] = v;
+    if (mean) {
+      const float* p = pts + (size_t)i * c;
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        if (j < c) acc[j] += __ldg(p + j);
+    }
+  }
+  num_points[v] = cnt;
+  if (mean) {
+    float fc = (float)cnt;
+#pragma unroll
+    for (int j = 0; j < 8; ++j)
+      if (j < c) mean[(size_t)v * c + j] = __fdiv_rn(acc[j], fc);
+  }
+}
+
+// payload body: element e = (voxel, slot, channel) of the voxel rows behind `lists`
+__device__ __forceinline__ void hv_payload_elem(const float* __restrict__ pts, int c, const int32_t* __restrict__ lists,
+                                                int64_t e, float* __restrict__ voxels) {
+  int j = (int)(e % c);
+  int64_t vs = e / c;
+  int i = lists[vs];
+  voxels[e] = (i == 0x7f7f7f7f) ? 0.f : __ldg(pts + (size_t)i * c + j);
+}
+
 // pass 1: key -> slot; entry = key<<32 | min(point index)
 __global__ void hv_insert_kernel(const float* __restrict__ pts, int n, int c, GeomDev g,
                                  unsigned long long* __restrict__ table, uint32_t cap_mask,
                                  int32_t* __restrict__ point_slot, int32_t* __restrict__ point2voxel) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const float* p = pts + (size_t)i * c;
-    float xyz[3] = {__ldg(p), __ldg(p + 1), __ldg(p + 2)};
-    int cx, cy, cz;
-    int slot = -1;
-    if (point_cell(xyz, g, cx, cy, cz)) {
-      uint32_t key = (uint32_t)((cz * g.grid[1] + cy) * g.grid[0] + cx);
-      unsigned long long mine = ((unsigned long long)key << 32) | (uint32_t)i;
-      uint32_t h = hash32(key) & cap_mask;
-      while (true) {
-        unsigned long long cur = table[h];
-        if (cur == HASH_EMPTY) {
-          unsigned long long old = atomicCAS(table + h, HASH_EMPTY, mine);
-          if (old == HASH_EMPTY) { slot = (int)h; break; }
-          cur = old;
-        }
-        if ((uint32_t)(cur >> 32) == key) {
-          atomicMin(table + h, mine);
-          slot = (int)h;
-          break;
-        }
-        h = (h + 1) & cap_mask;
-      }
-    }
-    point_slot[i] = slot;
+    point_slot[i] = hv_insert_point(pts + (size_t)i * c, (uint32_t)i, g, table, cap_mask);
     if (point2voxel) point2voxel[i] = -1;
   }
 }
@@ -125,26 +201,11 @@ __global__ void hv_assign_kernel(const unsigned long long* __restrict__ table,
   if (gid == 0) *d_voxel_num = min(*d_total, max_voxels);
   for (int i = gid; i < n; i += gridDim.x * blockDim.x) {
     if (!flag[i]) continue;
-    int s = point_slot[i];
-    int v = (int)rank[i];
-    if (v >= max_voxels) { slot2voxel[s] = -1; continue; }
-    slot2voxel[s] = v;
-    uint32_t key = (uint32_t)(table[s] >> 32);
-    int cx = key % g.grid[0];
-    key /= g.grid[0];
-    int cy = key % g.grid[1];
-    int cz = key / g.grid[1];
-    if (batch_idx >= 0) {
-      reinterpret_cast<int4*>(coors)[v] = make_int4(batch_idx, cz, cy, cx);
-    } else {
-      coors[(size_t)v * 3 + 0] = cz;
-      coors[(size_t)v * 3 + 1] = cy;
-      coors[(size_t)v * 3 + 2] = cx;
-    }
+    hv_assign_voxel(table, point_slot[i], (int)rank[i], max_voxels, 0, g, batch_idx, slot2voxel, coors);
   }
 }
 
-// pass 3: sorted insertion of the point index into its voxel's slot list (init 0x7f7f7f7f)
+// pass 3: sorted insertion of the point index into its voxel's slot list
 __global__ void hv_rank_kernel(const int32_t* __restrict__ point_slot, const int32_t* __restrict__ slot2voxel,
                                int n, int max_points, int32_t* __restrict__ lists) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -152,16 +213,7 @@ __global__ void hv_rank_kernel(const int32_t* __restrict__ point_slot, const int
     if (s < 0) continue;
     int v = slot2voxel[s];
     if (v < 0) continue;
-    int32_t* L = lists + (size_t)v * max_points;
-    int carry = i;
-    for (int t = 0; t < max_points; ++t) {
-      // cheap pre-check: a slot already holding a smaller index cannot take the carry
-      int seen = *((volatile int32_t*)(L + t));
-      if (seen < carry) continue;
-      int old = atomicMin(L + t, carry);
-      if (old == 0x7f7f7f7f) break;       // landed in a free slot
-      if (old > carry) carry = old;        // displaced a larger index: keep bubbling it
-    }
+    hv_rank_insert(lists + (size_t)v * max_points, max_points, i);
   }
 }
 
@@ -171,32 +223,8 @@ __global__ void hv_gather_kernel(const float* __restrict__ pts, int c, const int
                                  int32_t* __restrict__ num_points, float* __restrict__ mean,
                                  int32_t* __restrict__ point2voxel) {
   int m = *d_voxel_num;
-  for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < m; v += gridDim.x * blockDim.x) {
-    const int32_t* L = lists + (size_t)v * max_points;
-    float acc[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] = 0.f;
-    int cnt = 0;
-    for (int t = 0; t < max_points; ++t) {
-      int i = L[t];
-      if (i == 0x7f7f7f7f) break;
-      ++cnt;
-      if (point2voxel) point2voxel[i] = v;
-      if (mean) {
-        const float* p = pts + (size_t)i * c;
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-          if (j < c) acc[j] += __ldg(p + j);
-      }
-    }
-    num_points[v] = cnt;
-    if (mean) {
-      float fc = (float)cnt;
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        if (j < c) mean[(size_t)v * c + j] = __fdiv_rn(acc[j], fc);
-    }
-  }
+  for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < m; v += gridDim.x * blockDim.x)
+    hv_gather_voxel(pts, c, lists + (size_t)v * max_points, max_points, v, num_points, mean, point2voxel);
 }
 
 // optional payload: one thread per (voxel, slot, channel) element, coalesced writes
@@ -205,12 +233,99 @@ __global__ void hv_payload_kernel(const float* __restrict__ pts, int c, const in
                                   float* __restrict__ voxels) {
   int64_t total = (int64_t)(*d_voxel_num) * max_points * c;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total;
-       e += (int64_t)gridDim.x * blockDim.x) {
-    int j = (int)(e % c);
-    int64_t vs = e / c;
-    int i = lists[vs];
-    voxels[e] = (i == 0x7f7f7f7f) ? 0.f : __ldg(pts + (size_t)i * c + j);
+       e += (int64_t)gridDim.x * blockDim.x)
+    hv_payload_elem(pts, c, lists, e, voxels);
+}
+
+// ---- hard voxelization of B clouds in one launch sequence ------------------------------
+// The B clouds are numbered as one index space: point g of the batch is point g - off[b] of cloud b
+// (off = exclusive prefix of the clouds' row counts).  Each cloud has its own hash table of `cap`
+// entries (global slot = b * cap + h) and its own blocks of max_voxels rows in the lists and outputs.
+// Table entries carry g, so within a cloud the smallest entry is still the first point, and the
+// one scan over all flags numbers every cloud's voxels in its own first-come order once the cloud's
+// base rank[off[b]] is subtracted.  The lists keep cloud-local indices, so every per-point and
+// per-voxel body runs on exactly the values the single-cloud call gives it.
+struct HvBatchIn {
+  const float* pts[SRF_HV_BATCH_MAX];
+  int32_t off[SRF_HV_BATCH_MAX + 1];
+  int32_t n_batch;
+};
+
+// pass 1 of a batch; block 0 also copies the clouds' pointers and offsets into the workspace for the later passes
+__global__ void hvb_insert_kernel(const __grid_constant__ HvBatchIn in, int c, GeomDev g,
+                                  unsigned long long* __restrict__ table, uint32_t cap,
+                                  int32_t* __restrict__ point_slot, const float** __restrict__ ws_pts,
+                                  int32_t* __restrict__ ws_off) {
+  const int nb = in.n_batch, n = in.off[nb];
+  if (blockIdx.x == 0)
+    for (int t = threadIdx.x; t <= nb; t += blockDim.x) {
+      ws_off[t] = in.off[t];
+      if (t < nb) ws_pts[t] = in.pts[t];
+    }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    int lo = 0, hi = nb - 1;            // last cloud b with off[b] <= i (empty clouds have off[b] == off[b + 1])
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (in.off[mid] <= i) lo = mid; else hi = mid - 1;
+    }
+    const int h = hv_insert_point(in.pts[lo] + (size_t)(i - in.off[lo]) * c, (uint32_t)i, g, table + (size_t)lo * cap, cap - 1);
+    point_slot[i] = h < 0 ? -1 : lo * (int)cap + h;
   }
+}
+
+// pass 2c of a batch, and the per-cloud counts: cloud b has rank[off[b + 1]] - rank[off[b]] voxels
+__global__ void hvb_assign_kernel(const unsigned long long* __restrict__ table, const int32_t* __restrict__ point_slot,
+                                  const uint32_t* __restrict__ flag, const uint32_t* __restrict__ rank, int n,
+                                  const int32_t* __restrict__ off, int n_batch, uint32_t cap, GeomDev g, int max_voxels,
+                                  int32_t* __restrict__ slot2voxel, int32_t* __restrict__ coors,
+                                  int32_t* __restrict__ d_counts, const int32_t* __restrict__ d_total) {
+  const int gid = blockIdx.x * blockDim.x + threadIdx.x;
+  for (int b = gid; b < n_batch; b += gridDim.x * blockDim.x) {
+    const int o0 = off[b], o1 = off[b + 1];
+    const int base0 = o0 < n ? (int)rank[o0] : *d_total, base1 = o1 < n ? (int)rank[o1] : *d_total;
+    d_counts[b] = min(base1 - base0, max_voxels);
+  }
+  for (int i = gid; i < n; i += gridDim.x * blockDim.x) {
+    if (!flag[i]) continue;
+    const int s = point_slot[i], b = s / (int)cap;
+    hv_assign_voxel(table, s, (int)(rank[i] - rank[off[b]]), max_voxels, b * max_voxels, g, b, slot2voxel,
+                    coors + (size_t)b * max_voxels * 4);
+  }
+}
+
+// pass 3 of a batch: slot2voxel holds the list row b * max_voxels + v; the list gets the cloud-local index
+__global__ void hvb_rank_kernel(const int32_t* __restrict__ point_slot, const int32_t* __restrict__ slot2voxel, int n,
+                                const int32_t* __restrict__ off, uint32_t cap, int max_points, int32_t* __restrict__ lists) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int s = point_slot[i];
+    if (s < 0) continue;
+    const int row = slot2voxel[s];
+    if (row < 0) continue;
+    hv_rank_insert(lists + (size_t)row * max_points, max_points, i - off[s / (int)cap]);
+  }
+}
+
+// pass 4 of a batch: grid (x, B), one CTA row per cloud
+__global__ void hvb_gather_kernel(const float* const* __restrict__ pts, int c, const int32_t* __restrict__ lists,
+                                  int max_points, int max_voxels, const int32_t* __restrict__ d_counts,
+                                  int32_t* __restrict__ num_points, float* __restrict__ mean) {
+  const int b = blockIdx.y, m = d_counts[b];
+  const float* p = pts[b];
+  const size_t row0 = (size_t)b * max_voxels;
+  for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < m; v += gridDim.x * blockDim.x)
+    hv_gather_voxel(p, c, lists + (row0 + v) * max_points, max_points, v, num_points + row0,
+                    mean ? mean + row0 * c : nullptr, nullptr);
+}
+
+__global__ void hvb_payload_kernel(const float* const* __restrict__ pts, int c, const int32_t* __restrict__ lists,
+                                   int max_points, int max_voxels, const int32_t* __restrict__ d_counts,
+                                   float* __restrict__ voxels) {
+  const int b = blockIdx.y;
+  const float* p = pts[b];
+  const size_t row0 = (size_t)b * max_voxels * max_points;
+  const int64_t total = (int64_t)d_counts[b] * max_points * c;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x)
+    hv_payload_elem(p, c, lists + row0, e, voxels + row0 * c);
 }
 
 // ---- batched hard voxelization: compaction of per-sample blocks ---------------------------
@@ -287,6 +402,52 @@ static HvWs hv_layout(void* base, int n, int max_points, int max_voxels) {
   w.d_total = (int32_t*)take(256);
   w.slot2voxel = (int32_t*)take((size_t)w.cap * 4);
   w.lists = (int32_t*)take((size_t)max_voxels * max_points * 4);
+  w.bytes = off;
+  return w;
+}
+
+struct HvbWs {
+  unsigned long long* table;
+  uint32_t cap;
+  int64_t n;  // points of the whole batch
+  int32_t* point_slot;
+  uint32_t* flag;
+  uint32_t* rank;
+  uint32_t* blocksum;
+  int32_t* d_total;
+  int32_t* slot2voxel;
+  int32_t* lists;
+  const float** pts;
+  int32_t* off;
+  size_t bytes;
+};
+
+// counts: host row counts of the B clouds (all >= 0)
+static HvbWs hvb_layout(void* base, const int32_t* counts, int nb, int max_points, int max_voxels) {
+  HvbWs w;
+  int32_t n_max = 0;
+  w.n = 0;
+  for (int b = 0; b < nb; ++b) {
+    w.n += counts[b];
+    n_max = counts[b] > n_max ? counts[b] : n_max;
+  }
+  w.cap = hv_capacity(n_max);
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    size_t o = off;
+    off += (bytes + 255) / 256 * 256;
+    return (char*)base + o;
+  };
+  w.table = (unsigned long long*)take((size_t)nb * w.cap * 8);
+  w.point_slot = (int32_t*)take((size_t)w.n * 4);
+  w.flag = (uint32_t*)take((size_t)w.n * 4);
+  w.rank = (uint32_t*)take((size_t)w.n * 4);
+  w.blocksum = (uint32_t*)take((SCAN_BLOCKS + 4) * 4);
+  w.d_total = (int32_t*)take(256);
+  w.slot2voxel = (int32_t*)take((size_t)nb * w.cap * 4);
+  w.lists = (int32_t*)take((size_t)nb * max_voxels * max_points * 4);
+  w.pts = (const float**)take((size_t)nb * 8);
+  w.off = (int32_t*)take((size_t)(nb + 1) * 4);
   w.bytes = off;
   return w;
 }
@@ -385,6 +546,72 @@ int srf_hard_voxelize(const float* points, int32_t n, int32_t c, const srf_geom*
   if (voxels)
     hv_payload_kernel<<<launch_grid((int64_t)max_voxels * max_points * c, 256), 256, 0, st>>>(
         points, c, w.lists, max_points, d_voxel_num, voxels);
+  SRF_LAUNCH_CHECK();
+  return SRF_OK;
+}
+
+static bool hvb_counts_ok(const int32_t* counts, int nb) {
+  int64_t n = 0;
+  for (int b = 0; b < nb; ++b) {
+    if (counts[b] < 0) return false;
+    n += counts[b];
+  }
+  return n <= 0x7fffffff;
+}
+
+size_t srf_hard_voxelize_batch_ws_bytes(const int32_t* n, int32_t batch, int32_t max_points, int32_t max_voxels) {
+  if (!n || batch < 1 || batch > SRF_HV_BATCH_MAX || max_points <= 0 || max_voxels <= 0 || !hvb_counts_ok(n, batch)) return 0;
+  return hvb_layout(nullptr, n, batch, max_points, max_voxels).bytes;
+}
+
+int srf_hard_voxelize_batch(const float* const* points, const int32_t* n, int32_t batch, int32_t c, const srf_geom* g,
+                            int32_t max_points, int32_t max_voxels, float* voxels, int32_t* coors, int32_t* num_points,
+                            float* mean, int32_t* d_counts, void* ws, size_t ws_bytes, void* stream) {
+  SRF_CHECK_ARG(points && n && g && coors && num_points && d_counts, "srf_hard_voxelize_batch: null arg");
+  SRF_CHECK_ARG(batch >= 1 && batch <= SRF_HV_BATCH_MAX, "srf_hard_voxelize_batch: need 1 <= batch <= %d (got %d)",
+                SRF_HV_BATCH_MAX, batch);
+  SRF_CHECK_ARG(c >= 3 && c <= 8, "srf_hard_voxelize_batch: need 3 <= c <= 8 (got %d)", c);
+  SRF_CHECK_ARG(max_points > 0 && max_voxels > 0, "srf_hard_voxelize_batch: max_points/max_voxels must be > 0");
+  SRF_CHECK_ARG(hvb_counts_ok(n, batch), "srf_hard_voxelize_batch: row counts must be >= 0 and sum to < 2^31");
+  for (int b = 0; b < batch; ++b)
+    SRF_CHECK_ARG(points[b] || n[b] == 0, "srf_hard_voxelize_batch: cloud %d: null points", b);
+  GeomDev gd;
+  SRF_CHECK_ARG(fill_geom(&gd, g) == 0, "srf_hard_voxelize_batch: bad geometry");
+  HvbWs w = hvb_layout(ws, n, batch, max_points, max_voxels);
+  SRF_CHECK_ARG((int64_t)batch * w.cap < 0x7fffffff && (int64_t)batch * max_voxels < 0x7fffffff,
+                "srf_hard_voxelize_batch: batch x table capacity (%lld) and batch x max_voxels (%lld) must be < 2^31",
+                (long long)batch * w.cap, (long long)batch * max_voxels);
+  SRF_CHECK_ARG(ws && ws_bytes >= w.bytes, "srf_hard_voxelize_batch: workspace too small (%zu < %zu)", ws_bytes, w.bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (w.n == 0) {
+    SRF_CUDA(cudaMemsetAsync(d_counts, 0, (size_t)batch * 4, st));
+    return SRF_OK;
+  }
+  HvBatchIn in;
+  in.n_batch = batch;
+  in.off[0] = 0;
+  for (int b = 0; b < batch; ++b) {
+    in.pts[b] = points[b];
+    in.off[b + 1] = in.off[b] + n[b];
+  }
+  const int np = (int)w.n;
+  SRF_CUDA(cudaMemsetAsync(w.table, 0xff, (size_t)batch * w.cap * 8, st));
+  SRF_CUDA(cudaMemsetAsync(w.lists, 0x7f, (size_t)batch * max_voxels * max_points * 4, st));
+  const int gp = launch_grid(np, 256);
+  SRF_COUNT(voxels ? 6 : 5);
+  hvb_insert_kernel<<<gp, 256, 0, st>>>(in, c, gd, w.table, w.cap, w.point_slot, w.pts, w.off);
+  hv_flag_kernel<<<gp, 256, 0, st>>>(w.table, w.point_slot, np, w.flag);
+  int rc = scan_flags_launch(w.flag, w.rank, w.blocksum, np, w.d_total, 0, st);
+  if (rc) return rc;
+  hvb_assign_kernel<<<launch_grid(np > batch ? np : batch, 256), 256, 0, st>>>(
+      w.table, w.point_slot, w.flag, w.rank, np, w.off, batch, w.cap, gd, max_voxels, w.slot2voxel, coors, d_counts, w.d_total);
+  hvb_rank_kernel<<<gp, 256, 0, st>>>(w.point_slot, w.slot2voxel, np, w.off, w.cap, max_points, w.lists);
+  const int gv = max(1, launch_grid((int64_t)batch * max_voxels, 128) / batch);
+  hvb_gather_kernel<<<dim3(gv, batch), 128, 0, st>>>(w.pts, c, w.lists, max_points, max_voxels, d_counts, num_points, mean);
+  if (voxels) {
+    const int ge = max(1, launch_grid((int64_t)batch * max_voxels * max_points * c, 256) / batch);
+    hvb_payload_kernel<<<dim3(ge, batch), 256, 0, st>>>(w.pts, c, w.lists, max_points, max_voxels, d_counts, voxels);
+  }
   SRF_LAUNCH_CHECK();
   return SRF_OK;
 }

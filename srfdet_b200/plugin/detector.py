@@ -12,6 +12,7 @@ samples is B independent batch-1 calls of the reference (SURVEY.md §3.4), each 
 lidar2img.
 """
 import collections
+import ctypes
 import os
 
 import numpy as np
@@ -56,27 +57,36 @@ class SRFDetPointPath(nn.Module):
 
     @torch.no_grad()
     def hard_voxel_blocks(self, points, want_voxels=False, want_mean=False):
-        """Hard voxelization of B clouds without a host read: sample i fills block i of max_voxels rows.
+        """Hard voxelization of B clouds without a host read, in one srf_hard_voxelize_batch call: sample i fills block i
+        of max_voxels rows, as Voxelization.hard_padded(points[i], batch_idx=i) would.
         -> dict(voxels (B, M, T, C) | None, num_points (B, M), coors (B, M, 4) bzyx, mean (B, M, C) | None,
         count (B,) int32 device); rows past a block's count are unspecified."""
         assert not self.is_dynamic
         bs, c, dev = len(points), points[0].shape[1], points[0].device
         if any(p.shape[1] != c for p in points):
             raise ValueError('all clouds of a batch need the same number of point features')
-        mv = int(self.pts_voxel_layer._max_voxels())
-        if mv <= 0:
-            mv = max(max(p.shape[0] for p in points), 1)
-        T = int(self.pts_voxel_layer.max_num_points)
+        mv, T = self._block_rows([p.shape[0] for p in points]), int(self.pts_voxel_layer.max_num_points)
         blk = dict(voxels=torch.empty((bs, mv, T, c), dtype=torch.float32, device=dev) if want_voxels else None,
                    num_points=torch.empty((bs, mv), dtype=torch.int32, device=dev),
                    coors=torch.empty((bs, mv, 4), dtype=torch.int32, device=dev),
                    mean=torch.empty((bs, mv, c), dtype=torch.float32, device=dev) if want_mean else None,
-                   count=torch.zeros((bs,), dtype=torch.int32, device=dev))
-        for i, p in enumerate(points):
-            self.pts_voxel_layer.hard_padded(p, batch_idx=i, want_voxels=want_voxels, want_mean=want_mean,
-                                             out={k: None if v is None else v[i:i + 1] if k == 'count' else v[i]
-                                                  for k, v in blk.items()})
+                   count=torch.empty((bs,), dtype=torch.int32, device=dev))
+        clouds = [p.contiguous().float() for p in points]
+        ptrs = (ctypes.c_void_p * bs)(*[p.data_ptr() for p in clouds])
+        ns = (ctypes.c_int32 * bs)(*[p.shape[0] for p in clouds])
+        lib = L.load()
+        ws = torch.empty((int(lib.srf_hard_voxelize_batch_ws_bytes(ns, bs, T, mv)) + 255) // 256 * 256, dtype=torch.uint8,
+                         device=dev)
+        L.check(lib.srf_hard_voxelize_batch(ptrs, ns, bs, c, ctypes.byref(self.pts_voxel_layer.geom), T, mv,
+                                            L.ptr(blk['voxels']), L.ptr(blk['coors']), L.ptr(blk['num_points']),
+                                            L.ptr(blk['mean']), L.ptr(blk['count']), L.ptr(ws), ws.numel(), L.stream_ptr()),
+                'srf_hard_voxelize_batch')
         return blk
+
+    def _block_rows(self, counts):
+        """Rows of each sample's voxel block: the voxel layer's test max_voxels (a value <= 0: the largest cloud)."""
+        mv = int(self.pts_voxel_layer._max_voxels())
+        return mv if mv > 0 else max(max(counts), 1)
 
     @torch.no_grad()
     def pillar_rows(self, points, enc):
@@ -144,6 +154,9 @@ def _drop_init_cfg(cfg):
     return cfg
 
 
+# Camera-fusion samples per call: a deliberate limit of the fusion path (its image RoI sampling and the batched
+# camera tests cover up to 8 samples); LiDAR-only batches have no such limit.
+FUSION_MAX_SAMPLES = 8
 CheckpointKeys = collections.namedtuple('CheckpointKeys', ['missing_keys', 'unexpected_keys', 'set_aside_keys'])
 _IMAGE_PREFIXES = ('img_backbone.', 'img_neck.')
 
@@ -281,6 +294,32 @@ class SRFDet(SRFDetPointPath):
                 raise ValueError('this fusion config needs img_feats (the image-neck outputs, one (B, n_cam, C, H, W) map per '
                                  'level) and lidar2img (B, n_cam, 4, 4)')
             self._check_fusion_batch(len(points), img_feats, lidar2img)
+        if not self.is_dynamic:
+            self._check_voxel_batch([p.shape[0] for p in points], points[0].shape[1])
+
+    def _check_memory(self, points):
+        """Before the device work of an eager run or a graph capture (a replay allocates nothing): the free-memory check of
+        _check_voxel_batch."""
+        if not self.is_dynamic:
+            self._check_voxel_batch([p.shape[0] for p in points], points[0].shape[1], points[0].device)
+
+    def _check_voxel_batch(self, counts, c, device=None):
+        """Hard-voxel configs, before any device work: srf_hard_voxelize_batch takes at most SRF_HV_BATCH_MAX clouds, and,
+        given the CUDA device, its workspace and voxel blocks must fit in the device memory that is free (the rest of the
+        network scales with the batch too, so a batch that passes can still run out of memory later)."""
+        if len(counts) > L.HV_BATCH_MAX:
+            raise ValueError(f'{len(counts)} clouds: hard voxelization (srf_hard_voxelize_batch) takes at most '
+                             f'{L.HV_BATCH_MAX} clouds per call')
+        if not isinstance(device, torch.device) or device.type != 'cuda':
+            return
+        bs, mv, T = len(counts), self._block_rows(counts), int(self.pts_voxel_layer.max_num_points)
+        ws = L.load().srf_hard_voxelize_batch_ws_bytes((ctypes.c_int32 * bs)(*counts), bs, T, mv)
+        need = ws + bs * mv * (4 + 16 + (T * c * 4 if self.is_pillar else c * 4))
+        free = torch.cuda.mem_get_info(device)[0] + torch.cuda.memory_reserved(device) - torch.cuda.memory_allocated(device)
+        if need > free:
+            raise torch.cuda.OutOfMemoryError(
+                f'{bs} clouds: hard voxelization needs {need / 2**30:.2f} GiB of device memory (workspace and voxel blocks) and '
+                f'{free / 2**30:.2f} GiB are free: run fewer clouds (or views) per call')
 
     def _check_fusion_batch(self, n, img_feats, lidar2img):
         """n clouds need n samples of image maps and n camera sets (SURVEY.md §3.4: a batch of B fusion samples is B
@@ -302,9 +341,8 @@ class SRFDet(SRFDetPointPath):
             raise ValueError(f'image maps of batch {mb} for {n} clouds: the maps need one sample per cloud')
         if l2i != (n, n_cam, 4, 4) and not (n == 1 and l2i == (n_cam, 4, 4)):
             raise ValueError(f'lidar2img {l2i} does not match {n} sample(s) of {n_cam} cameras: pass ({n}, {n_cam}, 4, 4)')
-        if getattr(self.bbox_head, 'with_dpg', False) and n > L.GEMV_MAX_ROWS:
-            raise ValueError(f'{n} samples: the dynamic proposal generation projections (srf_gemv_f32) take at most '
-                             f'{L.GEMV_MAX_ROWS} samples per call')
+        if n > FUSION_MAX_SAMPLES:
+            raise ValueError(f'{n} samples: camera fusion takes at most {FUSION_MAX_SAMPLES} samples per call')
 
     @torch.no_grad()
     def _infer_eager(self, points, img_feats, lidar2img, precision):
@@ -328,6 +366,7 @@ class SRFDet(SRFDetPointPath):
         self._check_inputs(points, img_feats, lidar2img)
         precision = precision or registry.get_precision()
         if not self.use_graph:
+            self._check_memory(points)
             return self._infer_eager(points, img_feats, lidar2img, precision)
         key = (tuple(tuple(p.shape) for p in points), precision,
                None if img_feats is None else tuple((tuple(f.shape), f.stride()) for f in img_feats),
@@ -335,6 +374,7 @@ class SRFDet(SRFDetPointPath):
         n, n_img = len(points), len(img_feats or [])
 
         def statics():
+            self._check_memory(points)
             return ([p.contiguous().clone() for p in points] + [torch.empty_like(f).copy_(f) for f in img_feats or []]
                     + [None if lidar2img is None else lidar2img.clone()])
 
@@ -380,6 +420,16 @@ class SRFDet(SRFDetPointPath):
         if self.bbox_head.test_cfg.get('max_num') is None:
             raise ValueError('test-time augmentation needs test_cfg.max_num (merge_aug_bboxes_3d keeps that many boxes)')
 
+    def _check_aug_views(self, n_views):
+        """srf_merge_aug_bev's limits, before any device work: at most AUG_MAX_VIEWS views and MERGE_AUG_MAX_K candidates
+        (views x the head's max_per_img NMS rows) per sample."""
+        if not 1 <= n_views <= L.AUG_MAX_VIEWS:
+            raise ValueError(f'{n_views} distinct views: 1 to {L.AUG_MAX_VIEWS} are supported')
+        rows = int(self.bbox_head.test_cfg['max_per_img'])
+        if n_views * rows > L.MERGE_AUG_MAX_K:
+            raise ValueError(f'{n_views} views x {rows} boxes (test_cfg.max_per_img) = {n_views * rows} candidates per sample: '
+                             f'the merge of the views (srf_merge_aug_bev) takes at most {L.MERGE_AUG_MAX_K}')
+
     def _merge_views(self, out, bs, views):
         """Per-view NMS outputs of a (bs * A)-cloud batch, sample-major -> merge_aug_bboxes_3d per sample."""
         from .nms import merge_aug_device
@@ -406,10 +456,10 @@ class SRFDet(SRFDetPointPath):
         range, precision)."""
         from .points import augment_points, distinct_views
         self._check_aug()
-        self._check_inputs(points, None, None)
         views = distinct_views(views)
-        if not 1 <= len(views) <= L.AUG_MAX_VIEWS:
-            raise ValueError(f'{len(views)} distinct views: 1 to {L.AUG_MAX_VIEWS} are supported')
+        self._check_aug_views(len(views))
+        view_batch = [p for p in points for _ in views]                           # the B x A views the detector runs
+        self._check_inputs(view_batch, None, None)
         precision = precision or registry.get_precision()
         rng = None if point_cloud_range is None else [float(v) for v in point_cloud_range]
         n = len(points)
@@ -422,11 +472,15 @@ class SRFDet(SRFDetPointPath):
             return self._merge_views(self._infer_eager(batch, None, None, precision), n, views)
         inputs = list(points) + [counts]
         if not self.use_graph:
+            self._check_memory(view_batch)
             return run(*inputs)
         key = ('aug', tuple(tuple(p.shape) for p in points), tuple(views), None if rng is None else tuple(rng),
                counts is None, precision)
-        return self._graph_call(key, lambda: [p.contiguous().clone() for p in points] + [None if counts is None else counts.clone()],
-                                run, inputs)
+
+        def statics():
+            self._check_memory(view_batch)
+            return [p.contiguous().clone() for p in points] + [None if counts is None else counts.clone()]
+        return self._graph_call(key, statics, run, inputs)
 
     @torch.no_grad()
     def aug_test(self, points, img_metas, img=None, img_feats=None, rescale=False):
@@ -448,8 +502,10 @@ class SRFDet(SRFDetPointPath):
             if len(v) != 1:
                 raise ValueError(f'the samples of one augmentation have different flips / scales: {sorted(v)}')
             views.append(v.pop())
+        self._check_aug_views(a)
         clouds = [points[j][i] for i in range(bs) for j in range(a)]          # sample-major: the views of a sample together
         self._check_inputs(clouds, None, None)
+        self._check_memory(clouds)
         out = self._merge_views(self._infer_eager(clouds, None, None, registry.get_precision()), bs, views)
         res = self.bbox_head.format_nms(*out, [m for m in img_metas[0]])
         return [dict(pts_bbox=dict(boxes_3d=bx.to('cpu'), scores_3d=sc.cpu(), labels_3d=lb.cpu())) for bx, sc, lb in res]

@@ -80,7 +80,7 @@ def capture():
 
 
 def _family(name, a, s):
-    if name in ('srf_hard_voxelize', 'srf_dynamic_voxelize'):
+    if name in ('srf_hard_voxelize', 'srf_hard_voxelize_batch', 'srf_dynamic_voxelize'):
         return 'voxelize'
     if name in ('srf_dynamic_vfe', 'srf_dynamic_scatter'):
         return 'dynamic VFE'
@@ -128,6 +128,9 @@ def _work(name, a, s, ctx):
     if name == 'srf_hard_voxelize':
         m = ctx['n_voxels']
         return 0.0, n_pts * c_pts * 4 + m * (16 + 4) + m * c_pts * 4
+    if name == 'srf_hard_voxelize_batch':          # a[2] clouds, each counted as the frame's cloud
+        m = ctx['n_voxels']
+        return 0.0, a[2] * (n_pts * c_pts * 4 + m * (16 + 4) + m * c_pts * 4)
     if name == 'srf_dynamic_voxelize':
         return 0.0, n_pts * c_pts * 4 + n_pts * 16
     if name in ('srf_dynamic_vfe', 'srf_dynamic_scatter'):

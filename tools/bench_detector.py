@@ -1,6 +1,6 @@
 """Detector-level timings (CUDA events on the launching stream, 512 MiB L2 flush between steps, median of `--iters`):
 
-    python tools/bench_detector.py [--kinds nusc waymo pillar tta nusc_lc] [--iters 20]
+    python tools/bench_detector.py [--kinds nusc waymo pillar tta nusc_lc batch] [--iters 20]
 
 Per configuration (nusc_L, waymo_L; calibrated synthetic weights of RegionFeaturePipeline, production-size clouds,
 the configs' rotated NMS on) one JSON line per case:
@@ -33,6 +33,12 @@ camera rig turned about z per sample):
   run_frames x4      RegionFeaturePipeline(fusion=True).run_frames: 4 single-frame graphs in flight (frames/s);
   kernel             srf_img_roi_features alone at B = 1 and B = 4 (900 proposals per sample, 128 channels, fp32
                      channel-last output; us per call).
+batch (large LiDAR batches; not in the default kinds): 32 distinct 300k-point nuScenes clouds,
+  infer B=1..32      one CUDA graph over the batch for nusc_L (weights as above) and the pillar config (seeded weights),
+                     frames/s and torch.cuda.max_memory_allocated of the call (graphs of other batch sizes dropped first);
+  infer_aug B=4x4    4 clouds x the 4 distinct flip views in one graph (16 views, nusc_L);
+  voxelize B=4/32    srf_hard_voxelize_batch (one launch sequence, nusc_L voxel layer, means) against the B
+                     srf_hard_voxelize calls it replaces (us per batch, eager, L2 flushed), with a bit-for-bit check.
 The first line names the GPU and its power limit.
 """
 import argparse
@@ -229,12 +235,12 @@ def bench_pillar(iters, flush):
     det.reset_graphs()
 
 
-def bench_tta(iters, flush):
+def _tta_nusc_det():
+    """nusc_L with RegionFeaturePipeline's calibrated weights, rotated NMS and max_num = 500 for the TTA merge.
+    -> (detector, precision)"""
     from srfdet_b200 import synth
     from srfdet_b200.pipeline import RegionFeaturePipeline, backbone_cfg, head_cfg, MODEL_CFG
     from srfdet_b200.plugin import SRFDet
-    from srfdet_b200.plugin.nms import merge_aug_device
-    from srfdet_b200.plugin.points import augment_points
     pipe = RegionFeaturePipeline('nusc', fusion=False, scope='full', use_nms=True)
     pipe.calibrate(torch.as_tensor(synth.cloud('nusc', 44)).cuda())
     head = head_cfg('nusc', False, use_nms=True)
@@ -244,7 +250,15 @@ def bench_tta(iters, flush):
     for prefix, m in (('pts_backbone.', pipe.backbone), ('pts_neck.', pipe.neck), ('bbox_head.', pipe.head)):
         sd.update({prefix + k: v for k, v in m.state_dict().items()})
     det.load_checkpoint(sd)
-    name, prec = 'nusc_L', pipe.precision
+    return det, pipe.precision
+
+
+def bench_tta(iters, flush):
+    from srfdet_b200 import synth
+    from srfdet_b200.plugin.nms import merge_aug_device
+    from srfdet_b200.plugin.points import augment_points
+    det, prec = _tta_nusc_det()
+    name = 'nusc_L'
     pcr = [-55.2, -55.2, -5.0, 55.2, 55.2, 3.0]
     cloud = torch.as_tensor(synth.cloud('nusc', 1000)).cuda()
 
@@ -266,6 +280,66 @@ def bench_tta(iters, flush):
     out('kernel srf_merge_aug_bev (8 views x 300 rows, 10 classes)', ms, 0, us=round(ms * 1e3, 1),
         candidates=int(c8.sum()))
     det.reset_graphs()
+
+
+def bench_batch(iters, flush):
+    from srfdet_b200 import synth
+    from srfdet_b200.pipeline import init_synthetic_backbone, init_synthetic_head
+    from srfdet_b200.plugin import SRFDet
+    nusc, prec = _tta_nusc_det()
+    cfg = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'tests', 'golden', 'configs', 'pipeline',
+                       'srfdet_pillar_nusc_L.py')
+    pillar = SRFDet.from_config(cfg)
+    init_synthetic_backbone(pillar.pts_backbone, 1)
+    init_synthetic_backbone(pillar.pts_neck, 2)
+    init_synthetic_head(pillar.bbox_head, 3)
+    pillar = pillar.cuda()
+    pillar.use_graph = True
+    clouds = [torch.as_tensor(synth.cloud('nusc', 1000 + i)).cuda() for i in range(32)]
+
+    def out(name, case, ms, frames_n, **extra):
+        print(json.dumps(dict(config=name, case=case, precision=prec if name == 'nusc_L' else 'fp16', ms=round(ms, 4),
+                              frames_per_s=round(frames_n / ms * 1e3, 1) if frames_n else None, **extra)), flush=True)
+
+    def peak(fn):
+        """-> (median ms, GiB peak of allocated memory over capture and replays) with no other graph held."""
+        torch.cuda.synchronize()
+        torch.cuda.empty_cache()
+        torch.cuda.reset_peak_memory_stats()
+        ms = timed(fn, iters, flush)
+        return ms, round(torch.cuda.max_memory_allocated() / 2 ** 30, 2)
+    for name, det in (('nusc_L', nusc), ('pillar_nusc_L', pillar)):
+        for b in (1, 2, 4, 8, 16, 32):
+            det.reset_graphs()
+            ms, gib = peak(lambda: det.infer(clouds[:b]))
+            out(name, f'infer B={b} (one graph)', ms, b, max_memory_allocated_gib=gib)
+        det.reset_graphs()
+    del pillar
+    flips = [(1.0, False, False), (1.0, True, False), (1.0, False, True), (1.0, True, True)]
+    pcr = [-55.2, -55.2, -5.0, 55.2, 55.2, 3.0]
+    ms, gib = peak(lambda: nusc.infer_aug(clouds[:4], flips, pcr))
+    out('nusc_L', 'infer_aug B=4 x 4 distinct views (one graph: augment + batch of 16 + merge)', ms, 4, max_memory_allocated_gib=gib)
+    nusc.reset_graphs()
+    vox = nusc.pts_voxel_layer
+    for b in (4, 32):
+        def singles():
+            blk = dict(num_points=torch.empty((b, 160000), dtype=torch.int32, device='cuda'),
+                       coors=torch.empty((b, 160000, 4), dtype=torch.int32, device='cuda'),
+                       mean=torch.empty((b, 160000, 5), device='cuda'), count=torch.empty((b,), dtype=torch.int32, device='cuda'))
+            for i, p in enumerate(clouds[:b]):
+                vox.hard_padded(p, batch_idx=i, want_voxels=False, want_mean=True,
+                                out={k: v[i:i + 1] if k == 'count' else v[i] for k, v in blk.items()})
+            return blk
+        batched = lambda: nusc.hard_voxel_blocks(clouds[:b], want_mean=True)
+        got, ref = batched(), singles()
+        same = all(torch.equal(got['count'], ref['count']) and torch.equal(got[k][i, :int(ref['count'][i])],
+                                                                           ref[k][i, :int(ref['count'][i])])
+                   for k in ('num_points', 'coors', 'mean') for i in range(b))
+        ms_b, ms_s = timed(batched, iters * 2, flush), timed(singles, iters * 2, flush)
+        out('nusc_L', f'voxelize B={b}: srf_hard_voxelize_batch (one launch sequence)', ms_b, 0, us=round(ms_b * 1e3, 1),
+            bit_identical_to_single_calls=same, points=b * int(clouds[0].shape[0]))
+        out('nusc_L', f'voxelize B={b}: {b} srf_hard_voxelize calls', ms_s, 0, us=round(ms_s * 1e3, 1),
+            speedup_of_batch=round(ms_s / ms_b, 2))
 
 
 def _camera_maps(seed, b, c, n_cam=6):
@@ -320,7 +394,7 @@ def bench_nusc_lc(iters, flush):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar', 'tta', 'nusc_lc'])
+    ap.add_argument('--kinds', nargs='+', default=['nusc', 'waymo', 'pillar'], choices=['nusc', 'waymo', 'kitti', 'pillar', 'tta', 'nusc_lc', 'batch'])
     ap.add_argument('--iters', type=int, default=20)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -334,6 +408,8 @@ def main():
             bench_tta(a.iters, flush)
         elif kind == 'nusc_lc':
             bench_nusc_lc(a.iters, flush)
+        elif kind == 'batch':
+            bench_batch(a.iters, flush)
         else:
             bench_kind(kind, a.iters, flush)
 
